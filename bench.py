@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- self-play MCTS simulations/sec (BASELINE.json's metric) for the lockstep engine on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--games G] [--sims S] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--games G] [--sims S] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[3] "lockstep self-play 4,096 games x 200 sims/move on 1 B200",
 random-init ChessRL network, synthetic start/midgame positions (half the lanes advanced by 8-60 seeded random
@@ -18,6 +18,9 @@ A STEP is one move search for all G lanes: a fresh tree per game, S simulations,
   cpu_baseline : the oracle port of the reference path (python-chess restatement + mctree restatement + torch-CPU
                  fp32 network, all host threads) on a bounded sample of the same workload; reported, not the target.
   perft        : secondary metric of BASELINE.json (perft nodes/s over >= 65,536 lockstep boards), bit-exact totals.
+
+--dump-outputs DIR writes what the last timed step of each leg returned, as DIR/<name>.npy (float32 / float64), so that
+two builds can be compared output for output; the inputs depend only on the arguments.  See dump_outputs().
 """
 
 import argparse
@@ -621,6 +624,35 @@ def WORKLOAD(args):
     return "lockstep self-play %d games/GPU x %d sims/move, random-init ChessRL net (%s)" % (args.games, args.sims, which)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, stats, picks, chosen):
+    """Writes the last timed step's results as out_dir/<name>.npy, one row per lane:
+      visits, values, priors, moves, replies, results [lanes, 256], n_children, root_visits, root_values [lanes]
+        -- Engine.root_stats() after the last device-resident step (the `value` leg);
+      e2e_picks [lanes], e2e_chosen [lanes, 2] -- the picks and the (move, reply) words Engine.commit returned in the
+        last step of the `e2e` leg.
+    Integers are stored as float32 (exact: every value is below 2**24), float64 stays float64.  If all lanes together
+    would exceed DUMP_LIMIT_BYTES, a fixed seeded sample of lanes is written instead; lanes.npy lists the lane indices."""
+    arrays = {k: stats[k] for k in ("visits", "values", "priors", "moves", "replies", "results", "n_children",
+                                    "root_visits", "root_values")}
+    arrays["e2e_picks"] = picks
+    arrays["e2e_chosen"] = chosen
+    arrays = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    n = len(arrays["root_visits"])
+    per_lane = sum(v.nbytes for v in arrays.values()) // n + 8
+    lanes = np.arange(n)
+    if per_lane * n > DUMP_LIMIT_BYTES:
+        lanes = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // per_lane, replace=False))
+    arrays = {k: np.ascontiguousarray(v[lanes]) for k, v in arrays.items()}
+    arrays["lanes"] = lanes.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    sys.stderr.write("bench: wrote %d arrays for %d of %d lanes to %s\n" % (len(arrays), len(lanes), n, out_dir))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -640,7 +672,11 @@ def main():
     ap.add_argument("--whole-games", type=int, default=0, help="also play this many COMPLETE games (drain included)")
     ap.add_argument("--wg-lanes", type=int, default=None)
     ap.add_argument("--wg-sims", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (root statistics, e2e picks) as DIR/<name>.npy (rank 0's lanes)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -700,22 +736,24 @@ def main():
         st = eng.root_stats(want=("visits",))                              # device -> host
         _, plies, results = eng.games_get(0, G)
         picks = pick_moves(st["visits"], st["n_children"], st["root_visits"], plies, results == B.RESULT_NONE, True)
-        return eng.commit(picks, apply=False)                              # host -> device, device -> host
+        return picks, eng.commit(picks, apply=False)                       # host -> device, device -> host
 
     np.random.seed(0)
 
     def timed(fn, steps, warmup):
+        """-> (summed step ms, counter deltas, what the last timed fn() call returned)"""
         for _ in range(warmup):
             flush.fill_(1)
             fn()
         barrier()
         c0 = eng.counters()
         evs = []
+        last = None
         for _ in range(steps):
             flush.fill_(1)                                                 # L2 flush between timed iterations
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            fn()
+            last = fn()
             b.record()
             evs.append((a, b))
         barrier()
@@ -725,15 +763,18 @@ def main():
             t = torch.tensor([ms], device="cuda", dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, {k: c1[k] - c0[k] for k in c0}
+        return ms, {k: c1[k] - c0[k] for k in c0}, last
 
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ms_dev, cnt_dev = timed(device_step, args.steps, args.warmup)
+    ms_dev, cnt_dev, _ = timed(device_step, args.steps, args.warmup)
     clocks = sampler.stop()
+    dev_stats = eng.root_stats() if args.dump_outputs and rank == 0 else None     # the last device step's trees
     wall0 = time.perf_counter()
-    ms_e2e, cnt_e2e = timed(e2e_step, args.steps, max(1, min(args.warmup, 1)))
+    ms_e2e, cnt_e2e, (e2e_picks, e2e_chosen) = timed(e2e_step, args.steps, max(1, min(args.warmup, 1)))
     del wall0
+    if dev_stats is not None:
+        dump_outputs(args.dump_outputs, dev_stats, e2e_picks, e2e_chosen)
     sims_dev = cnt_dev["simulations"]
     sims_e2e = cnt_e2e["simulations"]
     if world > 1:

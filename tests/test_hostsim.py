@@ -27,6 +27,7 @@ def lib():
     L.hs_tree_new.restype = ctypes.c_void_p
     L.hs_tree_new.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int16)]
     L.hs_game_set.argtypes = [ctypes.c_void_p, u64p, u16p, ctypes.c_int]
+    L.hs_game_move.argtypes = [ctypes.c_void_p, ctypes.c_uint16]    # undeclared, the handle would pass as a 32-bit int
     L.hs_search.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_int]
     L.hs_search_wave.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_uint64, ctypes.c_int]
     L.hs_root_stats.argtypes = [ctypes.c_void_p, i32p, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_float),

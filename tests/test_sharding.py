@@ -1,5 +1,6 @@
 """Multi-process path on CPU (gloo, world_size 2): shard ranges, weight broadcast, finished-game gather."""
 import os
+import socket
 import subprocess
 import sys
 import textwrap
@@ -33,12 +34,20 @@ WORKER = textwrap.dedent("""
 """)
 
 
+def _free_port():
+    """A loopback port nobody holds right now: a fixed one may be taken by another job on a shared host."""
+    with socket.socket(socket.AF_INET, socket.SOCK_STREAM) as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
+
 def test_gloo_world2(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(WORKER % (ROOT, str(tmp_path)))
-    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29577")
+    port = str(_free_port())
+    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT=port)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-           "--master-addr", "127.0.0.1", "--master-port", "29577", str(script)]
+           "--master-addr", "127.0.0.1", "--master-port", port, str(script)]
     p = subprocess.run(cmd, capture_output=True, text=True, env=env, timeout=240)
     assert p.returncode == 0, p.stderr[-2000:]
     import json

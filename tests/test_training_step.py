@@ -9,6 +9,7 @@ max|g32 - g64| <= 2e-2 * max|g64| and ||g32 - g64|| <= 4e-3 * ||g64|| -- about t
 restatement itself evaluated in fp32 is off by 0.9e-2 / 1.2e-3 on the worst tensor); moving statistics 1e-5; the Adam
 update itself (same gradients fed to both) 1e-6.
 """
+import contextlib
 import random
 
 import numpy as np
@@ -46,13 +47,30 @@ def step_data():
     return pack, x, pol, val, tr, ref_losses, ref_grads, ref_stats
 
 
+@contextlib.contextmanager
+def _fixed_cpu_summation_order():
+    """One thread and ATen's own convolutions (no oneDNN).  The BatchNorm beta gradients are sums over the batch that
+    cancel heavily, so their fp32 error depends on how a sum is split: the CPU kernels split it by thread count, and
+    with the defaults the worst relative L2 error moves between 1.2e-3 and 7.3e-3 over 1-16 threads, above the bound
+    on a 16-core host.  With the order fixed it is 1.7e-3 whatever the host's core count."""
+    threads, onednn = torch.get_num_threads(), torch.backends.mkldnn.enabled
+    torch.set_num_threads(1)
+    torch.backends.mkldnn.enabled = False
+    try:
+        yield
+    finally:
+        torch.set_num_threads(threads)
+        torch.backends.mkldnn.enabled = onednn
+
+
 def _torch_step(pack, x, pol, val, tr, device="cpu"):
     params = [torch.tensor(w, device=device) for w in pack]
     for i in tr:
         params[i].requires_grad_(True)
-    total, lp, lv, reg, _ = training.loss_terms(params, torch.as_tensor(x, device=device), torch.as_tensor(pol, device=device),
-                                                torch.as_tensor(val, device=device), training=True)
-    grads = torch.autograd.grad(total, [params[i] for i in tr])
+    with _fixed_cpu_summation_order() if device == "cpu" else contextlib.nullcontext():
+        total, lp, lv, reg, _ = training.loss_terms(params, torch.as_tensor(x, device=device), torch.as_tensor(pol, device=device),
+                                                    torch.as_tensor(val, device=device), training=True)
+        grads = torch.autograd.grad(total, [params[i] for i in tr])
     return params, {"loss": total.item(), "policy_loss": lp.item(), "value_loss": lv.item(), "reg": reg.item()}, grads
 
 

@@ -61,6 +61,7 @@ SIGNATURES = {
     "crl_net_forward": (ctypes.c_int, [vp, vp, ctypes.c_int, vp, vp]),
     "crl_debug_conv": (ctypes.c_int, [vp, ctypes.c_int, vp, ctypes.c_int, ctypes.c_int, vp, vp, ctypes.c_int]),
     "crl_debug_tower": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp]),
+    "crl_debug_forward_counted": (ctypes.c_int, [vp, vp, ctypes.c_int, vp, vp, vp]),
     "crl_hash_eval": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_uint64, ctypes.c_int, vp, vp]),
     "crl_set_evaluator": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_uint64, ctypes.c_int]),
     "crl_games_set_host": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, c_u64p, c_u16p, c_i32p, ctypes.c_int]),

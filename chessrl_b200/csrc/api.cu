@@ -599,6 +599,17 @@ int crl_debug_tower(crl_engine* e, const void* planes_bf16_dev, int n, int layer
   return net_debug_tower(e, (const __nv_bfloat16*)planes_bf16_dev, n, layer, (__nv_bfloat16*)act_out_dev, logits_out_dev,
                          (__nv_bfloat16*)pf_out_dev, vf_out_dev, policy_dev, value_dev);
 }
+int crl_debug_forward_counted(crl_engine* e, const void* planes_bf16_dev, int n_bound, const int32_t* n_dev,
+                              float* policy_dev, float* value_dev) {
+  CHECK_ENGINE(e);
+  if (n_bound < 0 || !n_dev || (n_bound > 0 && (!planes_bf16_dev || !policy_dev || !value_dev))) {
+    set_error("crl_debug_forward_counted: bad arguments");
+    return CRL_EINVAL;
+  }
+  // the launch sequence of a search batch: host bound, row count read on the device, production tower and heads
+  return net_forward(e, (const __nv_bfloat16*)planes_bf16_dev, n_bound, (const int*)n_dev, policy_dev, value_dev, nullptr,
+                     -1, nullptr);
+}
 int crl_hash_eval(crl_engine* e, const uint64_t* boards_dev, int n, uint64_t seed, int policy_bits, float* policy_dev,
                   float* value_dev) {
   CHECK_ENGINE(e);

@@ -207,6 +207,22 @@ class Engine:
                                        _ptr(out["pf"]), _ptr(out["vf"]), _ptr(out["policy"]), _ptr(out["value"])))
         return out
 
+    def debug_forward_counted(self, planes_t, n_bound, count, policy=None, value=None):
+        """Test hook: net_forward as a search batch runs it -- launched for n_bound rows, with the row count `count` read
+        by the kernels from device memory (int, or a device int32 tensor of one element).  Rows at or after the count
+        of `policy` [n_bound,1968] / `value` [n_bound] (allocated when None) are left as they were."""
+        dev = self.device
+        if policy is None:
+            policy = torch.empty((n_bound, _lib.N_LABELS), dtype=torch.float32, device=dev)
+        if value is None:
+            value = torch.empty((n_bound,), dtype=torch.float32, device=dev)
+        if not torch.is_tensor(count):
+            count = torch.tensor([int(count)], dtype=torch.int32, device=dev)
+        assert count.dtype == torch.int32 and count.device == dev
+        check(self.lib.crl_debug_forward_counted(self.h, _ptr(planes_t), int(n_bound), _ptr(count), _ptr(policy),
+                                                 _ptr(value)))
+        return policy, value
+
     def hash_eval(self, boards_t, seed, policy_bits=24):
         n = boards_t.shape[1]
         policy = torch.empty((n, _lib.N_LABELS), dtype=torch.float32, device=self.device)

@@ -157,6 +157,11 @@ int crl_debug_conv(crl_engine* e, int layer, const void* in_dev, int cin, int n,
  *   policy_dev [n][1968], value_dev [n] as crl_net_forward.  Any tap may be NULL. */
 int crl_debug_tower(crl_engine* e, const void* planes_bf16_dev, int n, int layer, void* act_out_dev, float* logits_out_dev,
                     void* pf_out_dev, float* vf_out_dev, float* policy_dev, float* value_dev);
+/* test hook: crl_net_forward with the row count of a search batch -- the kernels are launched for n_bound rows of
+ * planes_bf16_dev and read the count *n_dev (device int32) themselves; only rows below min(n_bound, *n_dev) are
+ * evaluated and only those rows of policy_dev [n_bound][1968] / value_dev [n_bound] are written */
+int crl_debug_forward_counted(crl_engine* e, const void* planes_bf16_dev, int n_bound, const int32_t* n_dev,
+                              float* policy_dev, float* value_dev);
 /* the deterministic test evaluator on raw boards (SoA), same outputs as the oracle's hash_evaluator */
 int crl_hash_eval(crl_engine* e, const uint64_t* boards_dev, int n, uint64_t seed, int policy_bits,
                   float* policy_dev, float* value_dev);

@@ -15,7 +15,6 @@ import threading
 
 import numpy as np
 import pytest
-import torch
 
 import chessrl_oracle as O
 from chessrl_b200 import boards as B
@@ -23,51 +22,9 @@ from chessrl_b200 import model
 from chessrl_b200._lib import EVAL_NET
 from chessrl_b200.engine import Engine
 from chessrl_b200.lockstep import compute_policy
+from net_oracle import BatchedNetEvaluator
 
 pytestmark = pytest.mark.gpu
-
-
-class BatchedNetEvaluator:
-    """Oracle trees run in threads; their evaluation requests are served in one GPU batch whenever every live
-    thread is waiting (this is test plumbing, the numbers come from crl_net_forward)."""
-
-    def __init__(self, engine, n_threads):
-        self.e = engine
-        self.live = n_threads
-        self.cv = threading.Condition()
-        self.pending = []
-        self.gen = 0
-
-    def _flush(self):
-        games = [g for g, _ in self.pending]
-        planes = np.stack([O.planes(g) for g in games]).astype(np.float32)
-        x = torch.zeros(len(games), 8, 8, 128, dtype=torch.bfloat16, device=self.e.device)
-        x[..., :127] = torch.from_numpy(planes).to(self.e.device).to(torch.bfloat16)
-        p, v = self.e.net_forward(x)
-        p, v = p.cpu().numpy(), v.cpu().numpy()
-        for i, (_, slot) in enumerate(self.pending):
-            slot.append((p[i].copy(), np.float32(v[i])))
-        self.pending = []
-        self.gen += 1
-        self.cv.notify_all()
-
-    def __call__(self, game):
-        slot = []
-        with self.cv:
-            self.pending.append((game, slot))
-            if len(self.pending) >= self.live:
-                self._flush()
-            else:
-                gen = self.gen
-                while self.gen == gen:
-                    self.cv.wait()
-        return slot[0]
-
-    def done(self):
-        with self.cv:
-            self.live -= 1
-            if self.live > 0 and len(self.pending) >= self.live:
-                self._flush()
 
 
 def test_lockstep_real_network_matches_oracle_visit_counts():

@@ -22,6 +22,7 @@ vp = ctypes.c_void_p
 
 CRL_OK, CRL_EINVAL, CRL_ECUDA, CRL_ENOMEM, CRL_ESTATE = 0, -1, -2, -3, -4
 EVAL_NET, EVAL_HASH = 0, 1
+NET_BF16, NET_FP8 = 0, 1
 N_LABELS = 1968
 MAX_MOVES = 256
 N_WEIGHT_TENSORS = 140
@@ -62,6 +63,9 @@ SIGNATURES = {
     "crl_debug_conv": (ctypes.c_int, [vp, ctypes.c_int, vp, ctypes.c_int, ctypes.c_int, vp, vp, ctypes.c_int]),
     "crl_debug_tower": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp]),
     "crl_debug_forward_counted": (ctypes.c_int, [vp, vp, ctypes.c_int, vp, vp, vp]),
+    "crl_net_calibrate_host": (ctypes.c_int, [vp, vp, ctypes.c_int, c_f32p]),
+    "crl_net_load_fp8_host": (ctypes.c_int, [vp, ctypes.POINTER(c_f32p), c_i64p, ctypes.c_int, c_f32p]),
+    "crl_net_set_precision": (ctypes.c_int, [vp, ctypes.c_int]),
     "crl_hash_eval": (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_uint64, ctypes.c_int, vp, vp]),
     "crl_set_evaluator": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_uint64, ctypes.c_int]),
     "crl_games_set_host": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, c_u64p, c_u16p, c_i32p, ctypes.c_int]),

@@ -610,6 +610,27 @@ int crl_debug_forward_counted(crl_engine* e, const void* planes_bf16_dev, int n_
   return net_forward(e, (const __nv_bfloat16*)planes_bf16_dev, n_bound, (const int*)n_dev, policy_dev, value_dev, nullptr,
                      -1, nullptr);
 }
+int crl_net_calibrate_host(crl_engine* e, const void* planes_bf16_dev, int n, float* amax_host) {
+  CHECK_ENGINE(e);
+  if (!planes_bf16_dev || !amax_host) {
+    set_error("crl_net_calibrate_host: null arguments");
+    return CRL_EINVAL;
+  }
+  return net_calibrate(e, (const __nv_bfloat16*)planes_bf16_dev, n, amax_host);
+}
+int crl_net_load_fp8_host(crl_engine* e, const float* const* weights_host, const int64_t* sizes, int n_tensors,
+                          const float* act_amax_host) {
+  CHECK_ENGINE(e);
+  if (!weights_host || !sizes || !act_amax_host) {
+    set_error("crl_net_load_fp8_host: null arguments");
+    return CRL_EINVAL;
+  }
+  return net_load_fp8(e, weights_host, sizes, n_tensors, act_amax_host);
+}
+int crl_net_set_precision(crl_engine* e, int precision) {
+  CHECK_ENGINE(e);
+  return net_set_precision(e, precision);
+}
 int crl_hash_eval(crl_engine* e, const uint64_t* boards_dev, int n, uint64_t seed, int policy_bits, float* policy_dev,
                   float* value_dev) {
   CHECK_ENGINE(e);

@@ -159,6 +159,12 @@ int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int 
                     float* logits_out, __nv_bfloat16* pf_out, float* vf_out, float* policy, float* value);
 int net_debug_conv(crl_engine_impl* e, int layer, const __nv_bfloat16* in, int cin, int n, const __nv_bfloat16* residual,
                    __nv_bfloat16* out, int relu);
+// fp8 evaluation (crl_net_calibrate_host, crl_net_load_fp8_host, crl_net_set_precision)
+int net_calibrate(crl_engine_impl* e, const __nv_bfloat16* planes, int n, float* amax_host);
+int net_load_fp8(crl_engine_impl* e, const float* const* w, const int64_t* sizes, int n, const float* act_amax);
+int net_set_precision(crl_engine_impl* e, int precision);
+// true while the fp8 tower is selected: the search then encodes e4m3 planes into e->d_planes
+bool net_fp8(const crl_engine_impl* e);
 
 }  // namespace crl
 

@@ -28,9 +28,10 @@ struct EncShared {
 // six black piece bits, "no white piece", six white piece bits; bit 126 = side to move).  Step 2: all threads expand
 // mask bytes to bf16 and store 16 bytes each, 2 KB contiguous per block-wide store -- the kernel is then bound by the
 // 16 KB it writes per position, not by bit fiddling.
-template <int T>
+// OutT = uint8_t: e4m3 planes for the fp8 tower (1.0 = 0x38), 8 KB per position.
+template <int T, class OutT = __nv_bfloat16>
 __device__ __forceinline__ void write_planes(const EncShared& s, unsigned (*s_mask)[4],
-                                             __nv_bfloat16* __restrict__ out) {
+                                             OutT* __restrict__ out) {
   if (threadIdx.x < 64) {
     const int cell = threadIdx.x;
     const int sq = (7 - (cell >> 3)) * 8 + (cell & 7);
@@ -57,17 +58,34 @@ __device__ __forceinline__ void write_planes(const EncShared& s, unsigned (*s_ma
   }
   __syncthreads();
   uint4* dst = reinterpret_cast<uint4*>(out);
+  if constexpr (sizeof(OutT) == 1) {
 #pragma unroll
-  for (int j = 0; j < 1024 / T; ++j) {
-    const int id = j * T + threadIdx.x;             // 16-byte chunk id: 64 squares x 16 chunks of 8 channels
-    const int cell = id >> 4, chunk = id & 15;
-    const unsigned bits = (s_mask[cell][chunk >> 2] >> ((chunk & 3) * 8)) & 0xFFu;
-    uint4 q;
-    q.x = ((bits & 1) ? 0x3F80u : 0u) | ((bits & 2) ? 0x3F800000u : 0u);
-    q.y = ((bits & 4) ? 0x3F80u : 0u) | ((bits & 8) ? 0x3F800000u : 0u);
-    q.z = ((bits & 16) ? 0x3F80u : 0u) | ((bits & 32) ? 0x3F800000u : 0u);
-    q.w = ((bits & 64) ? 0x3F80u : 0u) | ((bits & 128) ? 0x3F800000u : 0u);
-    dst[id] = q;
+    for (int j = 0; j < 512 / T; ++j) {
+      const int id = j * T + threadIdx.x;           // 16-byte chunk id: 64 squares x 8 chunks of 16 channels
+      const int cell = id >> 3, chunk = id & 7;
+      const unsigned bits = (s_mask[cell][chunk >> 1] >> ((chunk & 1) * 16)) & 0xFFFFu;
+      uint32_t w[4];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        w[k] = 0;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) w[k] |= ((bits >> (4 * k + b)) & 1u) ? (0x38u << (8 * b)) : 0u;
+      }
+      dst[id] = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 1024 / T; ++j) {
+      const int id = j * T + threadIdx.x;             // 16-byte chunk id: 64 squares x 16 chunks of 8 channels
+      const int cell = id >> 4, chunk = id & 15;
+      const unsigned bits = (s_mask[cell][chunk >> 2] >> ((chunk & 3) * 8)) & 0xFFu;
+      uint4 q;
+      q.x = ((bits & 1) ? 0x3F80u : 0u) | ((bits & 2) ? 0x3F800000u : 0u);
+      q.y = ((bits & 4) ? 0x3F80u : 0u) | ((bits & 8) ? 0x3F800000u : 0u);
+      q.z = ((bits & 16) ? 0x3F80u : 0u) | ((bits & 32) ? 0x3F800000u : 0u);
+      q.w = ((bits & 64) ? 0x3F80u : 0u) | ((bits & 128) ? 0x3F800000u : 0u);
+      dst[id] = q;
+    }
   }
 }
 
@@ -99,8 +117,8 @@ __global__ void __launch_bounds__(ENC_THREADS) k_encode_boards(const u64* __rest
 // when which==0.  64 threads per row: the history walk is a short pointer chase by one thread, and with 32 resident
 // blocks per SM a whole 4,096-row batch is one wave, so every chase overlaps the other rows' stores.
 static constexpr int ENC_ROW_THREADS = 64;
-__global__ void __launch_bounds__(ENC_ROW_THREADS) k_encode_rows(Pools P, int which,
-                                                             __nv_bfloat16* __restrict__ planes) {
+template <class OutT>
+__global__ void __launch_bounds__(ENC_ROW_THREADS) k_encode_rows(Pools P, int which, OutT* __restrict__ planes) {
   __shared__ EncShared s;
   __shared__ unsigned s_mask[64][4];
   const int r = blockIdx.x;
@@ -123,7 +141,7 @@ __global__ void __launch_bounds__(ENC_ROW_THREADS) k_encode_rows(Pools P, int wh
     s.turn = (int)(meta & 1);
   }
   __syncthreads();
-  write_planes<ENC_ROW_THREADS>(s, s_mask, planes + (long long)r * 64 * 128);
+  write_planes<ENC_ROW_THREADS, OutT>(s, s_mask, planes + (long long)r * 64 * 128);
 }
 
 __global__ void k_policy_index(const u16* __restrict__ moves, const int* __restrict__ counts, int n,
@@ -203,7 +221,10 @@ int launch_eval_batch(crl_engine_impl* e, int which) {
   }
   {
     LaunchScope ls(e, KC_ENCODE);
-    k_encode_rows<<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(e->P, which, e->d_planes);
+    if (net_fp8(e))   // the fp8 tower reads e4m3 rows from the same buffer
+      k_encode_rows<uint8_t><<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(e->P, which, (uint8_t*)e->d_planes);
+    else
+      k_encode_rows<__nv_bfloat16><<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(e->P, which, e->d_planes);
     CRL_CUDA(cudaGetLastError());
   }
   return net_forward(e, e->d_planes, e->cur_rows, e->P.eval_n, e->d_policy, e->d_value, nullptr, -1, &e->pview);

@@ -887,7 +887,8 @@ int tree_run_steps(crl_engine_impl* e, int n_sims, int K) {
   const unsigned long long key = 1ull + (unsigned long long)e->eval_kind + 2ull * (unsigned long long)e->eval_bits +
                                  64ull * (e->eval_seed * 0x9E3779B97F4A7C15ull) + 0x100000000ull * (unsigned long long)K +
                                  (e->reuse ? 0x8000000000000000ull : 0ull) +
-                                 0x9E3779B97F4A7C15ull * (unsigned long long)(e->row_bound > 0 ? e->row_bound : 0);
+                                 0x9E3779B97F4A7C15ull * (unsigned long long)(e->row_bound > 0 ? e->row_bound : 0) +
+                                 (net_fp8(e) ? 0x4000000000000000ull : 0ull);
   if (e->sim_graph[par] == nullptr || e->sim_graph_key[par] != key) {
     if (e->sim_graph[par]) {
       cudaGraphExecDestroy(e->sim_graph[par]);

@@ -25,7 +25,10 @@
 #include "engine.cuh"
 
 #include <cuda.h>
+#include <cuda_fp16.h>
+#include <cuda_fp8.h>
 #include <math.h>
+#include <type_traits>
 #include <stdlib.h>
 #include <string.h>
 
@@ -536,6 +539,18 @@ __device__ __forceinline__ void umma2_bf16(uint32_t tmem_d, uint64_t desc_a, uin
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// e4m3 x e4m3 -> fp32, K = 32 per instruction (the same 32 bytes of a swizzle row as a bf16 K = 16 step)
+__device__ __forceinline__ void umma2_fp8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// instruction descriptor: fp32 accumulate, A = B = E4M3 (format 0), both K-major, N = 256, M = 256 (CTA pair)
+static constexpr uint32_t V2_IDESC_FP8 = (1u << 4) | ((TILE_N >> 3) << 17) | ((256u >> 4) << 24);
 // arrive (once the issued MMAs retire) on the barrier at this offset in BOTH CTAs of the pair
 __device__ __forceinline__ void umma2_commit_both(uint64_t* bar) {
   asm volatile(
@@ -784,6 +799,24 @@ struct LayerDesc {
   const float* shift;
   const __nv_bfloat16* residual;
   __nv_bfloat16* out;
+};
+// the fp8 tower's layer table (k_trunk4<..., FP8 = true>): activations are e4m3 codes x a power-of-two scale per layer.
+// scale[n] already holds weight scale x input scale x folded BatchNorm scale; the residual is the block input, stored
+// with its own layer's scale s_res; the output is stored as e4m3(a * inv_out) and means code x s_out.
+struct LayerDesc8 {
+  int map_in;
+  int map_w;
+  int k_chunks;          // Cin / 128
+  int relu;
+  int fuse_heads;
+  int write_out;
+  const float* scale;
+  const float* shift;
+  const uint8_t* residual;
+  uint8_t* out;
+  float s_res;
+  float s_out;
+  float inv_out;
 };
 struct TrunkParams {
   const int* n_dev;
@@ -1055,10 +1088,17 @@ __device__ __forceinline__ uint64_t make_kmajor_sw128_desc_sbo(uint32_t smem_add
   return (uint64_t)((smem_addr >> 4) & 0x3FFF) | ((uint64_t)(sbo_bytes >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
-template <int T4_NA, int T4_NB, bool SINGLE = false>
+// FP8 (a separate instantiation, <3, 7> only): the same pipeline on e4m3 operands.  A 128-byte swizzle row then holds
+// 128 channels, so a slice is 128 channels and the boxes keep their byte sizes; each MMA is kind::f8f6f4 with K = 32.
+// The epilogue applies the per-layer scales of LayerDesc8 and stores e4m3 codes; the last convolution (fused heads only)
+// rounds to bf16 exactly as the bf16 tower does.
+template <int T4_NA, int T4_NB, bool SINGLE = false, bool FP8 = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CONV_THREADS, 1)
 k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __restrict__ maps,
-         const LayerDesc* __restrict__ layers, TrunkParams p) {
+         const typename std::conditional<FP8, LayerDesc8, LayerDesc>::type* __restrict__ layers, TrunkParams p) {
+  using LD = typename std::conditional<FP8, LayerDesc8, LayerDesc>::type;
+  using ActT = typename std::conditional<FP8, uint8_t, __nv_bfloat16>::type;
+  constexpr int KSLICE = FP8 ? 128 : BLOCK_K;         // channels per 128-byte swizzle row
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   uint8_t* smem_a = smem;
@@ -1130,7 +1170,7 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
     int uses = 0;
     for (int grp = pair; grp < n_groups; grp += n_pairs) {
       for (int L = 0; L < NL; ++L, ++uses) {
-        const LayerDesc ld = layers[L];
+        const LD ld = layers[L];
         const CUtensorMap* map_a = ld.map_in == 0 ? &map_planes : maps + ld.map_in;
         const CUtensorMap* map_w = maps + ld.map_w;
         for (int X = 0; X < XN; ++X) {
@@ -1142,7 +1182,7 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
             // coordinates (channel, x, board, y): the box {64, 10, 2, 10} starts one pixel outside the board.
             // The planes are indexed by board, the activation scratch by this pair's slot.
             const int b0 = (ld.map_in == 0 ? tile * 4 : pair * 8 + X * 4) + (int)rank * 2;
-            tma2_load_4d_hint(smem_a + as * T4_A_SLOT, map_a, &a_full[as], kc * BLOCK_K, -1, b0, -1,
+            tma2_load_4d_hint(smem_a + as * T4_A_SLOT, map_a, &a_full[as], kc * KSLICE, -1, b0, -1,
                               ld.map_in == 0 ? p.hint_planes : L2_EVICT_NORMAL);
             if (rank != 0) mbar_arrive_remote(&a_full[as], 0);
             if (++as == T4_NA) {
@@ -1152,7 +1192,7 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
             for (int tap = 0; tap < 9; ++tap) {
               mbar_wait(&b_empty[bs], bphase ^ 1);
               if (rank == 0) mbar_arrive_expect_tx(&b_full[bs], 2 * T4_B_BYTES);
-              tma2_load_2d_hint(smem_b + bs * T4_B_BYTES, map_w, &b_full[bs], (tap * ld.k_chunks + kc) * BLOCK_K,
+              tma2_load_2d_hint(smem_b + bs * T4_B_BYTES, map_w, &b_full[bs], (tap * ld.k_chunks + kc) * KSLICE,
                                 (int)rank * 128, p.hint_weights);
               if (rank != 0) mbar_arrive_remote(&b_full[bs], 0);
               if (++bs == T4_NB) {
@@ -1185,7 +1225,10 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
               const int dy = tap / 3, dx = tap - 3 * dy;                 // already offset by +1
               const uint64_t da = make_kmajor_sw128_desc_sbo(img + (uint32_t)(dy * 20 + dx) * 128u, 1280u);
               const uint64_t db = make_kmajor_sw128_desc(smem_u32(smem_b + bs * T4_B_BYTES));
-              if (p.probe_nsplit) {
+              if constexpr (FP8) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) umma2_fp8(tmem_d, da + 2 * k, db + 2 * k, V2_IDESC_FP8, (kc | tap | k) != 0);
+              } else if (p.probe_nsplit) {
                 // (timing probe, see TrunkParams) rows 64..127 of this CTA's weight tile start 8 KB = 512 x 16 B further on
 #pragma unroll
                 for (int k = 0; k < BLOCK_K / 16; ++k) {
@@ -1224,7 +1267,7 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
     int uses = 0;
     for (int grp = pair; grp < n_groups; grp += n_pairs) {
       for (int L = 0; L < NL; ++L, ++uses) {
-        const LayerDesc ld = layers[L];
+        const LD ld = layers[L];
         asm volatile("bar.sync 1, 128;" ::: "memory");
         for (int i = threadIdx.x - 128; i < TILE_N; i += 128) {
           s_scale[i] = ld.scale[i];
@@ -1239,10 +1282,72 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
           const long long grow = (long long)board * 64 + ey * 8 + ex;                    // row by board (heads, tap)
           const long long srow = (long long)(pair * 8 + X * 4 + (int)rank * 2 + eb) * 64 + ey * 8 + ex;   // row by slot
           const bool valid = board < n_boards;
-          __nv_bfloat16* orow = ld.write_out ? ld.out + srow * TILE_N : nullptr;
-          const __nv_bfloat16* rrow = ld.residual ? ld.residual + srow * TILE_N : nullptr;
+          ActT* orow = ld.write_out ? ld.out + srow * TILE_N : nullptr;
+          const ActT* rrow = ld.residual ? ld.residual + srow * TILE_N : nullptr;
           __nv_bfloat16* drow = (p.dbg_out && L == p.dbg_layer) ? p.dbg_out + grow * TILE_N : nullptr;
           float h0 = 0.f, h1 = 0.f, h2 = 0.f;
+          if constexpr (FP8) {
+#pragma unroll 1
+            for (int c0 = 0; c0 < TILE_N; c0 += 32) {
+              uint32_t v[32];
+              tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + X * TILE_N + c0, v);
+              tmem_ld_wait();
+              if (!valid) continue;
+              uint4 res[2];
+              if (rrow) {
+                res[0] = *reinterpret_cast<const uint4*>(rrow + c0);
+                res[1] = *reinterpret_cast<const uint4*>(rrow + c0 + 16);
+              }
+              float a[32];
+#pragma unroll
+              for (int j = 0; j < 32; ++j) a[j] = __uint_as_float(v[j]) * s_scale[c0 + j] + s_shift[c0 + j];
+              if (rrow) {
+                const __nv_fp8x2_storage_t* r2 = reinterpret_cast<const __nv_fp8x2_storage_t*>(res);
+#pragma unroll
+                for (int h = 0; h < 16; ++h) {
+                  const float2 f = __half22float2(__half2(__nv_cvt_fp8x2_to_halfraw2(r2[h], __NV_E4M3)));
+                  a[2 * h] += f.x * ld.s_res;
+                  a[2 * h + 1] += f.y * ld.s_res;
+                }
+              }
+              if (ld.relu) {
+#pragma unroll
+                for (int j = 0; j < 32; ++j) a[j] = fmaxf(a[j], 0.f);
+              }
+              if (ld.fuse_heads) {
+#pragma unroll
+                for (int j = 0; j < 32; ++j) {
+                  const float x = __bfloat162float(__float2bfloat16_rn(a[j]));
+                  h0 = fmaf(x, s_hw[c0 + j], h0);
+                  h1 = fmaf(x, s_hw[256 + c0 + j], h1);
+                  h2 = fmaf(x, s_hw[512 + c0 + j], h2);
+                }
+                if (drow) {
+#pragma unroll
+                  for (int j = 0; j < 16; ++j)
+                    reinterpret_cast<__nv_bfloat162*>(drow + c0)[j] = __floats2bfloat162_rn(a[2 * j], a[2 * j + 1]);
+                }
+              } else if (orow || drow) {
+                alignas(16) __nv_fp8x2_storage_t pk[16];   // read back as two uint4
+#pragma unroll
+                for (int h = 0; h < 16; ++h)
+                  pk[h] = __nv_cvt_float2_to_fp8x2(make_float2(a[2 * h] * ld.inv_out, a[2 * h + 1] * ld.inv_out),
+                                                   __NV_SATFINITE, __NV_E4M3);
+                if (orow) {
+                  const uint4* src = reinterpret_cast<const uint4*>(pk);
+                  *reinterpret_cast<uint4*>(orow + c0) = src[0];
+                  *reinterpret_cast<uint4*>(orow + c0 + 16) = src[1];
+                }
+                if (drow) {   // the stored value code x s_out is exact in bf16
+#pragma unroll
+                  for (int h = 0; h < 16; ++h) {
+                    const float2 f = __half22float2(__half2(__nv_cvt_fp8x2_to_halfraw2(pk[h], __NV_E4M3)));
+                    reinterpret_cast<__nv_bfloat162*>(drow + c0)[h] = __floats2bfloat162_rn(f.x * ld.s_out, f.y * ld.s_out);
+                  }
+                }
+              }
+            }
+          } else {
 #pragma unroll 1
           for (int c0 = 0; c0 < TILE_N; c0 += 32) {
             uint32_t v[32];
@@ -1294,6 +1399,7 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
                 if (drow) *reinterpret_cast<uint4*>(drow + c0 + 8 * j) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
               }
             }
+          }
           }
           tcgen05_fence_before();
           mbar_arrive_remote(&tmem_empty[X], 0);
@@ -1405,6 +1511,40 @@ __global__ void __launch_bounds__(256) k_softmax_value(TailParams p) {
   if (lane == 0) p.value[pos] = tanhf(v + p.bv2[0]);
 }
 
+// fp8 tower input: bf16 planes -> e4m3 (round to nearest even, saturating; the encoder's 0 / 1 planes are exact), 8 per thread
+__global__ void __launch_bounds__(256) k_planes_to_e4m3(const uint4* __restrict__ in, uint2* __restrict__ out, long long n8) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n8) return;
+  const uint4 v = in[i];
+  const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+  uint32_t pk[2];
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const float2 f0 = make_float2(__uint_as_float(w[2 * h] << 16), __uint_as_float(w[2 * h] & 0xFFFF0000u));
+    const float2 f1 = make_float2(__uint_as_float(w[2 * h + 1] << 16), __uint_as_float(w[2 * h + 1] & 0xFFFF0000u));
+    pk[h] = (uint32_t)__nv_cvt_float2_to_fp8x2(f0, __NV_SATFINITE, __NV_E4M3) |
+            ((uint32_t)__nv_cvt_float2_to_fp8x2(f1, __NV_SATFINITE, __NV_E4M3) << 16);
+  }
+  out[i] = make_uint2(pk[0], pk[1]);
+}
+
+// calibration: *amax = max(*amax, max |x|) over n8 x 8 bf16 values (non-negative floats order as their bit patterns)
+__global__ void __launch_bounds__(256) k_absmax_bf16(const uint4* __restrict__ x, long long n8, unsigned* amax) {
+  float m = 0.f;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (long long)gridDim.x * blockDim.x) {
+    const uint4 v = x[i];
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int h = 0; h < 4; ++h) {
+      m = fmaxf(m, fabsf(__uint_as_float(w[h] << 16)));
+      m = fmaxf(m, fabsf(__uint_as_float(w[h] & 0xFFFF0000u)));
+    }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
+  if ((threadIdx.x & 31) == 0) atomicMax(amax, __float_as_uint(m));
+}
+
 // ======================================================================================================
 // host side: weight pack, tensor maps, forward
 // ======================================================================================================
@@ -1459,6 +1599,16 @@ struct NetWeights {
   CUtensorMap* d_maps = nullptr;            // [3 + N_CONVS] device copies: (unused: the planes map is a kernel
                                             // parameter), act[0], act[1], weights (128-filter boxes)
   LayerDesc* d_layers = nullptr;            // [N_CONVS]
+  // fp8 tower (crl_net_load_fp8_host); buffers are allocated by the first fp8 load
+  bool fp8_loaded = false;
+  bool fp8 = false;                         // the fp8 tower is selected
+  bool planes_fp8 = false;                  // dtype of the cached planes maps
+  uint8_t* w8[N_CONVS] = {nullptr};         // [256][9*Cin] e4m3, K-major
+  float* scale8[N_CONVS] = {nullptr};       // weight scale x input scale x BatchNorm scale
+  float* shift8[N_CONVS] = {nullptr};
+  uint8_t* act8[2] = {nullptr, nullptr};    // [act4_rows][64][256] e4m3 scratch by CTA-pair slot
+  CUtensorMap* d_maps8 = nullptr;
+  LayerDesc8* d_layers8 = nullptr;
 };
 
 static int make_act_map(NetWeights* nw, CUtensorMap* map, const void* base, int cin, int rows) {
@@ -1477,12 +1627,15 @@ static int make_act_map(NetWeights* nw, CUtensorMap* map, const void* base, int 
 }
 // v4: the same activations seen as (C, W, B, H), box {64, 10, 2, 10} = the zero-padded image of two boards laid out
 // [y][board][x] in shared memory (see k_trunk4)
-static int make_act_map4(NetWeights* nw, CUtensorMap* map, const void* base, int cin, int rows) {
+// fp8: e4m3 elements, box {128, 10, 2, 10} (the same 128 bytes per row)
+static int make_act_map4(NetWeights* nw, CUtensorMap* map, const void* base, int cin, int rows, bool fp8 = false) {
+  const cuuint64_t es = fp8 ? 1 : 2;
   cuuint64_t dims[4] = {(cuuint64_t)cin, 8, (cuuint64_t)rows, 8};
-  cuuint64_t strides[3] = {(cuuint64_t)cin * 2, (cuuint64_t)cin * 128, (cuuint64_t)cin * 16};
-  cuuint32_t box[4] = {BLOCK_K, 10, 2, 10};
+  cuuint64_t strides[3] = {(cuuint64_t)cin * es, (cuuint64_t)cin * 64 * es, (cuuint64_t)cin * 8 * es};
+  cuuint32_t box[4] = {fp8 ? 128u : (cuuint32_t)BLOCK_K, 10, 2, 10};
   cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = nw->encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
+  CUresult r = nw->encode(map, fp8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4,
+                          const_cast<void*>(base), dims, strides, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -1492,12 +1645,13 @@ static int make_act_map4(NetWeights* nw, CUtensorMap* map, const void* base, int
   return CRL_OK;
 }
 static int make_w_map(NetWeights* nw, CUtensorMap* map, const void* base, int k_total, int n_rows = TILE_N,
-                      int box_n = TILE_N) {
+                      int box_n = TILE_N, bool fp8 = false) {
   cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)n_rows};
-  cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-  cuuint32_t box[2] = {BLOCK_K, (cuuint32_t)box_n};
+  cuuint64_t strides[1] = {(cuuint64_t)k_total * (fp8 ? 1 : 2)};
+  cuuint32_t box[2] = {fp8 ? 128u : (cuuint32_t)BLOCK_K, (cuuint32_t)box_n};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = nw->encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+  CUresult r = nw->encode(map, fp8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
+                          const_cast<void*>(base), dims, strides, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -1594,6 +1748,8 @@ int net_create(crl_engine_impl* e) {
   CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 8)));
   CRL_CUDA(cudaFuncSetAttribute(k_trunk4<2, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(2, 9)));
   CRL_CUDA(cudaFuncSetAttribute(k_trunk4<2, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(2, 10)));
+  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 7, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 7)));
+  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 7, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 7)));
   {
     const char* r = getenv("CRL_T4_RING");   // tuning knob: 0 = 3/7 (default), 1 = 3/8, 2 = 2/9, 3 = 2/10
     nw->t4_ring = r ? atoi(r) : 0;
@@ -1679,6 +1835,32 @@ static inline uint16_t f2bf(float f) {   // round to nearest even
 //                               dense kernel [128][1968], bias [1968]
 //   130..139       value head: conv kernel [1][1][256][1], bias[1], BN x4 [1], dense kernel [64][256], bias[256],
 //                              dense kernel [256][1], bias[1]
+// pack indices of convolution L's kernel, bias and BatchNorm quadruple (-1: the stem has none)
+static void conv_tensors(int L, int* ik, int* ib, int* ibn) {
+  if (L == 0) {
+    *ik = 0;
+    *ib = 1;
+    *ibn = -1;
+  } else {
+    const int blk = (L - 1) / 2, second = (L - 1) % 2;
+    *ik = 2 + 12 * blk + 6 * second;
+    *ib = *ik + 1;
+    *ibn = *ik + 2;
+  }
+}
+// bias + BatchNorm folded into a per-filter scale and shift
+static void fold_bn(const float* const* w, int ib, int ibn, float* sc, float* sh) {
+  for (int o = 0; o < 256; ++o) {
+    float s = 1.f, b = w[ib][o];
+    if (ibn >= 0) {
+      s = w[ibn][o] / sqrtf(w[ibn + 3][o] + BN_EPS);
+      b = (b - w[ibn + 2][o]) * s + w[ibn + 1][o];
+    }
+    sc[o] = s;
+    sh[o] = b;
+  }
+}
+
 int net_load(crl_engine_impl* e, const float* const* w, const int64_t* sizes, int n) {
   NetWeights* nw = e->net;
   if (n != CRL_N_WEIGHT_TENSORS) {
@@ -1692,36 +1874,23 @@ int net_load(crl_engine_impl* e, const float* const* w, const int64_t* sizes, in
     }
     return true;
   };
+  nw->fp8 = false;            // a bf16 load drops the fp8 tower; crl_net_load_fp8_host builds it again
+  nw->fp8_loaded = false;
   std::vector<uint16_t> wt;
   std::vector<float> sc(256), sh(256);
   for (int L = 0; L < N_CONVS; ++L) {
     const int cin_real = L == 0 ? 127 : 256, cin = nw->cin[L];
-    int ik, ib, ibn = -1;
-    if (L == 0) {
-      ik = 0;
-      ib = 1;
-    } else {
-      const int blk = (L - 1) / 2, second = (L - 1) % 2;
-      ik = 2 + 12 * blk + 6 * second;
-      ib = ik + 1;
-      ibn = ik + 2;
-    }
+    int ik, ib, ibn;
+    conv_tensors(L, &ik, &ib, &ibn);
     if (!need(ik, (int64_t)9 * cin_real * 256) || !need(ib, 256)) return CRL_EINVAL;
+    if (ibn >= 0 && (!need(ibn, 256) || !need(ibn + 1, 256) || !need(ibn + 2, 256) || !need(ibn + 3, 256)))
+      return CRL_EINVAL;
     wt.assign((size_t)256 * 9 * cin, 0);
     for (int t = 0; t < 9; ++t)
       for (int c = 0; c < cin_real; ++c)
         for (int o = 0; o < 256; ++o)
           wt[(size_t)o * 9 * cin + t * cin + c] = f2bf(w[ik][((size_t)t * cin_real + c) * 256 + o]);
-    for (int o = 0; o < 256; ++o) {
-      float s = 1.f, b = w[ib][o];
-      if (ibn >= 0) {
-        if (!need(ibn, 256) || !need(ibn + 1, 256) || !need(ibn + 2, 256) || !need(ibn + 3, 256)) return CRL_EINVAL;
-        s = w[ibn][o] / sqrtf(w[ibn + 3][o] + BN_EPS);
-        b = (b - w[ibn + 2][o]) * s + w[ibn + 1][o];
-      }
-      sc[o] = s;
-      sh[o] = b;
-    }
+    fold_bn(w, ib, ibn, sc.data(), sh.data());
     CRL_CUDA(cudaMemcpyAsync(nw->w[L], wt.data(), wt.size() * 2, cudaMemcpyHostToDevice, e->stream));
     CRL_CUDA(cudaMemcpyAsync(nw->scale[L], sc.data(), 1024, cudaMemcpyHostToDevice, e->stream));
     CRL_CUDA(cudaMemcpyAsync(nw->shift[L], sh.data(), 1024, cudaMemcpyHostToDevice, e->stream));
@@ -1891,15 +2060,33 @@ int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, con
     set_error("crl_net_forward: %d positions exceed the engine capacity %d", n_host, nw->cap_rows);
     return CRL_EINVAL;
   }
+  const bool fp8 = nw->fp8;
+  if (fp8 && planes != e->d_planes) {
+    // a caller's bf16 planes: converted into the engine's planes buffer, where the search encodes its e4m3 rows
+    const long long n8 = (long long)n_host * 64 * 128 / 8;     // groups of 8 values
+    LaunchScope ls(e, KC_ENCODE);
+    k_planes_to_e4m3<<<(unsigned)div_up(n8, 256), 256, 0, e->stream>>>(reinterpret_cast<const uint4*>(planes),
+                                                                         reinterpret_cast<uint2*>(e->d_planes), n8);
+    CRL_CUDA(cudaGetLastError());
+    planes = e->d_planes;
+  }
   {
-    // the box may start at row n-1 for an odd n: rows beyond the map are zero-filled by the TMA unit
-    const int rows = planes == e->d_planes ? e->R : n_host;
-    if (planes != nw->planes_ptr || rows != nw->planes_rows) {
-      int rc = make_act_map(nw, &nw->map_planes, planes, 128, rows);
-      if (rc) return rc;
-      if ((rc = make_act_map4(nw, &nw->map_planes4, planes, 128, rows))) return rc;
+    // the box may start at row n-1 for an odd n: rows beyond the map are zero-filled by the TMA unit.  e4m3 planes in
+    // e->d_planes: the buffer holds R + 2 bf16 rows, so every row a caller may convert into it is inside the map; the
+    // rows after the batch are then stale buffer contents, not zeros.  That is harmless: an output row of the implicit
+    // GEMM depends on its own board's rows only, and the epilogue skips the boards at or after the row count.
+    const int rows = fp8 ? e->R + 2 : planes == e->d_planes ? e->R : n_host;
+    if (planes != nw->planes_ptr || rows != nw->planes_rows || fp8 != nw->planes_fp8) {
+      int rc;
+      if (fp8) {
+        if ((rc = make_act_map4(nw, &nw->map_planes4, planes, 128, rows, true))) return rc;
+      } else {
+        if ((rc = make_act_map(nw, &nw->map_planes, planes, 128, rows))) return rc;
+        if ((rc = make_act_map4(nw, &nw->map_planes4, planes, 128, rows))) return rc;
+      }
       nw->planes_ptr = planes;
       nw->planes_rows = rows;
+      nw->planes_fp8 = fp8;
     }
   }
   int rc;
@@ -1926,7 +2113,14 @@ int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, con
     if (single) pairs = tiles < 1 ? 1 : tiles;
     {
       LaunchScope ls(e, KC_CONV);
-      if (single) {
+      if (fp8) {
+        if (single)
+          k_trunk4<3, 7, true, true><<<dim3(2 * pairs), dim3(CONV_THREADS), t4_smem_bytes(3, 7), e->stream>>>(
+              nw->map_planes4, nw->d_maps8, nw->d_layers8, tp);
+        else
+          k_trunk4<3, 7, false, true><<<dim3(2 * pairs), dim3(CONV_THREADS), t4_smem_bytes(3, 7), e->stream>>>(
+              nw->map_planes4, nw->d_maps8, nw->d_layers8, tp);
+      } else if (single) {
         k_trunk4<3, 7, true><<<dim3(2 * pairs), dim3(CONV_THREADS), t4_smem_bytes(3, 7), e->stream>>>(nw->map_planes4, nw->d_maps4,
                                                                                                   nw->d_layers4, tp);
       } else if (nw->use_trunk4) {
@@ -2024,6 +2218,191 @@ int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int 
                                cudaMemcpyDeviceToDevice, e->stream));
   if (pf_out) CRL_CUDA(cudaMemcpyAsync(pf_out, nw->pf, (size_t)n * 128 * 2, cudaMemcpyDeviceToDevice, e->stream));
   if (vf_out) CRL_CUDA(cudaMemcpyAsync(vf_out, nw->vf, (size_t)n * 64 * 4, cudaMemcpyDeviceToDevice, e->stream));
+  return CRL_OK;
+}
+
+// ======================================================================================================
+// fp8 evaluation: calibration, quantised weight pack, precision switch (DESIGN.md section 3.1, row a7)
+// ======================================================================================================
+bool net_fp8(const crl_engine_impl* e) { return e->net && e->net->fp8; }
+
+// the fp8 tower exists as k_trunk4<3, 7> (two tiles and single tile) only
+static int fp8_tower_available(const NetWeights* nw, const char* fn) {
+  if (!nw->use_trunk4 || nw->t4_ring != 0 || nw->probe_nsplit) {
+    set_error("%s: the fp8 tower is k_trunk4<3, 7> only; CRL_NO_TRUNK / CRL_TRUNK_V3 / CRL_CONV_V1 / CRL_T4_RING / "
+              "CRL_T4_NSPLIT_PROBE select another tower",
+              fn);
+    return CRL_ESTATE;
+  }
+  return CRL_OK;
+}
+
+// activation scale of one layer: the power of two 2^ceil(log2(amax / 448)), 1 for amax = 0
+static float act_scale(float amax) {
+  const float r = amax / 448.f;
+  if (!(r > 0.f)) return 1.f;
+  int ex;
+  const float m = frexpf(r, &ex);   // r = m * 2^ex, m in [0.5, 1)
+  return ldexpf(1.f, m == 0.5f ? ex - 1 : ex);
+}
+
+int net_calibrate(crl_engine_impl* e, const __nv_bfloat16* planes, int n, float* amax_host) {
+  NetWeights* nw = e->net;
+  if (!nw || !nw->loaded) {
+    set_error("crl_net_calibrate_host: network weights are not loaded");
+    return CRL_ESTATE;
+  }
+  if (!nw->use_trunk4) {
+    set_error("crl_net_calibrate_host: the tap exists in the v4 tower kernel only");
+    return CRL_ESTATE;
+  }
+  if (n <= 0 || n > nw->cap_rows) {
+    set_error("crl_net_calibrate_host: %d positions (1..%d)", n, nw->cap_rows);
+    return CRL_EINVAL;
+  }
+  const size_t n_act = (size_t)n * 64 * 256;
+  void* buf = nullptr;
+  CRL_CUDA(cudaMalloc(&buf, n_act * 2 + (size_t)n * (CRL_N_LABELS + 1) * 4 + N_CONVS * 4));
+  __nv_bfloat16* act = (__nv_bfloat16*)buf;
+  float* policy = (float*)(act + n_act);
+  float* value = policy + (size_t)n * CRL_N_LABELS;
+  unsigned* amax = (unsigned*)(value + n);
+  const bool was_fp8 = nw->fp8;
+  nw->fp8 = false;                    // calibration measures the bf16 tower
+  int rc = CRL_OK;
+  cudaError_t ce = cudaMemsetAsync(amax, 0, N_CONVS * 4, e->stream);
+  for (int L = 0; L < N_CONVS && rc == CRL_OK && ce == cudaSuccess; ++L) {
+    rc = net_forward(e, planes, n, nullptr, policy, value, act, L);
+    if (rc == CRL_OK) {
+      const long long n8 = (long long)n_act / 8;
+      k_absmax_bf16<<<(unsigned)std::min<long long>(div_up(n8, 256), 4 * nw->n_sms), 256, 0, e->stream>>>(
+          reinterpret_cast<const uint4*>(act), n8, amax + L);
+      ce = cudaGetLastError();
+    }
+  }
+  if (rc == CRL_OK && ce == cudaSuccess) ce = cudaMemcpyAsync(amax_host, amax, N_CONVS * 4, cudaMemcpyDeviceToHost, e->stream);
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+  nw->fp8 = was_fp8;
+  cudaFree(buf);
+  if (rc != CRL_OK) return rc;
+  if (ce != cudaSuccess) return cuda_fail(ce, "crl_net_calibrate_host");
+  return CRL_OK;
+}
+
+int net_load_fp8(crl_engine_impl* e, const float* const* w, const int64_t* sizes, int n, const float* act_amax) {
+  NetWeights* nw = e->net;
+  nw->fp8 = false;                                     // whatever fails below, the engine is left in bf16
+  int rc = fp8_tower_available(nw, "crl_net_load_fp8_host");
+  if (rc) return rc;
+  for (int L = 0; L < N_CONVS; ++L) {
+    if (!(act_amax[L] >= 0.f) || !isfinite(act_amax[L])) {
+      set_error("crl_net_load_fp8_host: activation amax %d is %g (must be finite and >= 0)", L, (double)act_amax[L]);
+      return CRL_EINVAL;
+    }
+  }
+  if ((rc = net_load(e, w, sizes, n))) return rc;      // validates the pack, loads the bf16 tower, drops fp8 state
+  if (!nw->act8[0]) {
+    for (int L = 0; L < N_CONVS; ++L) {
+      if ((rc = dev_alloc(e, &nw->w8[L], (size_t)TILE_N * 9 * nw->cin[L]))) return rc;
+      if ((rc = dev_alloc(e, &nw->scale8[L], 256))) return rc;
+      if ((rc = dev_alloc(e, &nw->shift8[L], 256))) return rc;
+    }
+    for (int i = 0; i < 2; ++i) {
+      if ((rc = dev_alloc(e, &nw->act8[i], (size_t)nw->act4_rows * 64 * 256))) return rc;
+      CRL_CUDA(cudaMemsetAsync(nw->act8[i], 0, (size_t)nw->act4_rows * 64 * 256, e->stream));
+    }
+    if ((rc = dev_alloc(e, &nw->d_maps8, 3 + N_CONVS))) return rc;
+    if ((rc = dev_alloc(e, &nw->d_layers8, N_CONVS))) return rc;
+    std::vector<CUtensorMap> hm(3 + N_CONVS);
+    memset(hm.data(), 0, hm.size() * sizeof(CUtensorMap));
+    for (int i = 0; i < 2; ++i)
+      if ((rc = make_act_map4(nw, &hm[1 + i], nw->act8[i], 256, nw->act4_rows, true))) return rc;
+    for (int L = 0; L < N_CONVS; ++L)
+      if ((rc = make_w_map(nw, &hm[3 + L], nw->w8[L], 9 * nw->cin[L], TILE_N, 128, true))) return rc;
+    CRL_CUDA(cudaMemcpyAsync(nw->d_maps8, hm.data(), hm.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice, e->stream));
+    CRL_CUDA(cudaStreamSynchronize(e->stream));
+  }
+  float s_act[N_CONVS];
+  for (int L = 0; L < N_CONVS; ++L) s_act[L] = act_scale(act_amax[L]);
+  std::vector<uint8_t> wq;
+  std::vector<float> sc(256), sh(256), ws(256);
+  std::vector<LayerDesc8> hl(N_CONVS);
+  for (int L = 0; L < N_CONVS; ++L) {
+    const int cin_real = L == 0 ? 127 : 256, cin = nw->cin[L];
+    int ik, ib, ibn;
+    conv_tensors(L, &ik, &ib, &ibn);
+    const float* k = w[ik];
+    // per output channel: ws = max_k |W| / 448 (1 for an all-zero column), Wq = e4m3(W / ws)
+    for (int o = 0; o < 256; ++o) {
+      float m = 0.f;
+      for (int t = 0; t < 9 * cin_real; ++t) m = fmaxf(m, fabsf(k[(size_t)t * 256 + o]));
+      ws[o] = m > 0.f ? m / 448.f : 1.f;
+    }
+    wq.assign((size_t)256 * 9 * cin, 0);
+    for (int t = 0; t < 9; ++t)
+      for (int c = 0; c < cin_real; ++c)
+        for (int o = 0; o < 256; ++o)
+          wq[(size_t)o * 9 * cin + t * cin + c] =
+              __nv_cvt_float_to_fp8(k[((size_t)t * cin_real + c) * 256 + o] / ws[o], __NV_SATFINITE, __NV_E4M3);
+    fold_bn(w, ib, ibn, sc.data(), sh.data());
+    const float s_in = L == 0 ? 1.f : s_act[L - 1];
+    for (int o = 0; o < 256; ++o) sc[o] = ws[o] * s_in * sc[o];
+    CRL_CUDA(cudaMemcpyAsync(nw->w8[L], wq.data(), wq.size(), cudaMemcpyHostToDevice, e->stream));
+    CRL_CUDA(cudaMemcpyAsync(nw->scale8[L], sc.data(), 1024, cudaMemcpyHostToDevice, e->stream));
+    CRL_CUDA(cudaMemcpyAsync(nw->shift8[L], sh.data(), 1024, cudaMemcpyHostToDevice, e->stream));
+    CRL_CUDA(cudaStreamSynchronize(e->stream));
+    // the same dataflow as the bf16 v4 tower's layer table (net_create), on the e4m3 scratch
+    LayerDesc8& d = hl[L];
+    memset(&d, 0, sizeof(d));
+    d.map_w = 3 + L;
+    d.k_chunks = cin / 128;
+    d.scale = nw->scale8[L];
+    d.shift = nw->shift8[L];
+    d.s_out = s_act[L];
+    d.inv_out = 1.f / s_act[L];
+    if (L == 0) {
+      d.map_in = 0;
+      d.out = nw->act8[0];
+      d.write_out = 1;
+    } else if ((L - 1) % 2 == 0) {
+      d.map_in = 1;
+      d.out = nw->act8[1];
+      d.relu = 1;
+      d.write_out = 1;
+    } else {
+      d.map_in = 2;
+      d.out = nw->act8[0];
+      d.residual = nw->act8[0];
+      d.s_res = s_act[L - 2];       // the block input: the stem's or the previous block's output
+      d.relu = 1;
+      d.write_out = L != N_CONVS - 1;
+      d.fuse_heads = L == N_CONVS - 1;
+    }
+  }
+  CRL_CUDA(cudaMemcpyAsync(nw->d_layers8, hl.data(), hl.size() * sizeof(LayerDesc8), cudaMemcpyHostToDevice, e->stream));
+  CRL_CUDA(cudaStreamSynchronize(e->stream));
+  nw->fp8_loaded = true;
+  nw->fp8 = true;
+  return CRL_OK;
+}
+
+int net_set_precision(crl_engine_impl* e, int precision) {
+  NetWeights* nw = e->net;
+  if (precision == CRL_NET_BF16) {
+    nw->fp8 = false;
+    return CRL_OK;
+  }
+  if (precision != CRL_NET_FP8) {
+    set_error("crl_net_set_precision: unknown precision %d", precision);
+    return CRL_EINVAL;
+  }
+  int rc = fp8_tower_available(nw, "crl_net_set_precision");
+  if (rc) return rc;
+  if (!nw->fp8_loaded) {
+    set_error("crl_net_set_precision: no fp8 weights (crl_net_load_fp8_host)");
+    return CRL_ESTATE;
+  }
+  nw->fp8 = true;
   return CRL_OK;
 }
 

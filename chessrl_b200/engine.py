@@ -46,6 +46,7 @@ class Engine:
                                          int(avg_moves), self.max_inflight, vp(stream)))
         self.h = h
         self.weights_loaded = False
+        self.net_precision = "bf16"
 
     def close(self):
         if getattr(self, "h", None):
@@ -170,14 +171,55 @@ class Engine:
         return t.reshape(5, 64, 64)
 
     # ---- network ------------------------------------------------------------------------------------------
-    def load_weights(self, tensors):
-        """tensors: the 140-array weight pack (chessrl_b200.model.ChessModel.weights)."""
+    def load_weights(self, tensors, precision="bf16", calibration=None):
+        """tensors: the 140-array weight pack (chessrl_b200.model.ChessModel.weights).
+        precision="fp8" also builds the e4m3 tower (include/chessrl_b200.h crl_net_load_fp8_host) and selects it; its
+        activation scales come from `calibration`: 21 per-layer amax values (Engine.calibrate), bf16 planes
+        [n,8,8,128] to calibrate on, or None for model.calibration_planes(self)."""
+        if precision not in ("bf16", "fp8"):
+            raise ValueError("precision must be 'bf16' or 'fp8', not %r" % (precision,))
         arrs = [np.ascontiguousarray(np.asarray(t, dtype=np.float32).reshape(-1)) for t in tensors]
         n = len(arrs)
         ptrs = (_lib.c_f32p * n)(*[a.ctypes.data_as(_lib.c_f32p) for a in arrs])
         sizes = (ctypes.c_int64 * n)(*[a.size for a in arrs])
-        check(self.lib.crl_net_load_host(self.h, ptrs, sizes, n))
-        self.weights_loaded = True
+        if precision == "bf16" or calibration is None or torch.is_tensor(calibration):
+            # the bf16 tower; for fp8 it is also what calibrates (crl_net_load_fp8_host loads it again below)
+            self.net_precision = "bf16"
+            check(self.lib.crl_net_load_host(self.h, ptrs, sizes, n))
+            self.weights_loaded = True
+        if precision == "fp8":
+            if calibration is None:
+                from .model import calibration_planes
+                calibration = calibration_planes(self)
+            if torch.is_tensor(calibration):
+                calibration = self.calibrate(calibration)
+            amax = np.ascontiguousarray(np.asarray(calibration, dtype=np.float32).reshape(-1))
+            if amax.size != 21:
+                raise ValueError("calibration: 21 per-layer amax values expected, got %d" % amax.size)
+            self.net_precision = "bf16"                  # what a failed fp8 load leaves the engine in
+            check(self.lib.crl_net_load_fp8_host(self.h, ptrs, sizes, n, amax.ctypes.data_as(_lib.c_f32p)))
+            self.weights_loaded = True
+        self.net_precision = precision
+
+    def calibrate(self, planes_t):
+        """max |output| of each of the 21 tower convolutions over bf16 planes [n,8,8,128], from the bf16 tower
+        -> float32 [21] (the `calibration` of load_weights(precision="fp8"))."""
+        amax = np.zeros(21, dtype=np.float32)
+        part = np.zeros(21, dtype=np.float32)
+        step = self.max_games * self.max_inflight          # rows the engine's buffers hold
+        for i in range(0, planes_t.shape[0], step):
+            x = planes_t[i:i + step]
+            check(self.lib.crl_net_calibrate_host(self.h, _ptr(x), x.shape[0], part.ctypes.data_as(_lib.c_f32p)))
+            amax = np.maximum(amax, part)
+        return amax
+
+    def set_net_precision(self, precision):
+        """'bf16' or 'fp8' (the latter needs a load_weights(..., precision="fp8") since the last bf16 load)."""
+        code = {"bf16": _lib.NET_BF16, "fp8": _lib.NET_FP8}.get(precision)
+        if code is None:
+            raise ValueError("precision must be 'bf16' or 'fp8', not %r" % (precision,))
+        check(self.lib.crl_net_set_precision(self.h, code))
+        self.net_precision = precision
 
     def net_forward(self, planes_t):
         n = planes_t.shape[0]

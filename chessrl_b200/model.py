@@ -77,6 +77,34 @@ def random_pack(seed=0, perturb_bn=False):
     return out
 
 
+def calibration_planes(engine, n=256, seed=0, max_plies=80):
+    """The default fp8 calibration set (Engine.load_weights(precision="fp8")): bf16 planes [n,8,8,128] of `n` positions
+    reached by seeded uniformly random legal playouts of 0..max_plies plies from the start position, encoded with their
+    history like netencoder.get_game_state.  Depends only on (n, seed, max_plies)."""
+    import torch
+    from . import boards as B
+    rng = np.random.default_rng(seed)
+    start = B.record_from_fen()
+    cur = np.zeros((9, n), dtype=np.uint64)
+    hist = np.zeros((8, 8, n), dtype=np.uint64)
+    hist_len = np.zeros(n, dtype=np.uint8)
+    for i in range(n):
+        target = int(rng.integers(0, max_plies + 1))
+        moves = []
+        r = engine.game_replay(start, moves, records=True)
+        while len(moves) < target and r["result"] is None and len(r["legal"]):
+            moves.append(int(r["legal"][int(rng.integers(0, len(r["legal"])))]))
+            r = engine.game_replay(start, moves, records=True)
+        recs = r["records"][::-1][:9]
+        cur[:, i] = recs[0]
+        for j, rec in enumerate(recs[1:]):
+            hist[j, :, i] = rec[:8]
+        hist_len[i] = len(recs) - 1
+    dev = engine.device
+    return engine.encode(torch.from_numpy(cur.view(np.int64)).to(dev), torch.from_numpy(hist.view(np.int64)).to(dev),
+                         torch.from_numpy(hist_len).to(dev))
+
+
 class ChessModel(object):
     """Same constructor surface as the reference (model.py:17): ChessModel(compile_model=True, weights=None)."""
 

@@ -91,7 +91,7 @@ class LockstepRun:
     """
 
     def __init__(self, model, n_games, sims=900, lanes=None, noise=True, device=None, seed=None, max_moves=None,
-                 threads=1, evaluator=None, engine=None, reuse=True):
+                 threads=1, evaluator=None, engine=None, reuse=True, net_precision="bf16"):
         import time
         from ._lib import EVAL_HASH, EVAL_NET
         from .engine import Engine
@@ -110,7 +110,9 @@ class LockstepRun:
             avg_moves=edge_slots_per_node(lanes, sims + 1, device, bytes_per_edge=32 if reuse and threads == 1 else 24))
         if evaluator is None:
             if model is not None:
-                self.eng.load_weights(model.weights)
+                self.eng.load_weights(model.weights, precision=net_precision)
+            elif net_precision != "bf16":
+                self.eng.set_net_precision(net_precision)
             self.eng.set_evaluator(EVAL_NET)
         else:
             self.eng.set_evaluator(EVAL_HASH, int(evaluator[1]), int(evaluator[2]))
@@ -197,16 +199,17 @@ class LockstepRun:
 
 
 def play_games_lockstep(model, n_games, sims=900, lanes=None, noise=True, device=None, seed=None, max_moves=None,
-                        threads=1, evaluator=None, stats=None, reuse=True):
+                        threads=1, evaluator=None, stats=None, reuse=True, net_precision="bf16"):
     """`n_games` games in lockstep, `lanes` at a time; returns a DatasetGame in game-start order.
 
     The per-move host work is the numpy move policy only.  max_moves caps the agent moves of a game (it is then stored
     unfinished, result None).  evaluator: None = the network with `model`'s weights; ("hash", seed, bits) = the
     deterministic test evaluator.  stats: optional dict that receives steps / moves / simulations / seconds / lane
     occupancy of the run.  reuse: take evaluations from the previous move's tree where it holds the same node (same
-    games either way; include/chessrl_b200.h crl_set_reuse)."""
+    games either way; include/chessrl_b200.h crl_set_reuse).  net_precision: "bf16" (default) or "fp8", the opt-in e4m3
+    tower calibrated on model.calibration_planes (DESIGN.md section 3.1; not bit-exact with bf16)."""
     run = LockstepRun(model, n_games, sims=sims, lanes=lanes, noise=noise, device=device, seed=seed, max_moves=max_moves,
-                      threads=threads, evaluator=evaluator, reuse=reuse)
+                      threads=threads, evaluator=evaluator, reuse=reuse, net_precision=net_precision)
     try:
         while run.advance():
             pass
@@ -234,6 +237,9 @@ def main(argv=None):
                              "search are reused; the games are identical either way)")
     parser.add_argument('--precision', choices=("fp32", "tf32", "bf16"), default=None,
                         help="arithmetic of the training step (default fp32 = the parity setting; see chessrl_b200/training.py)")
+    parser.add_argument('--net-precision', choices=("bf16", "fp8"), default="bf16",
+                        help="arithmetic of the network's residual tower during self-play (default bf16; fp8 = e4m3 "
+                             "tensor cores with calibrated scales, faster but not bit-exact: DESIGN.md section 3.1)")
     args = parser.parse_args(argv)
     if args.precision:
         os.environ["CRL_TRAIN_PRECISION"] = args.precision
@@ -259,7 +265,7 @@ def main(argv=None):
     lanes = args.lanes if args.lanes is not None else default_lanes(share)
     data = (play_games_lockstep(agent.model, share, sims=args.sims, lanes=lanes, device=local_rank,
                                 threads=args.threads, max_moves=args.max_moves, stats=stats,
-                                reuse=not args.no_reuse) if share else DatasetGame())
+                                reuse=not args.no_reuse, net_precision=args.net_precision) if share else DatasetGame())
     if stats:
         full = max(1, stats["steps"] * stats["lanes"] * args.sims)
         logger.info("rank %d: %d games, %d agent moves in %d lockstep steps, %.1f s: %.0f simulations/s, lane occupancy %.1f %%"

@@ -162,6 +162,25 @@ int crl_debug_tower(crl_engine* e, const void* planes_bf16_dev, int n, int layer
  * evaluated and only those rows of policy_dev [n_bound][1968] / value_dev [n_bound] are written */
 int crl_debug_forward_counted(crl_engine* e, const void* planes_bf16_dev, int n_bound, const int32_t* n_dev,
                               float* policy_dev, float* value_dev);
+/* Opt-in fp8 evaluation.  The 21 tower convolutions run on e4m3 operands (tcgen05 kind::f8f6f4, fp32 accumulation):
+ * planes exactly, weights per output channel scaled to max |W| = 448, each layer's output (but the last, which feeds
+ * the bf16 heads) as e4m3 x a power-of-two scale 2^ceil(log2(amax / 448)) from calibration.  Heads, softmax and search
+ * are unchanged.  Not bit-exact with bf16; DESIGN.md section 3.1 states the definition and the measured deviation.
+ *   crl_net_calibrate_host : runs the bf16 tower on planes_bf16_dev [n][8][8][128] and writes max |output| of each
+ *                            convolution to amax_host [21]
+ *   crl_net_load_fp8_host  : crl_net_load_host, then the fp8 tower from the same pack and act_amax_host [21] (finite,
+ *                            >= 0, else CRL_EINVAL); selects fp8.  On any error the engine is left in bf16.
+ *   crl_net_set_precision  : CRL_NET_BF16 or CRL_NET_FP8 (CRL_ESTATE without an fp8 load).  crl_net_load_host returns
+ *                            the engine to bf16 and drops the fp8 tower.
+ * fp8 exists in the default tower only: with CRL_NO_TRUNK, CRL_TRUNK_V3, CRL_CONV_V1, CRL_T4_RING != 0 or
+ * CRL_T4_NSPLIT_PROBE set at crl_create, selecting it returns CRL_ESTATE.  In fp8 mode crl_net_forward,
+ * crl_debug_tower and crl_debug_forward_counted take bf16 planes as before and convert them. */
+#define CRL_NET_BF16 0
+#define CRL_NET_FP8 1
+int crl_net_calibrate_host(crl_engine* e, const void* planes_bf16_dev, int n, float* amax_host);
+int crl_net_load_fp8_host(crl_engine* e, const float* const* weights_host, const int64_t* sizes, int n_tensors,
+                          const float* act_amax_host);
+int crl_net_set_precision(crl_engine* e, int precision);
 /* the deterministic test evaluator on raw boards (SoA), same outputs as the oracle's hash_evaluator */
 int crl_hash_eval(crl_engine* e, const uint64_t* boards_dev, int n, uint64_t seed, int policy_bits,
                   float* policy_dev, float* value_dev);

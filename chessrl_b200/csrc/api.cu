@@ -99,6 +99,27 @@ static int ensure_stage(crl_engine_impl* e, size_t bytes) {
   return CRL_OK;
 }
 
+// The slots a search routes rows to: slot 1 joins while some lane names it as a player (DESIGN.md 3.5)
+static int route_slots(crl_engine_impl* e, const char* fn) {
+  const int slots = e->lanes_on_slot1 > 0 ? 2 : 1;
+  if (slots > 1) {
+    if (!e->slot_configured[1]) {
+      set_error("%s: %d lanes name network slot 1 as a player, but slot 1 has no evaluator (crl_net_select_slot, then "
+                "crl_net_load_host or crl_set_evaluator)", fn, e->lanes_on_slot1);
+      return CRL_ESTATE;
+    }
+    if (e->eval_kind[0] != e->eval_kind[1]) {
+      set_error("%s: the network slots hold evaluators of different kinds (hash and network); one search reads both "
+                "through one policy view", fn);
+      return CRL_ESTATE;
+    }
+  }
+  e->search_slots = slots;
+  e->P.n_slots = slots;
+  e->P.slot_stride = (int)e->slot_stride;
+  return CRL_OK;
+}
+
 static int check_pool_errors(crl_engine_impl* e) {
   int err = 0;
   CRL_CUDA(cudaMemcpyAsync(&err, e->P.err, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
@@ -149,6 +170,12 @@ __global__ void k_root_stats(Pools P, int* visits, double* values, float* priors
       if (results) results[o] = RESULT_NONE;
     }
   }
+}
+
+// lanes whose players changed: the previous tree was searched by another network, nothing of it is reused
+__global__ void k_unlink_lanes(Pools P, int first, int n, const u8* changed) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n && changed[i]) P.g_prev_root[first + i] = -1;
 }
 
 __global__ void k_node_dump(Pools P, int g, crl_node_host* out, int cap) {
@@ -303,7 +330,7 @@ int crl_create_ex(crl_engine** out, int device, int max_games, int max_nodes, in
 #undef A
   if (rc == CRL_OK) rc = pool_alloc(e, &e->d_list[0], R);
   if (rc == CRL_OK) rc = pool_alloc(e, &e->d_list[1], R);
-  if (rc == CRL_OK) rc = pool_alloc(e, &e->d_n, 4);
+  if (rc == CRL_OK) rc = pool_alloc(e, &e->d_n, 2 * SLOT_N_STRIDE);
   if (rc == CRL_OK) rc = pool_alloc(e, &e->d_tmp_moves, 2 * G);
   if (rc == CRL_OK) rc = pool_alloc(e, &e->d_tmp_pick, G);
   if (rc == CRL_OK) rc = pool_alloc(e, &e->d_planes, (R + 2) * 64 * 128);
@@ -314,6 +341,7 @@ int crl_create_ex(crl_engine** out, int device, int max_games, int max_nodes, in
   if (rc == CRL_OK) {
     P.eval_list = e->d_list[0];
     P.eval_n = e->d_n;
+    P.n_slots = 1;
     build_label_table(e->h_label_of);
     cudaError_t ce = cudaMemcpyAsync(e->d_label_of, e->h_label_of.data(), 5 * 4096 * sizeof(int16_t),
                                      cudaMemcpyHostToDevice, e->stream);
@@ -323,7 +351,7 @@ int crl_create_ex(crl_engine** out, int device, int max_games, int max_nodes, in
     cudaError_t ce = cudaMemsetAsync(P.g_prev_root, 0xFF, sizeof(int) * G, e->stream);
     if (ce != cudaSuccess) rc = cuda_fail(ce, "g_prev_root init");
   }
-  if (rc == CRL_OK) rc = net_create(e);
+  if (rc == CRL_OK) rc = net_create(e, 0);
   if (rc == CRL_OK) {
     cudaError_t ce = cudaStreamSynchronize(e->stream);
     if (ce != cudaSuccess) rc = cuda_fail(ce, "crl_create sync");
@@ -567,13 +595,35 @@ int crl_label_table_host(crl_engine* e, int16_t* idx_host) {
 }
 
 // ---- network -----------------------------------------------------------------------------------------
+int crl_net_select_slot(crl_engine* e, int slot) {
+  CHECK_ENGINE(e);
+  if (slot < 0 || slot >= CRL_NET_SLOTS) {
+    set_error("crl_net_select_slot: slot %d (0..%d)", slot, CRL_NET_SLOTS - 1);
+    return CRL_EINVAL;
+  }
+  e->sel_slot = slot;
+  e->net = e->nets[slot];
+  return CRL_OK;
+}
+
+// the selected slot gets what a configuration needs: slot 1 its rows in the result buffers, and its network when
+// weights are loaded into it (slot 0 has both from crl_create)
+static int configure_slot(crl_engine_impl* e, bool with_net) {
+  if (e->sel_slot == 0) return CRL_OK;
+  if (with_net) return net_slot_ensure(e, e->sel_slot);
+  return net_two_slot_layout(e);
+}
+
 int crl_net_load_host(crl_engine* e, const float* const* weights_host, const int64_t* sizes, int n_tensors) {
   CHECK_ENGINE(e);
   if (!weights_host || !sizes) {
     set_error("crl_net_load_host: null arguments");
     return CRL_EINVAL;
   }
-  return net_load(e, weights_host, sizes, n_tensors);
+  int rc = configure_slot(e, true);
+  if (rc == CRL_OK) rc = net_load(e, weights_host, sizes, n_tensors);
+  if (rc == CRL_OK) e->slot_configured[e->sel_slot] = true;
+  return rc;
 }
 int crl_net_forward(crl_engine* e, const void* planes_bf16_dev, int n, float* policy_dev, float* value_dev) {
   CHECK_ENGINE(e);
@@ -625,7 +675,10 @@ int crl_net_load_fp8_host(crl_engine* e, const float* const* weights_host, const
     set_error("crl_net_load_fp8_host: null arguments");
     return CRL_EINVAL;
   }
-  return net_load_fp8(e, weights_host, sizes, n_tensors, act_amax_host);
+  int rc = configure_slot(e, true);
+  if (rc == CRL_OK) rc = net_load_fp8(e, weights_host, sizes, n_tensors, act_amax_host);
+  if (rc == CRL_OK) e->slot_configured[e->sel_slot] = true;
+  return rc;
 }
 int crl_net_set_precision(crl_engine* e, int precision) {
   CHECK_ENGINE(e);
@@ -648,9 +701,64 @@ int crl_set_evaluator(crl_engine* e, int kind, uint64_t seed, int policy_bits) {
     set_error("crl_set_evaluator: bad arguments");
     return CRL_EINVAL;
   }
-  e->eval_kind = kind;
-  e->eval_seed = seed;
-  e->eval_bits = policy_bits;
+  int rc = configure_slot(e, false);
+  if (rc) return rc;
+  const int k = e->sel_slot;
+  e->eval_kind[k] = kind;
+  e->eval_seed[k] = seed;
+  e->eval_bits[k] = policy_bits;
+  e->slot_configured[k] = true;
+  return CRL_OK;
+}
+
+int crl_games_set_players_host(crl_engine* e, int first, int n, const uint8_t* white_slot_host,
+                               const uint8_t* black_slot_host) {
+  CHECK_ENGINE(e);
+  if (first < 0 || n <= 0 || first + n > e->G || !white_slot_host || !black_slot_host) {
+    set_error("crl_games_set_players_host: bad arguments (first %d, n %d, capacity %d)", first, n, e->G);
+    return CRL_EINVAL;
+  }
+  for (int i = 0; i < n; ++i)
+    if (white_slot_host[i] >= CRL_NET_SLOTS || black_slot_host[i] >= CRL_NET_SLOTS) {
+      set_error("crl_games_set_players_host: lane %d names slot %d / %d (0..%d)", first + i, white_slot_host[i],
+                black_slot_host[i], CRL_NET_SLOTS - 1);
+      return CRL_EINVAL;
+    }
+  const size_t G = e->G;
+  if (e->h_players.empty()) {        // the first call: the device copy and the per-lane searching slot
+    u8* players = nullptr;
+    int rc = pool_alloc(e, &players, 2 * G);
+    if (rc == CRL_OK) rc = pool_alloc(e, &e->P.g_slot, G);
+    if (rc) return rc;
+    e->P.g_players = players;
+    e->h_players.assign(2 * G, 0);
+  }
+  // staging: [white n][black n][changed n]; a lane whose players change is unlinked from its previous tree
+  int rc = ensure_stage(e, 3 * (size_t)n);
+  if (rc) return rc;
+  u8* h = (u8*)e->h_stage;
+  u8* d = (u8*)e->d_stage;
+  int changed = 0;
+  for (int i = 0; i < n; ++i) {
+    const size_t g = (size_t)first + i;
+    h[i] = white_slot_host[i];
+    h[n + i] = black_slot_host[i];
+    h[2 * n + i] = h[i] != e->h_players[g] || h[n + i] != e->h_players[G + g];
+    changed += h[2 * n + i];
+    e->lanes_on_slot1 += (h[i] == 1 || h[n + i] == 1) - (e->h_players[g] == 1 || e->h_players[G + g] == 1);
+    e->h_players[g] = h[i];
+    e->h_players[G + g] = h[n + i];
+  }
+  CRL_CUDA(cudaMemcpyAsync(d, h, 3 * (size_t)n, cudaMemcpyHostToDevice, e->stream));
+  CRL_CUDA(cudaMemcpyAsync((u8*)e->P.g_players + first, d, n, cudaMemcpyDeviceToDevice, e->stream));
+  CRL_CUDA(cudaMemcpyAsync((u8*)e->P.g_players + G + first, d + n, n, cudaMemcpyDeviceToDevice, e->stream));
+  if (changed) {
+    LaunchScope ls(e, KC_GAME);
+    k_unlink_lanes<<<div_up(n, 128), 128, 0, e->stream>>>(e->P, first, n, d + 2 * n);
+    CRL_CUDA(cudaGetLastError());
+    e->tree_ready = false;
+  }
+  CRL_CUDA(cudaStreamSynchronize(e->stream));   // the staging buffer is reused by the next call
   return CRL_OK;
 }
 
@@ -836,7 +944,9 @@ int crl_games_legal_host(crl_engine* e, int first, int n, uint16_t* legal_host, 
 int crl_games_policy_move_host(crl_engine* e, const uint8_t* mask_host, uint16_t* picks_host) {
   CHECK_ENGINE(e);
   const size_t G = e->G;
-  int rc = ensure_stage(e, G);
+  int rc = route_slots(e, "crl_games_policy_move_host");
+  if (rc) return rc;
+  rc = ensure_stage(e, G);
   if (rc) return rc;
   const u8* mask_dev = nullptr;
   if (mask_host) {
@@ -891,7 +1001,9 @@ int crl_reuse_count_host(crl_engine* e, int64_t* reused_host) {
 
 int crl_mcts_begin_move(crl_engine* e) {
   CHECK_ENGINE(e);
-  int rc = tree_begin_move(e, nullptr, e->reuse);
+  int rc = route_slots(e, "crl_mcts_begin_move");
+  if (rc) return rc;
+  rc = tree_begin_move(e, nullptr, e->reuse);
   if (rc) return rc;
   e->tree_ready = true;
   return CRL_OK;
@@ -912,6 +1024,8 @@ int crl_mcts_simulate(crl_engine* e, int n_sims, int inflight) {
     set_error("crl_mcts_simulate: %d simulations exceed the node pool (%d per game)", n_sims, e->NN - 1);
     return CRL_EINVAL;
   }
+  int rc = route_slots(e, "crl_mcts_simulate");
+  if (rc) return rc;
   return tree_simulate(e, n_sims, inflight);
 }
 

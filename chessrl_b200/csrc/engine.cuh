@@ -38,20 +38,29 @@ struct crl_engine_impl {
   std::vector<void*> allocs;       // everything cudaMalloc'ed
   int16_t* d_label_of = nullptr;   // [5][64][64]
   std::vector<int16_t> h_label_of;
-  // evaluator
-  int eval_kind = CRL_EVAL_NET;
-  uint64_t eval_seed = 0;
-  int eval_bits = 24;
+  // evaluator of every network slot (crl_net_select_slot picks the slot the configuration calls act on)
+  int eval_kind[CRL_NET_SLOTS] = {CRL_EVAL_NET, CRL_EVAL_NET};
+  uint64_t eval_seed[CRL_NET_SLOTS] = {0, 0};
+  int eval_bits[CRL_NET_SLOTS] = {24, 24};
+  bool slot_configured[CRL_NET_SLOTS] = {true, false};   // slot 1 has no evaluator until a load or crl_set_evaluator
+  int sel_slot = 0;
+  // two-network routing (DESIGN.md 3.5): slot k's rows of a batch are rows k * slot_stride + r of the list, policy, value
+  // and statistics buffers below (and of the logits); 0 until slot 1 is first configured, the buffers then hold 2 slots
+  long long slot_stride = 0;
+  std::vector<uint8_t> h_players;      // [2][G] host copy of the players (white slot, black slot); empty = all slot 0
+  int lanes_on_slot1 = 0;              // lanes that name slot 1 as a player
+  int search_slots = 1;                // slots the current search routes rows to (2 iff lanes_on_slot1 > 0)
   // evaluation workspaces (sized for G rows)
   __nv_bfloat16* d_planes = nullptr;   // [G][64][128]
   float* d_policy = nullptr;           // [G][1968]
   float* d_value = nullptr;            // [G]
   float* d_stats = nullptr;            // [G][2] softmax statistics (max logit, 1 / sum exp) of the rows evaluated by the network
   PolicyView pview{};                  // how the search kernels read the last evaluation batch (set by launch_eval_batch)
-  NetWeights* net = nullptr;
+  NetWeights* nets[CRL_NET_SLOTS] = {nullptr, nullptr};
+  NetWeights* net = nullptr;           // nets[sel_slot]
   bool tree_ready = false;
   int* d_list[2] = {nullptr, nullptr};   // compacted evaluation batches A (after our move) / B (leaf)
-  int* d_n = nullptr;                    // [2] their row counts
+  int* d_n = nullptr;                    // row counts: [0] / [1] batches A / B (slot 0), [2] scratch, [4] / [5] slot 1's
   u16* d_tmp_moves = nullptr;            // [2*G] scratch for picks
   int* d_tmp_pick = nullptr;             // [G]
   // device-driven perft (crl_perft_root_host): two frontier buffers of perft_cap boards + control block
@@ -147,14 +156,23 @@ int tree_policy_move(crl_engine_impl* e, const u8* mask_dev, u16* picks_dev);
 int tree_commit(crl_engine_impl* e, const int* pick_dev, u16* out_moves_dev, int apply);
 
 // net
-int net_create(crl_engine_impl* e);
+int net_create(crl_engine_impl* e, int slot);
 void net_destroy(crl_engine_impl* e);
+// the network of slot k, created with its planes buffer on first use (the result buffers must hold two slots already)
+int net_slot_ensure(crl_engine_impl* e, int slot);
+// lays the row lists and result buffers out for two slots (once, at the first configuration of slot 1)
+int net_two_slot_layout(crl_engine_impl* e);
 int net_load(crl_engine_impl* e, const float* const* w, const int64_t* sizes, int n);
 // n_dev may be null (then n_host rows); otherwise the row count is read on the device and n_host is the bound
 // view_out != null: the caller reads the policy through a PolicyView (the search kernels); where the network path allows it
 // the softmax kernel then writes only its statistics to e->d_stats and *view_out points at the logits, otherwise at `policy`
 int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, const int* n_dev, float* policy,
                 float* value, __nv_bfloat16* dbg_out = nullptr, int dbg_layer = -1, PolicyView* view_out = nullptr);
+// net_forward with the network of slot `slot` (a search batch of that slot's rows; `planes` = net_planes_buf)
+int net_forward_slot(crl_engine_impl* e, int slot, const void* planes, int n_host, const int* n_dev, float* policy,
+                     float* value, PolicyView* view_out);
+// the buffer the search encodes slot `slot`'s rows into (R + 2 bf16 rows; e4m3 rows while the slot runs fp8)
+void* net_planes_buf(const crl_engine_impl* e, int slot);
 int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int layer, __nv_bfloat16* act_out,
                     float* logits_out, __nv_bfloat16* pf_out, float* vf_out, float* policy, float* value);
 int net_debug_conv(crl_engine_impl* e, int layer, const __nv_bfloat16* in, int cin, int n, const __nv_bfloat16* residual,
@@ -163,8 +181,8 @@ int net_debug_conv(crl_engine_impl* e, int layer, const __nv_bfloat16* in, int c
 int net_calibrate(crl_engine_impl* e, const __nv_bfloat16* planes, int n, float* amax_host);
 int net_load_fp8(crl_engine_impl* e, const float* const* w, const int64_t* sizes, int n, const float* act_amax);
 int net_set_precision(crl_engine_impl* e, int precision);
-// true while the fp8 tower is selected: the search then encodes e4m3 planes into e->d_planes
-bool net_fp8(const crl_engine_impl* e);
+// true while slot `slot`'s fp8 tower is selected: the search then encodes e4m3 planes for that slot
+bool net_fp8(const crl_engine_impl* e, int slot);
 
 }  // namespace crl
 

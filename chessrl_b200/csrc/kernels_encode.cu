@@ -211,23 +211,43 @@ int launch_hash_eval_boards(crl_engine_impl* e, const u64* boards, int n, u64 se
 
 // Encodes the positions named by P.eval_list (which: 0 root, 1 state after our move, 2 node state) and runs
 // the configured evaluator on them; results land in e->d_policy / e->d_value, row r <-> game eval_list[r].
+// With two network slots in the search, each slot's share of the batch (its list and row count, at rows
+// k * slot_stride + r) is encoded in the slot's plane dtype and evaluated by the slot's evaluator; the search reads
+// both shares through slot 0's view, at their rows.
 int launch_eval_batch(crl_engine_impl* e, int which) {
-  if (e->eval_kind == CRL_EVAL_HASH) {
-    LaunchScope ls(e, KC_HASHEVAL);
-    k_hash_eval_rows<<<e->cur_rows, 256, 0, e->stream>>>(e->P, which, e->eval_seed, e->eval_bits, e->d_policy, e->d_value);
-    CRL_CUDA(cudaGetLastError());
-    e->pview = PolicyView{e->d_policy, CRL_N_LABELS, nullptr};
-    return CRL_OK;
+  for (int k = 0; k < e->search_slots; ++k) {
+    Pools P = e->P;
+    const long long off = (long long)k * e->slot_stride;
+    P.eval_list += off;
+    P.eval_n += SLOT_N_STRIDE * k;
+    float* policy = e->d_policy + off * CRL_N_LABELS;
+    float* value = e->d_value + off;
+    PolicyView view;
+    if (e->eval_kind[k] == CRL_EVAL_HASH) {
+      LaunchScope ls(e, KC_HASHEVAL);
+      k_hash_eval_rows<<<e->cur_rows, 256, 0, e->stream>>>(P, which, e->eval_seed[k], e->eval_bits[k], policy, value);
+      CRL_CUDA(cudaGetLastError());
+      view = PolicyView{e->d_policy, CRL_N_LABELS, nullptr};
+    } else {
+      void* planes = net_planes_buf(e, k);
+      if (!planes) {
+        set_error("network slot %d has no weights (crl_net_load_host)", k);
+        return CRL_ESTATE;
+      }
+      {
+        LaunchScope ls(e, KC_ENCODE);
+        if (net_fp8(e, k))   // the fp8 tower reads e4m3 rows from the same buffer
+          k_encode_rows<uint8_t><<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(P, which, (uint8_t*)planes);
+        else
+          k_encode_rows<__nv_bfloat16><<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(P, which, (__nv_bfloat16*)planes);
+        CRL_CUDA(cudaGetLastError());
+      }
+      int rc = net_forward_slot(e, k, planes, e->cur_rows, P.eval_n, policy, value, &view);
+      if (rc != CRL_OK) return rc;
+    }
+    if (k == 0) e->pview = view;
   }
-  {
-    LaunchScope ls(e, KC_ENCODE);
-    if (net_fp8(e))   // the fp8 tower reads e4m3 rows from the same buffer
-      k_encode_rows<uint8_t><<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(e->P, which, (uint8_t*)e->d_planes);
-    else
-      k_encode_rows<__nv_bfloat16><<<e->cur_rows, ENC_ROW_THREADS, 0, e->stream>>>(e->P, which, e->d_planes);
-    CRL_CUDA(cudaGetLastError());
-  }
-  return net_forward(e, e->d_planes, e->cur_rows, e->P.eval_n, e->d_policy, e->d_value, nullptr, -1, &e->pview);
+  return CRL_OK;
 }
 
 }  // namespace crl

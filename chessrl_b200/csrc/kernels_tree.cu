@@ -35,6 +35,16 @@ __device__ __forceinline__ int take_row(const Pools& P, int* counter) {
   return r;
 }
 
+// slot that searches lane g (two-network routing, DESIGN.md 3.5): the slot of the side to move at the lane's root
+__device__ __forceinline__ int lane_slot(const Pools& P, int g) { return P.n_slots > 1 ? (int)P.g_slot[g] : 0; }
+
+// a row of slot k's share of a batch: the buffer row k * slot_stride + r, which lists `item`
+__device__ __forceinline__ int take_slot_row(const Pools& P, int* list, int* counter, int k, int item) {
+  const int row = k * P.slot_stride + take_row(P, counter + SLOT_N_STRIDE * k);
+  list[row] = item;
+  return row;
+}
+
 __device__ __forceinline__ bool game_running(const Pools& P, int g) {
   return P.g_active[g] && P.g_result[g] == RESULT_NONE;
 }
@@ -367,22 +377,15 @@ __global__ void __launch_bounds__(TREE_BLOCK, 7) k_select_expand(Pools P, Policy
       atomicAdd((unsigned long long*)&P.counters[2], (unsigned long long)reused);
       P.s_node[g] = child;
       P.s_kind[g] = kind;
-      if (kind == KIND_EVAL_LEAF) {                // (defensive) the twin's evaluation did not fit: run it
-        const int rb = take_row(P, n_b);
-        list_b[rb] = g;
-        P.s_row[g] = rb;
-      }
+      if (kind == KIND_EVAL_LEAF)                  // (defensive) the twin's evaluation did not fit: run it
+        P.s_row[g] = take_slot_row(P, list_b, n_b, lane_slot(P, g), g);
       return;
     }
   }
   if (lane != 0) return;
   P.s_node[g] = child;
   P.s_kind[g] = kind;
-  if (kind == KIND_NEED_REPLY) {
-    int row = take_row(P, P.eval_n);
-    P.eval_list[row] = g;
-    P.s_row[g] = row;
-  }
+  if (kind == KIND_NEED_REPLY) P.s_row[g] = take_slot_row(P, P.eval_list, P.eval_n, lane_slot(P, g), g);
 }
 
 // ---- wave mode: K in-flight simulations per game (the reference's --threads K, mctree.py:173-176) -----------
@@ -403,6 +406,7 @@ __global__ void __launch_bounds__(TREE_BLOCK) k_select_wave(Pools P) {
   if (g >= P.G) return;
   const int left = game_running(P, g) ? P.g_sims_left[g] : 0;
   const int kmax = min(P.K, left);
+  const int ks = lane_slot(P, g);
   int used = 0;
   for (int j = 0; j < kmax; ++j) {
     int node = 0;
@@ -416,11 +420,7 @@ __global__ void __launch_bounds__(TREE_BLOCK) k_select_wave(Pools P) {
       P.s_node[slot] = leaf;
       P.s_kind[slot] = kind;
       if (kind != KIND_IDLE) vloss_add(P, g, leaf, 1);
-      if (kind == KIND_NEED_REPLY) {
-        const int row = take_row(P, P.eval_n);
-        P.eval_list[row] = slot;
-        P.s_row[slot] = row;
-      }
+      if (kind == KIND_NEED_REPLY) P.s_row[slot] = take_slot_row(P, P.eval_list, P.eval_n, ks, slot);
       __threadfence_block();
     }
     __syncwarp();
@@ -437,7 +437,9 @@ __global__ void __launch_bounds__(TREE_BLOCK) k_finalize_wave(Pools P, PolicyVie
                                                               const int16_t* __restrict__ label_of) {
   const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  if (g == 0 && lane == 0) atomicAdd((unsigned long long*)&P.counters[1], (unsigned long long)*P.eval_n);
+  if (g == 0 && lane == 0)
+    atomicAdd((unsigned long long*)&P.counters[1],
+              (unsigned long long)(*P.eval_n + (P.n_slots > 1 ? P.eval_n[SLOT_N_STRIDE] : 0)));
   if (g >= P.G) return;
   const int used = P.s_wave_n[g];
   for (int j = 0; j < used; ++j) {
@@ -485,14 +487,17 @@ __global__ void __launch_bounds__(256) k_wave_left(Pools P, int* out) {
 // rows of batch A (positions after our move) -> opponent reply, node state, batch B.
 // One WARP per row: the lanes gather the legal-masked policy in parallel and reduce to the FIRST maximum
 // (agentdistributed.py:56-58), then play the reply and build the node together (mctree.py:245-249).
+// blockIdx.y = network slot: the reply is predicted by the searching side's network, and the leaf goes to its batch B.
 __global__ void __launch_bounds__(TREE_BLOCK, 7) k_reply(Pools P, PolicyView pv, const int16_t* __restrict__ label_of,
                                                       int* list_b, int* n_b) {
   __shared__ u16 s_gen[TREE_WARPS][MAX_MOVES];
-  const int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int ks = blockIdx.y;
+  const int r0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  const int n_a = *P.eval_n;
-  if (r == 0 && lane == 0) atomicAdd((unsigned long long*)&P.counters[1], (unsigned long long)n_a);
-  if (r >= n_a) return;
+  const int n_a = P.eval_n[SLOT_N_STRIDE * ks];
+  if (r0 == 0 && lane == 0) atomicAdd((unsigned long long*)&P.counters[1], (unsigned long long)n_a);
+  if (r0 >= n_a) return;
+  const int r = ks * P.slot_stride + r0;
   const int slot = P.eval_list[r];
   const int g = slot / P.K;
   const int child = P.s_node[slot];
@@ -523,11 +528,7 @@ __global__ void __launch_bounds__(TREE_BLOCK, 7) k_reply(Pools P, PolicyView pv,
   const int kind = reply_child_warp(P, g, slot, child, best_i, lane, s_gen[threadIdx.x >> 5]);
   if (lane != 0) return;
   P.s_kind[slot] = kind;
-  if (kind == KIND_EVAL_LEAF) {
-    int rb = take_row(P, n_b);
-    list_b[rb] = slot;
-    P.s_row[slot] = rb;
-  }
+  if (kind == KIND_EVAL_LEAF) P.s_row[slot] = take_slot_row(P, list_b, n_b, ks, slot);
 }
 
 // the last simulation of a crl_mcts_simulate call has no following k_select_expand to finish it: this does
@@ -551,21 +552,23 @@ __global__ void __launch_bounds__(TREE_BLOCK) k_root_init(Pools P, const u8* __r
   }
   if (mask && !mask[g]) return;
   P.s_node[g] = 0;
+  if (P.n_slots > 1)                           // the side to move at the root searches with its slot
+    P.g_slot[g] = P.g_players[(meta_turn(P.g_cur[8LL * P.G + g]) ? 0 : P.G) + g];
   if (!root_init(P, g, use_prev != 0)) {       // priors taken over from the previous tree: no evaluation
     atomicAdd((unsigned long long*)&P.counters[2], 1ull);
     return;
   }
-  int row = take_row(P, P.eval_n);
-  P.eval_list[row] = g;
-  P.s_row[g] = row;
+  P.s_row[g] = take_slot_row(P, P.eval_list, P.eval_n, lane_slot(P, g), g);
 }
 
+// blockIdx.y = network slot (its rows start at row blockIdx.y * slot_stride)
 __global__ void __launch_bounds__(TREE_BLOCK) k_root_priors(Pools P, PolicyView pv,
                                                             const int16_t* __restrict__ label_of) {
-  const int r = blockIdx.x * blockDim.x + threadIdx.x;
-  const int n = *P.eval_n;
-  if (r == 0) atomicAdd((unsigned long long*)&P.counters[1], (unsigned long long)n);
-  if (r >= n) return;
+  const int r0 = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n = P.eval_n[SLOT_N_STRIDE * blockIdx.y];
+  if (r0 == 0) atomicAdd((unsigned long long*)&P.counters[1], (unsigned long long)n);
+  if (r0 >= n) return;
+  const int r = blockIdx.y * P.slot_stride + r0;
   const int g = P.eval_list[r];
   store_priors_of(P, g, 0, [&](int label) { return policy_at(pv, r, label); }, label_of);
 }
@@ -574,8 +577,9 @@ __global__ void __launch_bounds__(TREE_BLOCK) k_root_priors(Pools P, PolicyView 
 __global__ void __launch_bounds__(TREE_BLOCK) k_policy_move(Pools P, PolicyView pv,
                                                             const int16_t* __restrict__ label_of,
                                                             u16* __restrict__ picks) {
-  const int r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r >= *P.eval_n) return;
+  const int r0 = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r0 >= P.eval_n[SLOT_N_STRIDE * blockIdx.y]) return;
+  const int r = blockIdx.y * P.slot_stride + r0;
   const int g = P.eval_list[r];
   const NodeRec& root = P.nodes[(long long)g * P.NN];
   const u16* moves = P.e_move + (long long)g * P.EA + root.edge0;
@@ -736,6 +740,13 @@ static int use_list(crl_engine_impl* e, int which) {
 // Tree(root) for every running game (or the masked subset): node 0, its legal moves, its priors
 // use_prev: a new move search of ALL lanes with evaluation reuse on -- the pools swap roles first, so the tree just
 // searched becomes the previous tree the new one looks its twins up in
+// the row counters of batches A and B, of every slot the search routes rows to
+static int clear_counts(crl_engine_impl* e) {
+  CRL_CUDA(cudaMemsetAsync(e->d_n, 0, 2 * sizeof(int), e->stream));
+  if (e->search_slots > 1) CRL_CUDA(cudaMemsetAsync(e->d_n + SLOT_N_STRIDE, 0, 2 * sizeof(int), e->stream));
+  return CRL_OK;
+}
+
 int tree_begin_move(crl_engine_impl* e, const u8* mask_dev, bool use_prev) {
   if (use_prev) {
     std::swap(e->P.nodes, e->P.nodes_prev);
@@ -743,7 +754,7 @@ int tree_begin_move(crl_engine_impl* e, const u8* mask_dev, bool use_prev) {
     std::swap(e->P.e_child, e->P.e_child_prev);
     e->tree_parity ^= 1;
   }
-  CRL_CUDA(cudaMemsetAsync(e->d_n, 0, 2 * sizeof(int), e->stream));
+  if (int rc = clear_counts(e)) return rc;
   use_list(e, 0);
   e->P.K = 1;                 // root batch: one row per game
   e->P.reuse = e->reuse ? 1 : 0;
@@ -757,7 +768,8 @@ int tree_begin_move(crl_engine_impl* e, const u8* mask_dev, bool use_prev) {
   if (rc != CRL_OK) return rc;
   {
     LaunchScope ls(e, KC_TREE);
-    k_root_priors<<<div_up(e->G, TREE_BLOCK), TREE_BLOCK, 0, e->stream>>>(e->P, e->pview, e->d_label_of);
+    k_root_priors<<<dim3(div_up(e->G, TREE_BLOCK), e->search_slots), TREE_BLOCK, 0, e->stream>>>(e->P, e->pview,
+                                                                                                 e->d_label_of);
     CRL_CUDA(cudaGetLastError());
   }
   return CRL_OK;
@@ -765,7 +777,7 @@ int tree_begin_move(crl_engine_impl* e, const u8* mask_dev, bool use_prev) {
 
 // one lockstep simulation of every running game: the fixed kernel sequence described at the top of this file
 static int one_simulation(crl_engine_impl* e) {
-  CRL_CUDA(cudaMemsetAsync(e->d_n, 0, 2 * sizeof(int), e->stream));
+  if (int rc = clear_counts(e)) return rc;
   use_list(e, 0);
   e->P.K = 1;
   e->P.reuse = e->reuse ? 1 : 0;
@@ -780,8 +792,8 @@ static int one_simulation(crl_engine_impl* e) {
   if (rc != CRL_OK) return rc;
   {
     LaunchScope ls(e, KC_TREE);
-    k_reply<<<div_up((long long)e->G * 32, TREE_BLOCK), TREE_BLOCK, 0, e->stream>>>(e->P, e->pview, e->d_label_of,
-                                                                                   e->d_list[1], e->d_n + 1);
+    k_reply<<<dim3(div_up((long long)e->G * 32, TREE_BLOCK), e->search_slots), TREE_BLOCK, 0, e->stream>>>(
+        e->P, e->pview, e->d_label_of, e->d_list[1], e->d_n + 1);
     CRL_CUDA(cudaGetLastError());
   }
   use_list(e, 1);
@@ -799,7 +811,7 @@ static int finish_simulations(crl_engine_impl* e) {
 
 // one WAVE of every running game: up to K selects per game, two evaluation batches of up to G*K rows, backups
 static int one_wave(crl_engine_impl* e, int K) {
-  CRL_CUDA(cudaMemsetAsync(e->d_n, 0, 2 * sizeof(int), e->stream));
+  if (int rc = clear_counts(e)) return rc;
   use_list(e, 0);
   e->P.K = K;
   e->P.reuse = 0;             // the wave schedule evaluates everything (twins are looked up in the exact schedule only)
@@ -813,8 +825,8 @@ static int one_wave(crl_engine_impl* e, int K) {
   if (rc != CRL_OK) return rc;
   {
     LaunchScope ls(e, KC_TREE);
-    k_reply<<<div_up((long long)e->cur_rows * 32, TREE_BLOCK), TREE_BLOCK, 0, e->stream>>>(e->P, e->pview, e->d_label_of,
-                                                                                         e->d_list[1], e->d_n + 1);
+    k_reply<<<dim3(div_up((long long)e->cur_rows * 32, TREE_BLOCK), e->search_slots), TREE_BLOCK, 0, e->stream>>>(
+        e->P, e->pview, e->d_label_of, e->d_list[1], e->d_n + 1);
     CRL_CUDA(cudaGetLastError());
   }
   use_list(e, 1);
@@ -884,11 +896,15 @@ int tree_run_steps(crl_engine_impl* e, int n_sims, int K) {
   // the kernel parameters (pool pointers included) are baked into the captured graph; with evaluation reuse the tree
   // pools swap roles at every move, so there is one graph per parity
   const int par = e->tree_parity & 1;
-  const unsigned long long key = 1ull + (unsigned long long)e->eval_kind + 2ull * (unsigned long long)e->eval_bits +
-                                 64ull * (e->eval_seed * 0x9E3779B97F4A7C15ull) + 0x100000000ull * (unsigned long long)K +
-                                 (e->reuse ? 0x8000000000000000ull : 0ull) +
-                                 0x9E3779B97F4A7C15ull * (unsigned long long)(e->row_bound > 0 ? e->row_bound : 0) +
-                                 (net_fp8(e) ? 0x4000000000000000ull : 0ull);
+  // the evaluator configuration of every slot the search routes rows to
+  auto slot_key = [e](int k) {
+    return (unsigned long long)e->eval_kind[k] + 2ull * (unsigned long long)e->eval_bits[k] +
+           64ull * (e->eval_seed[k] * 0x9E3779B97F4A7C15ull) + (net_fp8(e, k) ? 0x4000000000000000ull : 0ull);
+  };
+  unsigned long long key = 1ull + slot_key(0) + 0x100000000ull * (unsigned long long)K +
+                           (e->reuse ? 0x8000000000000000ull : 0ull) +
+                           0x9E3779B97F4A7C15ull * (unsigned long long)(e->row_bound > 0 ? e->row_bound : 0);
+  if (e->search_slots > 1) key = (key * 0x100000001B3ull) ^ (slot_key(1) * 0xC2B2AE3D27D4EB4Full) ^ 0x2000000000000000ull;
   if (e->sim_graph[par] == nullptr || e->sim_graph_key[par] != key) {
     if (e->sim_graph[par]) {
       cudaGraphExecDestroy(e->sim_graph[par]);
@@ -933,7 +949,8 @@ int tree_policy_move(crl_engine_impl* e, const u8* mask_dev, u16* picks_dev) {
   e->row_bound = bound;
   if (rc != CRL_OK) return rc;
   LaunchScope ls(e, KC_TREE);
-  k_policy_move<<<div_up(e->G, TREE_BLOCK), TREE_BLOCK, 0, e->stream>>>(e->P, e->pview, e->d_label_of, picks_dev);
+  k_policy_move<<<dim3(div_up(e->G, TREE_BLOCK), e->search_slots), TREE_BLOCK, 0, e->stream>>>(e->P, e->pview,
+                                                                                               e->d_label_of, picks_dev);
   CRL_CUDA(cudaGetLastError());
   return CRL_OK;
 }

@@ -1556,7 +1556,10 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 struct NetWeights {
+  int slot = 0;                             // network slot (crl_net_select_slot)
   int cap_rows = 0;                         // activation capacity in boards (even)
+  void* planes_buf = nullptr;               // where the search encodes this slot's rows (R + 2 bf16 rows; slot 0: e->d_planes)
+  float* stats = nullptr;                   // softmax statistics of this slot's search rows (e->d_stats + 2 x slot rows)
   bool loaded = false;
   __nv_bfloat16* w[N_CONVS] = {nullptr};    // [256][9*Cin] K-major
   float* scale[N_CONVS] = {nullptr};
@@ -1577,7 +1580,7 @@ struct NetWeights {
   CUtensorMap map_w2[N_CONVS];              // weight boxes of 128 filters (one CTA's half)
   __nv_bfloat16* pf = nullptr;              // [cap][128] policy features (bf16)
   float* vf = nullptr;                      // [cap][64] value features
-  float* logits = nullptr;                  // [cap][2048] policy logits
+  float* logits = nullptr;                  // [cap + 256][2048] policy logits (slot k: rows k x slot_stride of one buffer)
   __nv_bfloat16* wp_bf16 = nullptr;         // [2048][128] policy dense kernel, K-major, zero padded
   float* bp_pad = nullptr;                  // [2048]
   float* ones = nullptr;                    // [2048]
@@ -1674,10 +1677,21 @@ static int dev_alloc(crl_engine_impl* e, T** p, size_t count) {
   return CRL_OK;
 }
 
-int net_create(crl_engine_impl* e) {
+int net_create(crl_engine_impl* e, int slot) {
   NetWeights* nw = new NetWeights();
-  e->net = nw;
+  e->nets[slot] = nw;
+  if (e->sel_slot == slot) e->net = nw;
+  nw->slot = slot;
   nw->cap_rows = (e->R + 2) & ~1;
+  nw->stats = e->d_stats + 2 * (long long)slot * e->slot_stride;
+  if (slot == 0) {
+    nw->planes_buf = e->d_planes;
+  } else {
+    __nv_bfloat16* pb = nullptr;
+    int rc0 = dev_alloc(e, &pb, (size_t)(e->R + 2) * 64 * 128);
+    if (rc0) return rc0;
+    nw->planes_buf = pb;
+  }
   void* fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
   cudaError_t err = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres);
@@ -1702,7 +1716,11 @@ int net_create(crl_engine_impl* e) {
     nw->use_v2 = !(v1 && v1[0] == '1');
     if ((rc = dev_alloc(e, &nw->pf, (size_t)(nw->cap_rows + 256) * 128))) return rc;
     if ((rc = dev_alloc(e, &nw->vf, (size_t)(nw->cap_rows + 256) * 64))) return rc;
-    if ((rc = dev_alloc(e, &nw->logits, (size_t)(nw->cap_rows + 256) * 2048))) return rc;
+    if (slot == 0) {
+      if ((rc = dev_alloc(e, &nw->logits, (size_t)(nw->cap_rows + 256) * 2048))) return rc;
+    } else {                              // its rows of the two-slot logits buffer (net_two_slot_layout)
+      nw->logits = e->nets[0]->logits + (size_t)slot * e->slot_stride * 2048;
+    }
     if ((rc = dev_alloc(e, &nw->wp_bf16, (size_t)2048 * 128))) return rc;
     if ((rc = dev_alloc(e, &nw->bp_pad, 2048))) return rc;
     if ((rc = dev_alloc(e, &nw->ones, 2048))) return rc;
@@ -1815,8 +1833,71 @@ int net_create(crl_engine_impl* e) {
 }
 
 void net_destroy(crl_engine_impl* e) {
-  delete e->net;
+  for (int k = 0; k < CRL_NET_SLOTS; ++k) {
+    delete e->nets[k];
+    e->nets[k] = nullptr;
+  }
   e->net = nullptr;
+}
+
+// replaces the device buffer *p (old_count elements, in e->allocs) by one of new_count elements; contents are not kept
+template <class T>
+static int regrow(crl_engine_impl* e, T** p, size_t new_count) {
+  T* q = nullptr;
+  int rc = dev_alloc(e, &q, new_count);
+  if (rc) return rc;
+  for (size_t i = 0; i < e->allocs.size(); ++i)
+    if (e->allocs[i] == (void*)*p) {
+      cudaFree(*p);
+      e->allocs.erase(e->allocs.begin() + i);
+      break;
+    }
+  *p = q;
+  return CRL_OK;
+}
+
+// The first configuration of slot 1: the row lists, policy, value, statistics and logits buffers grow to two slots of
+// slot_stride rows each, so that one PolicyView and one value array serve both slots' rows (DESIGN.md 3.5).  Nothing
+// in flight reads them between API calls (every crl_mcts_simulate call finishes its simulations); the captured
+// simulation graphs name the old buffers and are dropped.
+int net_two_slot_layout(crl_engine_impl* e) {
+  if (e->slot_stride) return CRL_OK;
+  NetWeights* n0 = e->nets[0];
+  const long long S = (long long)n0->cap_rows + 256;     // the rows of one slot's logits
+  CRL_CUDA(cudaStreamSynchronize(e->stream));
+  int rc;
+  for (int i = 0; i < 2; ++i)
+    if ((rc = regrow(e, &e->d_list[i], (size_t)(2 * S)))) return rc;
+  if ((rc = regrow(e, &e->d_policy, (size_t)(2 * S) * CRL_N_LABELS))) return rc;
+  if ((rc = regrow(e, &e->d_value, (size_t)(2 * S)))) return rc;
+  if ((rc = regrow(e, &e->d_stats, (size_t)(4 * S)))) return rc;
+  if ((rc = regrow(e, &n0->logits, (size_t)(2 * S) * 2048))) return rc;
+  CRL_CUDA(cudaMemsetAsync(e->d_list[0], 0, (size_t)(2 * S) * sizeof(int), e->stream));
+  CRL_CUDA(cudaMemsetAsync(e->d_list[1], 0, (size_t)(2 * S) * sizeof(int), e->stream));
+  e->slot_stride = S;
+  e->P.slot_stride = (int)S;
+  e->P.eval_list = e->d_list[0];
+  n0->stats = e->d_stats;
+  if (NetWeights* n1 = e->nets[1]) {
+    n1->stats = e->d_stats + 2 * S;
+    n1->logits = n0->logits + (size_t)S * 2048;
+  }
+  e->pview = PolicyView{e->d_policy, CRL_N_LABELS, nullptr};
+  for (int i = 0; i < 2; ++i) {
+    if (e->sim_graph[i]) cudaGraphExecDestroy(e->sim_graph[i]);
+    e->sim_graph[i] = nullptr;
+    e->sim_graph_key[i] = 0;
+  }
+  return CRL_OK;
+}
+
+int net_slot_ensure(crl_engine_impl* e, int slot) {
+  if (e->nets[slot]) return CRL_OK;
+  int rc = net_two_slot_layout(e);
+  if (rc) return rc;
+  if ((rc = net_create(e, slot))) return rc;
+  CRL_CUDA(cudaStreamSynchronize(e->stream));
+  return CRL_OK;
 }
 
 static inline uint16_t f2bf(float f) {   // round to nearest even
@@ -1943,9 +2024,8 @@ int net_load(crl_engine_impl* e, const float* const* w, const int64_t* sizes, in
   return CRL_OK;
 }
 
-static int launch_conv(crl_engine_impl* e, const CUtensorMap& map_in, int L, const int* n_dev, int n_host,
+static int launch_conv(crl_engine_impl* e, NetWeights* nw, const CUtensorMap& map_in, int L, const int* n_dev, int n_host,
                        const __nv_bfloat16* residual, __nv_bfloat16* out, int relu) {
-  NetWeights* nw = e->net;
   ConvParams p;
   p.n_rows_dev = n_dev;
   p.n_rows_host = n_host;
@@ -1964,9 +2044,8 @@ static int launch_conv(crl_engine_impl* e, const CUtensorMap& map_in, int L, con
   return CRL_OK;
 }
 
-static int launch_conv_v2(crl_engine_impl* e, const CUtensorMap& map_in, int L, const int* n_dev, int n_host,
-                          const __nv_bfloat16* residual, __nv_bfloat16* out, int relu, bool fuse_heads) {
-  NetWeights* nw = e->net;
+static int launch_conv_v2(crl_engine_impl* e, NetWeights* nw, const CUtensorMap& map_in, int L, const int* n_dev,
+                          int n_host, const __nv_bfloat16* residual, __nv_bfloat16* out, int relu, bool fuse_heads) {
   ConvParams2 p;
   memset(&p, 0, sizeof(p));
   p.n_units_dev = n_dev;
@@ -1996,9 +2075,8 @@ static int launch_conv_v2(crl_engine_impl* e, const CUtensorMap& map_in, int L, 
 }
 
 // policy dense layer (128 -> 1968, zero padded to 2048) as a tcgen05 GEMM, then softmax + value head
-static int launch_heads_v2(crl_engine_impl* e, const int* n_dev, int n_host, float* policy, float* value,
+static int launch_heads_v2(crl_engine_impl* e, NetWeights* nw, const int* n_dev, int n_host, float* policy, float* value,
                            PolicyView* view_out) {
-  NetWeights* nw = e->net;
   ConvParams2 p;
   memset(&p, 0, sizeof(p));
   p.n_units_dev = n_dev;
@@ -2037,8 +2115,8 @@ static int launch_heads_v2(crl_engine_impl* e, const int* n_dev, int n_host, flo
     if (full) {
       *view_out = PolicyView{policy, CRL_N_LABELS, nullptr};
     } else {
-      t.stats = e->d_stats;
-      *view_out = PolicyView{nw->logits, 2048, e->d_stats};
+      t.stats = nw->stats;
+      *view_out = PolicyView{nw->logits, 2048, nw->stats};
     }
   }
   LaunchScope ls(e, KC_HEADS);
@@ -2047,10 +2125,9 @@ static int launch_heads_v2(crl_engine_impl* e, const int* n_dev, int n_host, flo
   return CRL_OK;
 }
 
-int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, const int* n_dev, float* policy,
-                float* value, __nv_bfloat16* dbg_out, int dbg_layer, PolicyView* view_out) {
+static int forward_nw(crl_engine_impl* e, NetWeights* nw, const __nv_bfloat16* planes, int n_host, const int* n_dev,
+                      float* policy, float* value, __nv_bfloat16* dbg_out, int dbg_layer, PolicyView* view_out) {
   if (view_out) *view_out = PolicyView{policy, CRL_N_LABELS, nullptr};   // unless the heads below switch to statistics
-  NetWeights* nw = e->net;
   if (!nw || !nw->loaded) {
     set_error("network weights are not loaded (crl_net_load_host)");
     return CRL_ESTATE;
@@ -2061,21 +2138,22 @@ int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, con
     return CRL_EINVAL;
   }
   const bool fp8 = nw->fp8;
-  if (fp8 && planes != e->d_planes) {
-    // a caller's bf16 planes: converted into the engine's planes buffer, where the search encodes its e4m3 rows
+  __nv_bfloat16* const own = (__nv_bfloat16*)nw->planes_buf;
+  if (fp8 && planes != own) {
+    // a caller's bf16 planes: converted into the slot's planes buffer, where the search encodes its e4m3 rows
     const long long n8 = (long long)n_host * 64 * 128 / 8;     // groups of 8 values
     LaunchScope ls(e, KC_ENCODE);
     k_planes_to_e4m3<<<(unsigned)div_up(n8, 256), 256, 0, e->stream>>>(reinterpret_cast<const uint4*>(planes),
-                                                                         reinterpret_cast<uint2*>(e->d_planes), n8);
+                                                                         reinterpret_cast<uint2*>(own), n8);
     CRL_CUDA(cudaGetLastError());
-    planes = e->d_planes;
+    planes = own;
   }
   {
     // the box may start at row n-1 for an odd n: rows beyond the map are zero-filled by the TMA unit.  e4m3 planes in
-    // e->d_planes: the buffer holds R + 2 bf16 rows, so every row a caller may convert into it is inside the map; the
+    // the slot's planes buffer: it holds R + 2 bf16 rows, so every row a caller may convert into it is inside the map; the
     // rows after the batch are then stale buffer contents, not zeros.  That is harmless: an output row of the implicit
     // GEMM depends on its own board's rows only, and the epilogue skips the boards at or after the row count.
-    const int rows = fp8 ? e->R + 2 : planes == e->d_planes ? e->R : n_host;
+    const int rows = fp8 ? e->R + 2 : planes == own ? e->R : n_host;
     if (planes != nw->planes_ptr || rows != nw->planes_rows || fp8 != nw->planes_fp8) {
       int rc;
       if (fp8) {
@@ -2135,24 +2213,25 @@ int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, con
         k_trunk<<<2 * pairs, CONV_THREADS, V2_SMEM_BYTES, e->stream>>>(nw->map_planes, nw->d_maps, nw->d_layers, tp);
       CRL_CUDA(cudaGetLastError());
     }
-    return launch_heads_v2(e, n_dev, n_host, policy, value, view_out);
+    return launch_heads_v2(e, nw, n_dev, n_host, policy, value, view_out);
   }
   if (nw->use_v2) {
-    if ((rc = launch_conv_v2(e, nw->map_planes, 0, n_dev, n_host, nullptr, nw->act[0], 0, false))) return rc;
+    if ((rc = launch_conv_v2(e, nw, nw->map_planes, 0, n_dev, n_host, nullptr, nw->act[0], 0, false))) return rc;
     for (int b = 0; b < 10; ++b) {
-      if ((rc = launch_conv_v2(e, nw->map_act[0], 1 + 2 * b, n_dev, n_host, nullptr, nw->act[1], 1, false))) return rc;
+      if ((rc = launch_conv_v2(e, nw, nw->map_act[0], 1 + 2 * b, n_dev, n_host, nullptr, nw->act[1], 1, false))) return rc;
       const bool last = b == 9;   // the last convolution feeds only the heads: fuse them, skip the activation write
-      if ((rc = launch_conv_v2(e, nw->map_act[1], 2 + 2 * b, n_dev, n_host, nw->act[0], last ? nullptr : nw->act[0], 1, last)))
+      if ((rc = launch_conv_v2(e, nw, nw->map_act[1], 2 + 2 * b, n_dev, n_host, nw->act[0], last ? nullptr : nw->act[0], 1,
+                               last)))
         return rc;
     }
-    return launch_heads_v2(e, n_dev, n_host, policy, value, view_out);
+    return launch_heads_v2(e, nw, n_dev, n_host, policy, value, view_out);
   }
   // stem: conv only (model.py:33-34 -- no BatchNorm / activation after it)
-  if ((rc = launch_conv(e, nw->map_planes, 0, n_dev, n_host, nullptr, nw->act[0], 0))) return rc;
+  if ((rc = launch_conv(e, nw, nw->map_planes, 0, n_dev, n_host, nullptr, nw->act[0], 0))) return rc;
   for (int b = 0; b < 10; ++b) {
     // x -> conv+BN+ReLU -> conv+BN -> +x -> ReLU  (model.py:111-122); the block output overwrites x in place
-    if ((rc = launch_conv(e, nw->map_act[0], 1 + 2 * b, n_dev, n_host, nullptr, nw->act[1], 1))) return rc;
-    if ((rc = launch_conv(e, nw->map_act[1], 2 + 2 * b, n_dev, n_host, nw->act[0], nw->act[0], 1))) return rc;
+    if ((rc = launch_conv(e, nw, nw->map_act[0], 1 + 2 * b, n_dev, n_host, nullptr, nw->act[1], 1))) return rc;
+    if ((rc = launch_conv(e, nw, nw->map_act[1], 2 + 2 * b, n_dev, n_host, nw->act[0], nw->act[0], 1))) return rc;
   }
   HeadParams hp;
   hp.n_rows_dev = n_dev;
@@ -2174,6 +2253,18 @@ int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, con
   return CRL_OK;
 }
 
+int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, const int* n_dev, float* policy,
+                float* value, __nv_bfloat16* dbg_out, int dbg_layer, PolicyView* view_out) {
+  return forward_nw(e, e->net, planes, n_host, n_dev, policy, value, dbg_out, dbg_layer, view_out);
+}
+
+int net_forward_slot(crl_engine_impl* e, int slot, const void* planes, int n_host, const int* n_dev, float* policy,
+                     float* value, PolicyView* view_out) {
+  return forward_nw(e, e->nets[slot], (const __nv_bfloat16*)planes, n_host, n_dev, policy, value, nullptr, -1, view_out);
+}
+
+void* net_planes_buf(const crl_engine_impl* e, int slot) { return e->nets[slot] ? e->nets[slot]->planes_buf : nullptr; }
+
 // debug / test hook: one convolution layer on caller-provided activations (see tests/test_gpu_net.py)
 int net_debug_conv(crl_engine_impl* e, int layer, const __nv_bfloat16* in, int cin, int n, const __nv_bfloat16* residual,
                    __nv_bfloat16* out, int relu) {
@@ -2189,8 +2280,8 @@ int net_debug_conv(crl_engine_impl* e, int layer, const __nv_bfloat16* in, int c
   CUtensorMap m;
   int rc = make_act_map(nw, &m, in, cin, n);
   if (rc) return rc;
-  if (nw->use_v2) return launch_conv_v2(e, m, layer, nullptr, n, residual, out, relu, false);
-  return launch_conv(e, m, layer, nullptr, n, residual, out, relu);
+  if (nw->use_v2) return launch_conv_v2(e, nw, m, layer, nullptr, n, residual, out, relu, false);
+  return launch_conv(e, nw, m, layer, nullptr, n, residual, out, relu);
 }
 
 
@@ -2224,7 +2315,7 @@ int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int 
 // ======================================================================================================
 // fp8 evaluation: calibration, quantised weight pack, precision switch (DESIGN.md section 3.1, row a7)
 // ======================================================================================================
-bool net_fp8(const crl_engine_impl* e) { return e->net && e->net->fp8; }
+bool net_fp8(const crl_engine_impl* e, int slot) { return e->nets[slot] && e->nets[slot]->fp8; }
 
 // the fp8 tower exists as k_trunk4<3, 7> (two tiles and single tile) only
 static int fp8_tower_available(const NetWeights* nw, const char* fn) {
@@ -2389,12 +2480,16 @@ int net_load_fp8(crl_engine_impl* e, const float* const* w, const int64_t* sizes
 int net_set_precision(crl_engine_impl* e, int precision) {
   NetWeights* nw = e->net;
   if (precision == CRL_NET_BF16) {
-    nw->fp8 = false;
+    if (nw) nw->fp8 = false;
     return CRL_OK;
   }
   if (precision != CRL_NET_FP8) {
     set_error("crl_net_set_precision: unknown precision %d", precision);
     return CRL_EINVAL;
+  }
+  if (!nw) {
+    set_error("crl_net_set_precision: no fp8 weights in slot %d (crl_net_load_fp8_host)", e->sel_slot);
+    return CRL_ESTATE;
   }
   int rc = fp8_tower_available(nw, "crl_net_set_precision");
   if (rc) return rc;

@@ -49,6 +49,8 @@ struct NodeRec {
   u8 evald;       // 1 once the node has been evaluated: reply, n_legal, v and its children's priors are final
 };
 
+static constexpr int SLOT_N_STRIDE = 4;   // distance between the row counters of slot 0 and slot 1
+
 struct Pools {
   int G, NN, EA;
   // --- games ---
@@ -93,6 +95,13 @@ struct Pools {
   int* eval_list;   // [G*K] slot of every batch row
   int* eval_n;      // [1]
   int row_cap;      // rows the evaluation kernels of this launch sequence cover (G*K, or the host's bound: crl_mcts_set_row_bound)
+  // --- two networks (crl_games_set_players_host, DESIGN.md 3.5): a lane's rows go to the batch of the slot that moves at
+  // its root; slot k's rows are rows k * slot_stride + r of the list, policy, value and statistics buffers, and its row
+  // count is eval_n[SLOT_N_STRIDE * k] (likewise for batch B's counter)
+  int n_slots;          // 1: every row belongs to slot 0 (g_players / g_slot are not read)
+  int slot_stride;
+  const u8* g_players;  // [2][G] slot playing white / black
+  u8* g_slot;           // [G] slot searching at the lane's root (set by k_root_init)
   int* err;         // [1] ERR_* flags
   long long* counters;  // [0] simulations [1] evaluations run [2] evaluations taken from the previous tree instead
 };

@@ -7,6 +7,7 @@ raises -- there is no CPU path.
 
 from __future__ import annotations
 
+import contextlib
 import ctypes
 
 import numpy as np
@@ -23,6 +24,9 @@ def _ptr(t):
 
 def _np(a, ctype):
     return a.ctypes.data_as(ctypes.POINTER(ctype))
+
+
+NET_SLOTS = 2      # CRL_NET_SLOTS: networks one engine holds (include/chessrl_b200.h crl_net_select_slot)
 
 
 class Engine:
@@ -46,7 +50,8 @@ class Engine:
                                          int(avg_moves), self.max_inflight, vp(stream)))
         self.h = h
         self.weights_loaded = False
-        self.net_precision = "bf16"
+        self.net_precision = "bf16"                     # slot 0's
+        self.slot_precision = ["bf16"] * NET_SLOTS      # every network slot's (load_weights / set_net_precision)
 
     def close(self):
         if getattr(self, "h", None):
@@ -171,11 +176,32 @@ class Engine:
         return t.reshape(5, 64, 64)
 
     # ---- network ------------------------------------------------------------------------------------------
-    def load_weights(self, tensors, precision="bf16", calibration=None):
+    @contextlib.contextmanager
+    def _slot(self, slot):
+        """The network calls inside act on network slot `slot`; the engine is back on slot 0 afterwards."""
+        slot = int(slot)
+        if slot == 0:
+            yield
+            return
+        check(self.lib.crl_net_select_slot(self.h, slot))
+        try:
+            yield
+        finally:
+            check(self.lib.crl_net_select_slot(self.h, 0))
+
+    def load_weights(self, tensors, precision="bf16", calibration=None, slot=0):
         """tensors: the 140-array weight pack (chessrl_b200.model.ChessModel.weights).
         precision="fp8" also builds the e4m3 tower (include/chessrl_b200.h crl_net_load_fp8_host) and selects it; its
         activation scales come from `calibration`: 21 per-layer amax values (Engine.calibrate), bf16 planes
-        [n,8,8,128] to calibrate on, or None for model.calibration_planes(self)."""
+        [n,8,8,128] to calibrate on, or None for model.calibration_planes(self).
+        slot: the network slot (0 or 1) the weights go to; slot 1 is the second player of games_set_players."""
+        if slot != 0:
+            with self._slot(slot):
+                self._load_weights(tensors, precision, calibration, slot)
+            return
+        self._load_weights(tensors, precision, calibration, 0)
+
+    def _load_weights(self, tensors, precision, calibration, slot):
         if precision not in ("bf16", "fp8"):
             raise ValueError("precision must be 'bf16' or 'fp8', not %r" % (precision,))
         arrs = [np.ascontiguousarray(np.asarray(t, dtype=np.float32).reshape(-1)) for t in tensors]
@@ -184,26 +210,37 @@ class Engine:
         sizes = (ctypes.c_int64 * n)(*[a.size for a in arrs])
         if precision == "bf16" or calibration is None or torch.is_tensor(calibration):
             # the bf16 tower; for fp8 it is also what calibrates (crl_net_load_fp8_host loads it again below)
-            self.net_precision = "bf16"
+            self._set_precision_attr(slot, "bf16")
             check(self.lib.crl_net_load_host(self.h, ptrs, sizes, n))
-            self.weights_loaded = True
+            if slot == 0:
+                self.weights_loaded = True
         if precision == "fp8":
             if calibration is None:
                 from .model import calibration_planes
                 calibration = calibration_planes(self)
             if torch.is_tensor(calibration):
-                calibration = self.calibrate(calibration)
+                calibration = self._calibrate(calibration)
             amax = np.ascontiguousarray(np.asarray(calibration, dtype=np.float32).reshape(-1))
             if amax.size != 21:
                 raise ValueError("calibration: 21 per-layer amax values expected, got %d" % amax.size)
-            self.net_precision = "bf16"                  # what a failed fp8 load leaves the engine in
+            self._set_precision_attr(slot, "bf16")           # what a failed fp8 load leaves the slot in
             check(self.lib.crl_net_load_fp8_host(self.h, ptrs, sizes, n, amax.ctypes.data_as(_lib.c_f32p)))
-            self.weights_loaded = True
-        self.net_precision = precision
+            if slot == 0:
+                self.weights_loaded = True
+        self._set_precision_attr(slot, precision)
 
-    def calibrate(self, planes_t):
+    def _set_precision_attr(self, slot, precision):
+        self.slot_precision[slot] = precision
+        if slot == 0:
+            self.net_precision = precision
+
+    def calibrate(self, planes_t, slot=0):
         """max |output| of each of the 21 tower convolutions over bf16 planes [n,8,8,128], from the bf16 tower
         -> float32 [21] (the `calibration` of load_weights(precision="fp8"))."""
+        with self._slot(slot):
+            return self._calibrate(planes_t)
+
+    def _calibrate(self, planes_t):
         amax = np.zeros(21, dtype=np.float32)
         part = np.zeros(21, dtype=np.float32)
         step = self.max_games * self.max_inflight          # rows the engine's buffers hold
@@ -213,19 +250,21 @@ class Engine:
             amax = np.maximum(amax, part)
         return amax
 
-    def set_net_precision(self, precision):
+    def set_net_precision(self, precision, slot=0):
         """'bf16' or 'fp8' (the latter needs a load_weights(..., precision="fp8") since the last bf16 load)."""
         code = {"bf16": _lib.NET_BF16, "fp8": _lib.NET_FP8}.get(precision)
         if code is None:
             raise ValueError("precision must be 'bf16' or 'fp8', not %r" % (precision,))
-        check(self.lib.crl_net_set_precision(self.h, code))
-        self.net_precision = precision
+        with self._slot(slot):
+            check(self.lib.crl_net_set_precision(self.h, code))
+        self._set_precision_attr(int(slot), precision)
 
-    def net_forward(self, planes_t):
+    def net_forward(self, planes_t, slot=0):
         n = planes_t.shape[0]
         policy = torch.empty((n, _lib.N_LABELS), dtype=torch.float32, device=self.device)
         value = torch.empty((n,), dtype=torch.float32, device=self.device)
-        check(self.lib.crl_net_forward(self.h, _ptr(planes_t), n, _ptr(policy), _ptr(value)))
+        with self._slot(slot):
+            check(self.lib.crl_net_forward(self.h, _ptr(planes_t), n, _ptr(policy), _ptr(value)))
         return policy, value
 
     def debug_conv(self, layer, x_t, residual_t=None, relu=False):
@@ -234,7 +273,7 @@ class Engine:
         check(self.lib.crl_debug_conv(self.h, int(layer), _ptr(x_t), cin, n, _ptr(residual_t), _ptr(out), int(relu)))
         return out
 
-    def debug_tower(self, planes_t, layer=20):
+    def debug_tower(self, planes_t, layer=20, slot=0):
         """The production forward pass with taps: dict(act = output of convolution `layer` [n,8,8,256] bf16,
         logits [n,1968], pf [n,128] bf16, vf [n,64], policy [n,1968], value [n])."""
         n = planes_t.shape[0]
@@ -245,11 +284,12 @@ class Engine:
                "vf": torch.empty((n, 64), dtype=torch.float32, device=dev),
                "policy": torch.empty((n, _lib.N_LABELS), dtype=torch.float32, device=dev),
                "value": torch.empty((n,), dtype=torch.float32, device=dev)}
-        check(self.lib.crl_debug_tower(self.h, _ptr(planes_t), n, int(layer), _ptr(out["act"]), _ptr(out["logits"]),
-                                       _ptr(out["pf"]), _ptr(out["vf"]), _ptr(out["policy"]), _ptr(out["value"])))
+        with self._slot(slot):
+            check(self.lib.crl_debug_tower(self.h, _ptr(planes_t), n, int(layer), _ptr(out["act"]), _ptr(out["logits"]),
+                                           _ptr(out["pf"]), _ptr(out["vf"]), _ptr(out["policy"]), _ptr(out["value"])))
         return out
 
-    def debug_forward_counted(self, planes_t, n_bound, count, policy=None, value=None):
+    def debug_forward_counted(self, planes_t, n_bound, count, policy=None, value=None, slot=0):
         """Test hook: net_forward as a search batch runs it -- launched for n_bound rows, with the row count `count` read
         by the kernels from device memory (int, or a device int32 tensor of one element).  Rows at or after the count
         of `policy` [n_bound,1968] / `value` [n_bound] (allocated when None) are left as they were."""
@@ -261,8 +301,9 @@ class Engine:
         if not torch.is_tensor(count):
             count = torch.tensor([int(count)], dtype=torch.int32, device=dev)
         assert count.dtype == torch.int32 and count.device == dev
-        check(self.lib.crl_debug_forward_counted(self.h, _ptr(planes_t), int(n_bound), _ptr(count), _ptr(policy),
-                                                 _ptr(value)))
+        with self._slot(slot):
+            check(self.lib.crl_debug_forward_counted(self.h, _ptr(planes_t), int(n_bound), _ptr(count), _ptr(policy),
+                                                     _ptr(value)))
         return policy, value
 
     def hash_eval(self, boards_t, seed, policy_bits=24):
@@ -273,8 +314,28 @@ class Engine:
         return policy, value
 
     # ---- games + search -----------------------------------------------------------------------------------
-    def set_evaluator(self, kind, seed=0, policy_bits=24):
-        check(self.lib.crl_set_evaluator(self.h, int(kind), int(seed), int(policy_bits)))
+    def set_evaluator(self, kind, seed=0, policy_bits=24, slot=0):
+        with self._slot(slot):
+            check(self.lib.crl_set_evaluator(self.h, int(kind), int(seed), int(policy_bits)))
+
+    def games_set_players(self, white, black, first=0):
+        """Network slot (0 or 1) that plays white / black in lanes first..first+len(white)-1 (scalars apply to all
+        lanes from `first` on).  A search evaluates a lane's rows with the slot of the side to move at its root
+        (include/chessrl_b200.h crl_games_set_players_host).  The players persist across games_set / games_restart."""
+        n = self.max_games - int(first)
+        w = np.asarray(white, dtype=np.uint8)
+        b = np.asarray(black, dtype=np.uint8)
+        if w.ndim == 0 and b.ndim == 0:
+            w, b = np.full(n, w, dtype=np.uint8), np.full(n, b, dtype=np.uint8)
+        elif w.ndim == 0:
+            w = np.full(b.shape, w, dtype=np.uint8)
+        elif b.ndim == 0:
+            b = np.full(w.shape, b, dtype=np.uint8)
+        w, b = np.ascontiguousarray(w), np.ascontiguousarray(b)
+        if w.shape != b.shape or w.ndim != 1:
+            raise ValueError("white and black: one slot per lane, of the same length")
+        check(self.lib.crl_games_set_players_host(self.h, int(first), int(w.size), _np(w, ctypes.c_uint8),
+                                                  _np(b, ctypes.c_uint8)))
 
     @staticmethod
     def pack_move_lists(move_lists):

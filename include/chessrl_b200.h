@@ -218,6 +218,25 @@ int crl_games_legal_host(crl_engine* e, int first, int n, uint16_t* legal_host, 
 /* AgentDistributed.best_move(real_game=True) (agentdistributed.py:56-58): policy argmax over legal moves for
  * every game with mask_host[g] != 0 (NULL = all running games); writes picks_host [n_games] and plays them. */
 int crl_games_policy_move_host(crl_engine* e, const uint8_t* mask_host, uint16_t* picks_host);
+/* Two networks in one engine: a match between them in one lockstep batch (chessrl_b200/arena.py, DESIGN.md 3.5).
+ *   crl_net_select_slot       : the network slot (0 or 1, else CRL_EINVAL) that crl_net_load_host,
+ *                               crl_net_load_fp8_host, crl_net_calibrate_host, crl_net_set_precision, crl_set_evaluator,
+ *                               crl_net_forward, crl_debug_tower, crl_debug_forward_counted and crl_debug_conv act on.
+ *                               Each slot has its own weights, precision and evaluator (kind, seed, policy bits).  The
+ *                               slot is 0 after crl_create; slot 1 allocates nothing until a load or crl_set_evaluator
+ *                               configures it, and configuring one slot leaves the other's outputs bit-identical.
+ *   crl_games_set_players_host: for lanes first..first+n-1, the slot that plays white (white_slot_host [n]) and the one
+ *                               that plays black (black_slot_host [n]); 0 and 0 after crl_create.  They persist through
+ *                               crl_games_set_host / crl_games_restart_host.  A lane whose players change loses its
+ *                               evaluation-reuse twin, and a search must begin again (crl_mcts_begin_move).
+ * A search (crl_mcts_begin_move, crl_mcts_simulate, K = 1 and wave mode) and crl_games_policy_move_host evaluate every
+ * row of a lane with the slot of the side to move at the lane's root: the root, the opponent replies it predicts and
+ * its leaves.  While no lane names slot 1 the search runs exactly as with one network.  CRL_ESTATE when a lane names
+ * slot 1 but slot 1 has no evaluator, or when the two slots hold evaluators of different kinds (hash and network). */
+#define CRL_NET_SLOTS 2
+int crl_net_select_slot(crl_engine* e, int slot);
+int crl_games_set_players_host(crl_engine* e, int first, int n, const uint8_t* white_slot_host,
+                               const uint8_t* black_slot_host);
 /* Tree(root) (mctree.py:104-111): a fresh tree per running game rooted at its current position,
  * root.visits = 1, root evaluated once for its children's priors. */
 int crl_mcts_begin_move(crl_engine* e);

@@ -5,11 +5,15 @@ plays one game; the side to move searches with its own network -- root, predicte
 (crl_games_set_players_host) -- so one lockstep step advances every running game by one ply, for about the cost of a
 self-play step (DESIGN.md 3.5).  Openings come in pairs: each is played once with A as white and once with B as white.
 
+Either side may instead be the fixed-depth alpha-beta opponent (AlphaBetaPlayer, DESIGN.md 3.6): a yardstick of fixed
+strength that needs no weights.  Its moves come from Engine.games_ab_move on the same lanes.
+
     python -m chessrl_b200.arena A B --games N [--lanes L] [--sims S] [--threads K] [--precision-a bf16|fp8]
         [--precision-b bf16|fp8] [--opening-plies P | --openings FILE] [--max-plies M] [--seed X] [--out match.json]
 
 A and B are weights files (.h5) or model directories (their newest model-<n>.h5); they may be the same file with
-different precisions, which measures what fp8 evaluation costs in playing strength.
+different precisions, which measures what fp8 evaluation costs in playing strength.  `alphabeta[:D[:Q]]` in place of
+either names the alpha-beta opponent at depth D and quiescence depth Q (default alphabeta:3:4).
 """
 
 from __future__ import annotations
@@ -39,17 +43,61 @@ class HashPlayer:
         self.policy_bits = int(policy_bits)
 
 
+AB_DEPTH, AB_QDEPTH = 3, 4     # the alpha-beta opponent's defaults (DESIGN.md 3.6: cost and ladder)
+
+
+class AlphaBetaPlayer:
+    """The fixed-depth alpha-beta opponent (include/chessrl_b200.h crl_games_ab_move_host): material and position
+    evaluation, `depth` full-width plies (1..5), then up to `qdepth` plies of captures and queen promotions (0..8).
+    Deterministic: the same position gives the same move.  It searches on the lanes' own positions and needs no network
+    slot."""
+
+    def __init__(self, depth=AB_DEPTH, qdepth=AB_QDEPTH):
+        self.depth = int(depth)
+        self.qdepth = int(qdepth)
+        if not (1 <= self.depth <= 5 and 0 <= self.qdepth <= 8):
+            raise ValueError("alpha-beta depth 1..5 and qdepth 0..8, not %d / %d" % (self.depth, self.qdepth))
+
+    SPEC = "alphabeta"
+
+    @classmethod
+    def parse(cls, spec):
+        """'alphabeta', 'alphabeta:D' or 'alphabeta:D:Q' -> AlphaBetaPlayer; None for any other string."""
+        parts = spec.split(":")
+        if parts[0] != cls.SPEC or len(parts) > 3:
+            return None
+        try:
+            nums = [int(p) for p in parts[1:]]
+        except ValueError:
+            raise ValueError("alpha-beta player: 'alphabeta[:D[:Q]]', not %r" % (spec,))
+        return cls(*nums)
+
+    def __str__(self):
+        return "%s:%d:%d" % (self.SPEC, self.depth, self.qdepth)
+
+    __repr__ = __str__
+
+    def moves(self, engine, mask):
+        """This player's moves in the lanes of `mask` (MOVE_NONE elsewhere)."""
+        return engine.games_ab_move(self.depth, self.qdepth, mask=mask.astype(np.uint8))[0]
+
+
 def _as_player(x):
-    """A ChessModel, an Agent, a weights path, a model directory or a HashPlayer -> HashPlayer or ChessModel."""
+    """A ChessModel, an Agent, a weights path, a model directory, 'alphabeta[:D[:Q]]', a HashPlayer or an
+    AlphaBetaPlayer -> HashPlayer, AlphaBetaPlayer or ChessModel."""
     from .model import ChessModel
     from .selfplay import get_model_path
-    if isinstance(x, (HashPlayer, ChessModel)):
+    if isinstance(x, (HashPlayer, AlphaBetaPlayer, ChessModel)):
         return x
     if hasattr(x, "model") and isinstance(x.model, ChessModel):      # an Agent
         return x.model
     if isinstance(x, str):
+        ab = AlphaBetaPlayer.parse(x)
+        if ab is not None:
+            return ab
         return ChessModel(weights=get_model_path(x) if os.path.isdir(x) else x)
-    raise ValueError("a ChessModel, an Agent, a weights path, a model directory or a HashPlayer is needed, not %r" % (x,))
+    raise ValueError("a ChessModel, an Agent, a weights path, a model directory, a HashPlayer or an AlphaBetaPlayer is "
+                     "needed, not %r" % (x,))
 
 
 def _configure(engine, player, slot, precision):
@@ -103,7 +151,8 @@ def summarize(games):
 def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", precision_b="bf16", openings=None,
                opening_plies=4, max_plies=512, seed=None, device=None, engine=None):
     """`games` games of A against B, each side searching its own moves with `sims` simulations (`inflight` in flight
-    per game, the reference's threads) and playing the most visited root child.  Game 2i and 2i+1 start from opening i,
+    per game, the reference's threads) and playing the most visited root child; an AlphaBetaPlayer side plays the move
+    of its fixed-depth search instead.  Game 2i and 2i+1 start from opening i,
     with A as white in the first and B as white in the second.  Openings are `openings` (a list of UCI move lists,
     used in turn) or `opening_plies` seeded random legal plies.  A game that reaches `max_plies` plies stops unfinished.
     `engine`: an engine to play on (default: a new Engine with `lanes` lanes on `device`).
@@ -114,8 +163,13 @@ def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", pr
     if games <= 0:
         raise ValueError("games must be positive")
     pa, pb = _as_player(a), _as_player(b)
-    if isinstance(pa, HashPlayer) != isinstance(pb, HashPlayer):
+    ab = [p if isinstance(p, AlphaBetaPlayer) else None for p in (pa, pb)]
+    searchers = [k for k, p in enumerate((pa, pb)) if ab[k] is None]       # the sides that search with MCTS
+    if len(searchers) == 2 and isinstance(pa, HashPlayer) != isinstance(pb, HashPlayer):
         raise ValueError("a match is between two networks or two hash players (one search cannot mix them)")
+    # network slot of each searching side: A 0 and B 1 when both search; a single searching side takes slot 0, so that
+    # the search runs on one slot, as with one network
+    slot_of = {k: (k if len(searchers) == 2 else 0) for k in searchers}
     if lanes is None:
         lanes = games if engine is None else min(games, engine.max_games)
     lanes = max(1, min(games, int(lanes)))
@@ -123,8 +177,9 @@ def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", pr
     if own:
         from .engine import Engine
         from .selfplay import edge_slots_per_node
-        engine = Engine(max_games=lanes, max_nodes=int(sims) + 1, device=device, max_inflight=int(inflight),
-                        avg_moves=edge_slots_per_node(lanes, int(sims) + 1, device))
+        nodes = int(sims) + 1 if searchers else 2
+        engine = Engine(max_games=lanes, max_nodes=nodes, device=device, max_inflight=int(inflight),
+                        avg_moves=edge_slots_per_node(lanes, nodes, device))
     e = engine
     if e.max_games < lanes:
         raise ValueError("the engine has %d lanes, %d asked for" % (e.max_games, lanes))
@@ -134,8 +189,8 @@ def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", pr
     opening_of = [None] * n_open                   # UCI lists, fixed at the first game of each pair
     out = [None] * games
     try:
-        _configure(e, pa, 0, precision_a)          # (a load replays on lane 0: configure before the games are set)
-        _configure(e, pb, 1, precision_b)
+        for k in searchers:                        # (a load replays on lane 0: configure before the games are set)
+            _configure(e, (pa, pb)[k], slot_of[k], (precision_a, precision_b)[k])
         e.set_reuse(False)
         e.games_set(np.tile(B.record_from_fen(), (e.max_games, 1)))
         lane_game = np.full(e.max_games, -1, dtype=np.int64)
@@ -150,7 +205,10 @@ def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", pr
                 next_game += 1
                 lane_game[lane] = j
                 a_white = j % 2 == 0
-                e.games_set_players([0 if a_white else 1], [1 if a_white else 0], first=int(lane))
+                if len(searchers) == 2:
+                    e.games_set_players([0 if a_white else 1], [1 if a_white else 0], first=int(lane))
+                elif searchers:
+                    e.games_set_players([0], [0], first=int(lane))
                 i = j // 2
                 if opening_of[i] is None and fixed is not None:
                     opening_of[i] = fixed[i % len(fixed)]
@@ -177,7 +235,7 @@ def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", pr
         live[first] = True
         if not live.all():
             e.games_set_active(live.astype(np.uint8))
-        _, plies, results = e.games_get(0, e.max_games)
+        rec, plies, results = e.games_get(0, e.max_games)
         while True:
             over = live & ((results != B.RESULT_NONE) | (plies >= max_plies))
             if over.any():                         # harvest, then refill or park
@@ -196,21 +254,38 @@ def play_match(a, b, games, sims, lanes=None, inflight=1, precision_a="bf16", pr
                     e.games_set_active(live.astype(np.uint8))
                 if not live.any():
                     break
-                _, plies, results = e.games_get(0, e.max_games)
+                rec, plies, results = e.games_get(0, e.max_games)
                 continue                           # a refilled opening may already have ended the game
-            # one ply of every running game: the side to move searches with its network and plays its most visited child
-            n_run = int(live.sum())
-            small = SMALL_BATCH_ROWS // max(1, int(inflight))
-            e.set_row_bound(small if 0 < n_run <= small < e.max_games else 0)
-            e.mcts_begin_move()
-            e.mcts_simulate(int(sims), int(inflight))
-            st = e.root_stats(want=("visits", "moves"))
-            picks = pick_moves(st["visits"], st["n_children"], st["root_visits"], plies, live, noise=False)
-            rows = np.nonzero(picks >= 0)[0]
+            # one ply of every running game: the side to move searches with its network and plays its most visited
+            # child, or plays its alpha-beta move
+            white = (rec[:, 8] & np.uint64(1)).astype(bool)
+            a_to_move = white == (lane_game % 2 == 0)
+            ab_turn = [live & (a_to_move if k == 0 else ~a_to_move) if ab[k] is not None else None for k in (0, 1)]
+            searching = live.copy()
+            for t in ab_turn:
+                if t is not None:
+                    searching &= ~t
             mv = np.full(e.max_games, B.MOVE_NONE, dtype=np.uint16)
-            mv[rows] = st["moves"][rows, picks[rows]]
+            if searching.any():
+                parked = not np.array_equal(searching, live)
+                if parked:                         # the alpha-beta side's lanes sit out the search
+                    e.games_set_active(searching.astype(np.uint8))
+                n_run = int(searching.sum())
+                small = SMALL_BATCH_ROWS // max(1, int(inflight))
+                e.set_row_bound(small if 0 < n_run <= small < e.max_games else 0)
+                e.mcts_begin_move()
+                e.mcts_simulate(int(sims), int(inflight))
+                st = e.root_stats(want=("visits", "moves"))
+                picks = pick_moves(st["visits"], st["n_children"], st["root_visits"], plies, searching, noise=False)
+                rows = np.nonzero(picks >= 0)[0]
+                mv[rows] = st["moves"][rows, picks[rows]]
+                if parked:                         # resumed before the play: games_play skips parked lanes
+                    e.games_set_active(live.astype(np.uint8))
+            for k in (0, 1):
+                if ab_turn[k] is not None and ab_turn[k].any():
+                    mv = np.where(ab_turn[k], ab[k].moves(e, ab_turn[k]), mv)
             e.games_play(mv)
-            _, plies, results = e.games_get(0, e.max_games)
+            rec, plies, results = e.games_get(0, e.max_games)
     finally:
         if own:
             e.close()
@@ -222,11 +297,18 @@ def _read_openings(path):
         return [line.split() for line in f if line.strip() and not line.lstrip().startswith("#")]
 
 
+def _label(arg, precision):
+    """How a CLI player is reported: 'alphabeta:D:Q' (its full parameters) or 'path (precision)'."""
+    ab = AlphaBetaPlayer.parse(arg)
+    return str(ab) if ab is not None else "%s (%s)" % (arg, precision)
+
+
 def main(argv=None):
-    ap = argparse.ArgumentParser(description="Plays a search-vs-search match between two networks and prints the score "
-                                             "and the Elo difference A - B with its 95 % interval.")
-    ap.add_argument("a", help="weights file (.h5) or model directory of player A")
-    ap.add_argument("b", help="weights file (.h5) or model directory of player B (may be A's)")
+    ap = argparse.ArgumentParser(description="Plays a search-vs-search match between two networks, or a network and the "
+                                             "alpha-beta opponent, and prints the score and the Elo difference A - B with "
+                                             "its 95 % interval.")
+    ap.add_argument("a", help="weights file (.h5) or model directory of player A, or alphabeta[:D[:Q]]")
+    ap.add_argument("b", help="weights file (.h5) or model directory of player B (may be A's), or alphabeta[:D[:Q]]")
     ap.add_argument("--games", type=int, required=True)
     ap.add_argument("--lanes", type=int, default=None, help="concurrent games (default: one per game)")
     ap.add_argument("--sims", type=int, default=100, help="simulations per move")
@@ -246,13 +328,15 @@ def main(argv=None):
                                 openings=_read_openings(args.openings) if args.openings else None,
                                 opening_plies=args.opening_plies, max_plies=args.max_plies, seed=args.seed)
     summary["wall_s"] = round(time.time() - t0, 3)
-    print("A %s (%s) vs B %s (%s): %d games, +%d -%d =%d (%d unfinished), score %.4f, Elo %+.1f [%+.1f, %+.1f], %.1f s"
-          % (args.a, args.precision_a, args.b, args.precision_b, summary["played"], summary["a_wins"], summary["b_wins"],
-             summary["draws"], summary["unfinished"], summary["score"], summary["elo"], summary["elo_low"],
-             summary["elo_high"], summary["wall_s"]))
+    label_a, label_b = _label(args.a, args.precision_a), _label(args.b, args.precision_b)
+    print("A %s vs B %s: %d games, +%d -%d =%d (%d unfinished), score %.4f, Elo %+.1f [%+.1f, %+.1f], %.1f s"
+          % (label_a, label_b, summary["played"], summary["a_wins"], summary["b_wins"], summary["draws"],
+             summary["unfinished"], summary["score"], summary["elo"], summary["elo_low"], summary["elo_high"],
+             summary["wall_s"]))
     if args.out:
         with open(args.out, "w") as f:
-            json.dump({"a": args.a, "b": args.b, "precision_a": args.precision_a, "precision_b": args.precision_b,
+            json.dump({"a": args.a, "b": args.b, "player_a": label_a, "player_b": label_b,
+                       "precision_a": args.precision_a, "precision_b": args.precision_b,
                        "sims": args.sims, "threads": args.threads, "summary": summary, "games": games}, f, indent=1)
     return summary
 

@@ -3,11 +3,13 @@
 The reference plays N games of its agent -- moving by the argmax of the legal-masked policy,
 `Agent.best_move(game, real_game=True)` (benchmark.py:88-90, agent.py:39-43) -- against a Stockfish process wrapped
 in GameStockfish, and tallies played / won / drawn.  Stockfish is out of scope here (no binary, SURVEY.md 8(f)-4);
-the loop itself is kept: the same agent side, the same tally, and an opponent that is either a seeded uniformly
-random mover or a second network (also policy argmax).  `workers` concurrent games become `workers` lockstep lanes of
-one engine; every ply of every running game is one batched network evaluation.
+the loop itself is kept: the same agent side, the same tally, and an opponent that is a seeded uniformly random mover,
+a second network (also policy argmax) or the fixed-depth alpha-beta opponent (arena.AlphaBetaPlayer, DESIGN.md 3.6),
+the fixed yardstick that stands in for Stockfish.  `workers` concurrent games become `workers` lockstep lanes of one
+engine; every ply of every running game is one batched network evaluation or one batched alpha-beta call.
 
-    python -m chessrl_b200.benchmark modeldir [--games 10] [--workers 2] [--opponent random|path/to/weights.h5]
+    python -m chessrl_b200.benchmark modeldir [--games 10] [--workers 2]
+        [--opponent random|path/to/weights.h5|alphabeta[:D[:Q]]]
 """
 
 from __future__ import annotations
@@ -20,6 +22,7 @@ import numpy as np
 
 from . import boards as B
 from ._lib import EVAL_NET
+from .arena import AlphaBetaPlayer
 from .lib.logger import Logger
 from .model import ChessModel
 from .selfplay import get_model_path
@@ -36,12 +39,15 @@ def _as_model(x):
 
 
 def play_policy_games(agent, opponent="random", games=10, lanes=None, seed=None, device=None, max_plies=2000):
-    """`games` games, agent (policy argmax) versus `opponent` ("random", or a ChessModel / Agent / weights path that
-    also moves by policy argmax).  The agent's colour is drawn per game like benchmark.py:70.
+    """`games` games, agent (policy argmax) versus `opponent` ("random"; a ChessModel / Agent / weights path that
+    also moves by policy argmax; or an AlphaBetaPlayer / 'alphabeta[:D[:Q]]', searched on the agent's engine).  The
+    agent's colour is drawn per game like benchmark.py:70.
     Returns one dict per game in game order: {'color', 'result' (white point of view, None if capped), 'moves'}."""
     from .engine import Engine
     agent_model = _as_model(agent)
-    opp_model = None if isinstance(opponent, str) and opponent == "random" else _as_model(opponent)
+    ab = opponent if isinstance(opponent, AlphaBetaPlayer) else (
+        AlphaBetaPlayer.parse(opponent) if isinstance(opponent, str) else None)
+    opp_model = None if ab is not None or (isinstance(opponent, str) and opponent == "random") else _as_model(opponent)
     rng = random.Random(seed)
     lanes = max(1, min(games, games if lanes is None else int(lanes)))
     a = Engine(max_games=lanes, max_nodes=2, avg_moves=218, device=device)
@@ -99,6 +105,8 @@ def play_policy_games(agent, opponent="random", games=10, lanes=None, seed=None,
                 if b is not None:
                     picks = b.policy_move(mask=opp_turn.astype(np.uint8))
                     a.games_play(np.where(opp_turn, picks, none))
+                elif ab is not None:
+                    a.games_play(ab.moves(a, opp_turn))
                 else:
                     legal, cnt = a.games_legal(0, lanes)
                     mv = none.copy()
@@ -115,7 +123,8 @@ def play_policy_games(agent, opponent="random", games=10, lanes=None, seed=None,
 def benchmark(model_dir, workers=1, games=10, stockfish_depth=10, log=False, opponent="random", seed=None):
     """Plays `games` games and returns dict(played, won, drawn) like the reference (benchmark.py:103-143).
     `workers` = concurrent games (lockstep lanes here, processes there).  `stockfish_depth` is accepted for signature
-    compatibility only: the opponent is `opponent` (see play_policy_games), not Stockfish."""
+    compatibility only: the opponent is `opponent` (see play_policy_games), not Stockfish; the depth-selected fixed
+    opponent here is opponent="alphabeta:D[:Q]"."""
     logger = Logger.get_instance()
     if log:
         logger.info("Setting up %d concurrent games." % workers)
@@ -140,7 +149,8 @@ def main(argv=None):
     ap.add_argument("model_dir", metavar="modeldir")
     ap.add_argument("--games", type=int, default=10)
     ap.add_argument("--workers", type=int, default=2, help="concurrent games (lockstep lanes)")
-    ap.add_argument("--opponent", default="random", help="'random' or a path to the opponent's weights")
+    ap.add_argument("--opponent", default="random",
+                    help="'random', a path to the opponent's weights, or alphabeta[:D[:Q]] (fixed-depth alpha-beta)")
     ap.add_argument("--seed", type=int, default=None)
     args = ap.parse_args(argv)
     print(benchmark(args.model_dir, workers=args.workers, games=args.games, log=True, opponent=args.opponent, seed=args.seed))

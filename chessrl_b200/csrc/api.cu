@@ -961,6 +961,27 @@ int crl_games_policy_move_host(crl_engine* e, const uint8_t* mask_host, uint16_t
   return check_pool_errors(e);
 }
 
+int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, uint16_t* move_host,
+                           int32_t* score_host, int64_t* nodes_host) {
+  CHECK_ENGINE(e);
+  const size_t G = e->G;
+  const u8* mask_dev = nullptr;
+  if (mask_host) {
+    int rc = ensure_stage(e, G);
+    if (rc) return rc;
+    memcpy(e->h_stage, mask_host, G);
+    CRL_CUDA(cudaMemcpyAsync(e->d_stage, e->h_stage, G, cudaMemcpyHostToDevice, e->stream));
+    mask_dev = (const u8*)e->d_stage;
+  }
+  int rc = launch_ab_move(e, mask_dev, depth, qdepth);
+  if (rc) return rc;
+  if (move_host) CRL_CUDA(cudaMemcpyAsync(move_host, e->ab_out_move, G * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (score_host) CRL_CUDA(cudaMemcpyAsync(score_host, e->ab_out_score, G * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (nodes_host) CRL_CUDA(cudaMemcpyAsync(nodes_host, e->ab_out_nodes, G * 8, cudaMemcpyDeviceToHost, e->stream));
+  CRL_CUDA(cudaStreamSynchronize(e->stream));
+  return CRL_OK;
+}
+
 int crl_set_reuse(crl_engine* e, int enable) {
   CHECK_ENGINE(e);
   if (enable && !e->P.nodes_prev) {

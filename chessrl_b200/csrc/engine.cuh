@@ -71,6 +71,17 @@ struct crl_engine_impl {
                                          // faster); CRL_PERFT_PAIR=5 / 6: the last two plies in one pass (k_perft_pair,
                                          // 96- / 80-register build)
   bool perft_pdl = true;                 // plies launched as programmatic dependent launches (CRL_NO_PDL=1: plain launches)
+  // fixed-depth alpha-beta (crl_games_ab_move_host): scratch allocated at the first call; items are lane * MAX_MOVES + k
+  u16* ab_moves = nullptr;               // [G][MAX_MOVES] root moves
+  int* ab_cnt = nullptr;                 // [G] root move count, -1 for a lane that is not searched
+  int* ab_items = nullptr;               // [G * MAX_MOVES] items of this call (k_ab_root appends them)
+  int* ab_score = nullptr;               // [G][MAX_MOVES] exact value of every root child
+  unsigned long long* ab_nodes = nullptr;   // [G][MAX_MOVES] positions visited below every root child
+  unsigned long long* ab_ctl = nullptr;  // [0] items, [1] items taken
+  u16* ab_out_move = nullptr;            // [G]
+  int* ab_out_score = nullptr;           // [G]
+  long long* ab_out_nodes = nullptr;     // [G]
+  int ab_grid = 0;                       // blocks of k_ab_items that fill the GPU
   // pinned staging
   void* h_stage = nullptr;
   size_t h_stage_bytes = 0;
@@ -138,6 +149,9 @@ int launch_perft_root(crl_engine_impl* e, const u64* root, u64* buf0, u64* buf1,
 int launch_encode_boards(crl_engine_impl* e, const u64* boards, const u64* hist, const u8* hist_len, int n,
                          __nv_bfloat16* planes);
 int launch_policy_index(crl_engine_impl* e, const u16* moves, const int* counts, int n, int16_t* idx);
+// fixed-depth alpha-beta of every lane with mask_dev[g] != 0 (null: all) that is active and unfinished; results in
+// e->ab_out_move / ab_out_score / ab_out_nodes (CRL_EINVAL for depth / qdepth out of range)
+int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth);
 int launch_hash_eval_boards(crl_engine_impl* e, const u64* boards, int n, u64 seed, int bits, float* policy,
                             float* value);
 

@@ -433,6 +433,25 @@ class Engine:
         torch.cuda.current_stream(self.device).synchronize()
         return picks
 
+    def games_ab_move(self, depth, qdepth=4, mask=None):
+        """Fixed-depth alpha-beta (DESIGN.md 3.6, include/chessrl_b200.h crl_games_ab_move_host) on the current position
+        of every active, unfinished lane with mask[g] != 0 (None = all lanes).  Plays nothing.
+        Returns numpy (moves uint16 [max_games], MOVE_NONE for lanes not searched; scores int32, centipawns for the side
+        to move, +-(32000 - plies) for a mate; nodes int64, positions visited)."""
+        G = self.max_games
+        moves = np.zeros(G, dtype=np.uint16)
+        scores = np.zeros(G, dtype=np.int32)
+        nodes = np.zeros(G, dtype=np.int64)
+        m = None
+        if mask is not None:
+            mask = np.ascontiguousarray(np.asarray(mask, dtype=np.uint8))
+            if mask.shape != (G,):
+                raise ValueError("mask: one entry per lane (%d), got shape %s" % (G, mask.shape))
+            m = _np(mask, ctypes.c_uint8)
+        check(self.lib.crl_games_ab_move_host(self.h, m, int(depth), int(qdepth), _np(moves, ctypes.c_uint16),
+                                              _np(scores, ctypes.c_int32), _np(nodes, ctypes.c_int64)))
+        return moves, scores, nodes
+
     def mcts_begin_move(self):
         check(self.lib.crl_mcts_begin_move(self.h))
 

@@ -218,6 +218,13 @@ int crl_games_legal_host(crl_engine* e, int first, int n, uint16_t* legal_host, 
 /* AgentDistributed.best_move(real_game=True) (agentdistributed.py:56-58): policy argmax over legal moves for
  * every game with mask_host[g] != 0 (NULL = all running games); writes picks_host [n_games] and plays them. */
 int crl_games_policy_move_host(crl_engine* e, const uint8_t* mask_host, uint16_t* picks_host);
+/* Fixed-depth alpha-beta (DESIGN.md 3.6) on the current position of every lane with mask_host[i] != 0 that is
+   active and unfinished: its move (MOVE_NONE for every other lane), its score in centipawns for the side to move
+   and the positions the search visited.  Plays nothing and leaves every other engine state unchanged.
+   CRL_EINVAL for depth / qdepth out of range (1..5 / 0..8).  mask_host NULL = all lanes; move_host [n_games],
+   score_host [n_games] and nodes_host [n_games] may each be NULL. */
+int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth,
+                           uint16_t* move_host, int32_t* score_host, int64_t* nodes_host);
 /* Two networks in one engine: a match between them in one lockstep batch (chessrl_b200/arena.py, DESIGN.md 3.5).
  *   crl_net_select_slot       : the network slot (0 or 1, else CRL_EINVAL) that crl_net_load_host,
  *                               crl_net_load_fp8_host, crl_net_calibrate_host, crl_net_set_precision, crl_set_evaluator,

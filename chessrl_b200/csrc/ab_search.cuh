@@ -211,4 +211,29 @@ CRL_HD bool ab_limits_ok(int depth, int qdepth) {
   return depth >= 1 && depth <= AB_MAX_DEPTH && qdepth >= 0 && qdepth <= AB_MAX_QDEPTH;
 }
 
+// ---- the seeded near-best root pick (DESIGN.md 3.7, crl_games_ab_pick_host) -------------------------------------------
+// s[0..n), n >= 1: the root children's scores in generation order; best = max s[k]; ply = meta_ply of the root record.
+//   the first k with s[k] = best        if margin = 0, ply >= pick_plies or |best| >= AB_MATE - AB_MAX_PLY - 1 (a mate);
+//   else C[mix64(salt + ply) mod |C|]   with C = [k : s[k] >= best - margin] in generation order.
+// Integer arithmetic only (best - s[k] <= margin cannot overflow: |s[k]| <= AB_INF), so the kernels, the g++ build and
+// oracle/ab_oracle.py agree bit for bit.
+CRL_HD int ab_pick_index(const int* s, int n, int ply, int margin, int pick_plies, u64 salt) {
+  int best = s[0], first = 0;
+  for (int k = 1; k < n; ++k)
+    if (s[k] > best) {
+      best = s[k];
+      first = k;
+    }
+  if (margin == 0 || ply >= pick_plies || best >= AB_MATE - AB_MAX_PLY - 1 || best <= -(AB_MATE - AB_MAX_PLY - 1))
+    return first;
+  unsigned c = 0;
+  for (int k = 0; k < n; ++k) c += best - s[k] <= margin;
+  unsigned r = (unsigned)(mix64(salt + (u64)ply) % c);
+  for (int k = 0; k < n; ++k)
+    if (best - s[k] <= margin && r-- == 0) return k;
+  return first;                                                          // (not reached: r < |C|)
+}
+
+CRL_HD bool ab_pick_ok(int margin, int pick_plies) { return margin >= 0 && pick_plies >= 0; }
+
 }  // namespace crl

@@ -982,6 +982,33 @@ int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, i
   return CRL_OK;
 }
 
+int crl_games_ab_pick_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, int margin, int pick_plies,
+                           const uint64_t* salt_host, uint16_t* move_host, int32_t* score_host, int64_t* nodes_host) {
+  CHECK_ENGINE(e);
+  const size_t G = e->G;
+  if (!salt_host) {
+    set_error("crl_games_ab_pick_host: salt_host is NULL (one salt per lane)");
+    return CRL_EINVAL;
+  }
+  // staging: the salts at offset 0, then the mask
+  int rc = ensure_stage(e, G * 9);
+  if (rc) return rc;
+  memcpy(e->h_stage, salt_host, G * 8);
+  const u8* mask_dev = nullptr;
+  if (mask_host) {
+    memcpy((char*)e->h_stage + G * 8, mask_host, G);
+    mask_dev = (const u8*)e->d_stage + G * 8;
+  }
+  CRL_CUDA(cudaMemcpyAsync(e->d_stage, e->h_stage, mask_host ? G * 9 : G * 8, cudaMemcpyHostToDevice, e->stream));
+  rc = launch_ab_move(e, mask_dev, depth, qdepth, (const u64*)e->d_stage, margin, pick_plies);
+  if (rc) return rc;
+  if (move_host) CRL_CUDA(cudaMemcpyAsync(move_host, e->ab_out_move, G * 2, cudaMemcpyDeviceToHost, e->stream));
+  if (score_host) CRL_CUDA(cudaMemcpyAsync(score_host, e->ab_out_score, G * 4, cudaMemcpyDeviceToHost, e->stream));
+  if (nodes_host) CRL_CUDA(cudaMemcpyAsync(nodes_host, e->ab_out_nodes, G * 8, cudaMemcpyDeviceToHost, e->stream));
+  CRL_CUDA(cudaStreamSynchronize(e->stream));
+  return CRL_OK;
+}
+
 int crl_set_reuse(crl_engine* e, int enable) {
   CHECK_ENGINE(e);
   if (enable && !e->P.nodes_prev) {

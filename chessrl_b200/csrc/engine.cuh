@@ -149,9 +149,9 @@ int launch_perft_root(crl_engine_impl* e, const u64* root, u64* buf0, u64* buf1,
 int launch_encode_boards(crl_engine_impl* e, const u64* boards, const u64* hist, const u8* hist_len, int n,
                          __nv_bfloat16* planes);
 int launch_policy_index(crl_engine_impl* e, const u16* moves, const int* counts, int n, int16_t* idx);
-// fixed-depth alpha-beta of every lane with mask_dev[g] != 0 (null: all) that is active and unfinished; results in
-// e->ab_out_move / ab_out_score / ab_out_nodes (CRL_EINVAL for depth / qdepth out of range)
-int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth);
+// fixed-depth alpha-beta of every active, unfinished lane with mask_dev[g] != 0 (null: all) into e->ab_out_*; salt_dev null:
+// the first maximum, else the seeded near-best pick of DESIGN.md 3.7 (a salt per lane).  CRL_EINVAL for out-of-range limits
+int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth, const u64* salt_dev = nullptr, int margin = 0, int pick_plies = 0);
 int launch_hash_eval_boards(crl_engine_impl* e, const u64* boards, int n, u64 seed, int bits, float* policy,
                             float* value);
 

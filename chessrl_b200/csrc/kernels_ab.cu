@@ -7,6 +7,7 @@
 //   k_ab_items   each thread takes the next item from an atomic counter until none is left (subtrees differ by orders
 //                of magnitude in size, so a fixed assignment would leave most threads idle behind the largest ones)
 //   k_ab_reduce  per lane: the first maximum, its move, its score and the positions visited
+//   k_ab_pick    in its place for crl_games_ab_pick_host: the seeded near-best pick (ab_search.cuh ab_pick_index)
 #include "engine.cuh"
 #include "ab_search.cuh"
 
@@ -79,6 +80,33 @@ __global__ void __launch_bounds__(AB_BLOCK) k_ab_reduce(int G, const int* __rest
   out_nodes[g] = (long long)total;
 }
 
+// k_ab_reduce with the seeded near-best pick of ab_pick_index (crl_games_ab_pick_host, DESIGN.md 3.7): salt[g] per lane,
+// ply from the lane's record; the score is the picked child's, the node count the same sum
+__global__ void __launch_bounds__(AB_BLOCK) k_ab_pick(const u64* __restrict__ cur, int G, const int* __restrict__ cnt,
+                                                      const u16* __restrict__ moves, const int* __restrict__ score,
+                                                      const unsigned long long* __restrict__ nodes,
+                                                      const u64* __restrict__ salt, int margin, int pick_plies,
+                                                      u16* __restrict__ out_move, int* __restrict__ out_score,
+                                                      long long* __restrict__ out_nodes) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= G) return;
+  const int n = cnt[g];
+  u16 mv = MOVE_NONE;
+  int sc = 0;
+  unsigned long long total = 0;
+  if (n > 0) {
+    const long long o = (long long)g * MAX_MOVES;
+    const int k = ab_pick_index(score + o, n, meta_ply(cur[8LL * G + g]), margin, pick_plies, salt[g]);
+    total = 1;
+    for (int i = 0; i < n; ++i) total += nodes[o + i];
+    mv = moves[o + k];
+    sc = score[o + k];
+  }
+  out_move[g] = mv;
+  out_score[g] = sc;
+  out_nodes[g] = (long long)total;
+}
+
 // scratch of the search, allocated at the first call (an engine that never searches holds none of it)
 static int ab_ensure(crl_engine_impl* e) {
   if (e->ab_moves) return CRL_OK;
@@ -113,10 +141,16 @@ static int ab_ensure(crl_engine_impl* e) {
   return CRL_OK;
 }
 
-int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth) {
+int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth, const u64* salt_dev, int margin,
+                   int pick_plies) {
+  const char* fn = salt_dev ? "crl_games_ab_pick_host" : "crl_games_ab_move_host";
   if (!ab_limits_ok(depth, qdepth)) {
-    set_error("crl_games_ab_move_host: depth %d / qdepth %d out of range (1..%d / 0..%d)", depth, qdepth, (int)AB_MAX_DEPTH,
+    set_error("%s: depth %d / qdepth %d out of range (1..%d / 0..%d)", fn, depth, qdepth, (int)AB_MAX_DEPTH,
               (int)AB_MAX_QDEPTH);
+    return CRL_EINVAL;
+  }
+  if (salt_dev && !ab_pick_ok(margin, pick_plies)) {
+    set_error("%s: margin %d / pick_plies %d must be >= 0", fn, margin, pick_plies);
     return CRL_EINVAL;
   }
   int rc = ab_ensure(e);
@@ -138,8 +172,14 @@ int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth
   }
   {
     LaunchScope ls(e, KC_MOVEGEN);
-    k_ab_reduce<<<div_up(e->G, AB_BLOCK), AB_BLOCK, 0, e->stream>>>(e->G, e->ab_cnt, e->ab_moves, e->ab_score, e->ab_nodes,
-                                                                    e->ab_out_move, e->ab_out_score, e->ab_out_nodes);
+    if (salt_dev)
+      k_ab_pick<<<div_up(e->G, AB_BLOCK), AB_BLOCK, 0, e->stream>>>(
+          e->P.g_cur, e->G, e->ab_cnt, e->ab_moves, e->ab_score, e->ab_nodes, salt_dev, margin, pick_plies,
+          e->ab_out_move, e->ab_out_score, e->ab_out_nodes);
+    else
+      k_ab_reduce<<<div_up(e->G, AB_BLOCK), AB_BLOCK, 0, e->stream>>>(e->G, e->ab_cnt, e->ab_moves, e->ab_score,
+                                                                      e->ab_nodes, e->ab_out_move, e->ab_out_score,
+                                                                      e->ab_out_nodes);
     CRL_CUDA(cudaGetLastError());
   }
   return CRL_OK;

@@ -452,6 +452,29 @@ class Engine:
                                               _np(scores, ctypes.c_int32), _np(nodes, ctypes.c_int64)))
         return moves, scores, nodes
 
+    def games_ab_pick(self, depth, qdepth, margin, pick_plies, salt, mask=None):
+        """games_ab_move with the seeded near-best root pick (DESIGN.md 3.7, include/chessrl_b200.h
+        crl_games_ab_pick_host): a lane at ply < pick_plies whose best score is not a mate plays one of the root moves
+        within `margin` centipawns of the best, chosen by splitmix64(salt[g] + ply); otherwise the first best move.
+        salt: one uint64 per lane.  Returns the same triple as games_ab_move; the score is the picked move's."""
+        G = self.max_games
+        s = np.ascontiguousarray(np.asarray(salt, dtype=np.uint64))
+        if s.shape != (G,):
+            raise ValueError("salt: one entry per lane (%d), got shape %s" % (G, s.shape))
+        moves = np.zeros(G, dtype=np.uint16)
+        scores = np.zeros(G, dtype=np.int32)
+        nodes = np.zeros(G, dtype=np.int64)
+        m = None
+        if mask is not None:
+            mask = np.ascontiguousarray(np.asarray(mask, dtype=np.uint8))
+            if mask.shape != (G,):
+                raise ValueError("mask: one entry per lane (%d), got shape %s" % (G, mask.shape))
+            m = _np(mask, ctypes.c_uint8)
+        check(self.lib.crl_games_ab_pick_host(self.h, m, int(depth), int(qdepth), int(margin), int(pick_plies),
+                                              _np(s, ctypes.c_uint64), _np(moves, ctypes.c_uint16),
+                                              _np(scores, ctypes.c_int32), _np(nodes, ctypes.c_int64)))
+        return moves, scores, nodes
+
     def mcts_begin_move(self):
         check(self.lib.crl_mcts_begin_move(self.h))
 

@@ -225,6 +225,14 @@ int crl_games_policy_move_host(crl_engine* e, const uint8_t* mask_host, uint16_t
    score_host [n_games] and nodes_host [n_games] may each be NULL. */
 int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth,
                            uint16_t* move_host, int32_t* score_host, int64_t* nodes_host);
+/* crl_games_ab_move_host with a seeded near-best root pick (DESIGN.md 3.7), for generating varied training games: a
+   lane at ply < pick_plies whose best score is not a mate plays one of the root moves scored within `margin`
+   centipawns of the best, chosen by splitmix64(salt_host[lane] + ply); otherwise the first best move, as
+   crl_games_ab_move_host.  score_host is the picked move's score; nodes_host is unchanged.  margin 0 gives
+   crl_games_ab_move_host's answer.  salt_host [n_games] is required.  CRL_EINVAL for the depth / qdepth limits above
+   and for margin < 0 or pick_plies < 0.  Plays nothing and leaves every other engine state unchanged. */
+int crl_games_ab_pick_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, int margin, int pick_plies,
+                           const uint64_t* salt_host, uint16_t* move_host, int32_t* score_host, int64_t* nodes_host);
 /* Two networks in one engine: a match between them in one lockstep batch (chessrl_b200/arena.py, DESIGN.md 3.5).
  *   crl_net_select_slot       : the network slot (0 or 1, else CRL_EINVAL) that crl_net_load_host,
  *                               crl_net_load_fp8_host, crl_net_calibrate_host, crl_net_set_precision, crl_set_evaluator,

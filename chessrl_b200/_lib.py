@@ -80,6 +80,8 @@ SIGNATURES = {
     "crl_games_ab_move_host": (ctypes.c_int, [vp, c_u8p, ctypes.c_int, ctypes.c_int, c_u16p, c_i32p, c_i64p]),
     "crl_games_ab_pick_host": (ctypes.c_int, [vp, c_u8p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_u64p,
                                               c_u16p, c_i32p, c_i64p]),
+    "crl_games_ab_search_host": (ctypes.c_int, [vp, c_u8p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                ctypes.c_int, c_u64p, c_u16p, c_i32p, c_i64p]),
     "crl_net_select_slot": (ctypes.c_int, [vp, ctypes.c_int]),
     "crl_games_set_players_host": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, c_u8p, c_u8p]),
     "crl_mcts_begin_move": (ctypes.c_int, [vp]),

@@ -12,8 +12,9 @@ strength that needs no weights.  Its moves come from Engine.games_ab_move on the
         [--precision-b bf16|fp8] [--opening-plies P | --openings FILE] [--max-plies M] [--seed X] [--out match.json]
 
 A and B are weights files (.h5) or model directories (their newest model-<n>.h5); they may be the same file with
-different precisions, which measures what fp8 evaluation costs in playing strength.  `alphabeta[:D[:Q]]` in place of
-either names the alpha-beta opponent at depth D and quiescence depth Q (default alphabeta:3:4).
+different precisions, which measures what fp8 evaluation costs in playing strength.  `alphabeta[:D[:Q[:r]]]` in place
+of either names the alpha-beta opponent at depth D and quiescence depth Q (default alphabeta:3:4); a trailing `:r` has it
+score repeated positions inside its search as draws (DESIGN.md 3.6, off by default).
 """
 
 from __future__ import annotations
@@ -50,11 +51,13 @@ class AlphaBetaPlayer:
     """The fixed-depth alpha-beta opponent (include/chessrl_b200.h crl_games_ab_move_host): material and position
     evaluation, `depth` full-width plies (1..5), then up to `qdepth` plies of captures and queen promotions (0..8).
     Deterministic: the same position gives the same move.  It searches on the lanes' own positions and needs no network
-    slot."""
+    slot.  repetitions: a position inside the search that repeats an earlier one of its reversible run, in the game or
+    on the search path, scores 0 (crl_games_ab_search_host CRL_AB_REPETITIONS); the move then depends on the game too."""
 
-    def __init__(self, depth=AB_DEPTH, qdepth=AB_QDEPTH):
+    def __init__(self, depth=AB_DEPTH, qdepth=AB_QDEPTH, repetitions=False):
         self.depth = int(depth)
         self.qdepth = int(qdepth)
+        self.repetitions = bool(repetitions)
         if not (1 <= self.depth <= 5 and 0 <= self.qdepth <= 8):
             raise ValueError("alpha-beta depth 1..5 and qdepth 0..8, not %d / %d" % (self.depth, self.qdepth))
 
@@ -62,28 +65,32 @@ class AlphaBetaPlayer:
 
     @classmethod
     def parse(cls, spec):
-        """'alphabeta', 'alphabeta:D' or 'alphabeta:D:Q' -> AlphaBetaPlayer; None for any other string."""
+        """'alphabeta', 'alphabeta:D', 'alphabeta:D:Q' or 'alphabeta:D:Q:r' -> AlphaBetaPlayer; None for any other
+        string."""
         parts = spec.split(":")
-        if parts[0] != cls.SPEC or len(parts) > 3:
+        if parts[0] != cls.SPEC or len(parts) > 4:
             return None
         try:
-            nums = [int(p) for p in parts[1:]]
+            if len(parts) == 4 and parts[3] != "r":
+                raise ValueError
+            nums = [int(p) for p in parts[1:3]]
         except ValueError:
-            raise ValueError("alpha-beta player: 'alphabeta[:D[:Q]]', not %r" % (spec,))
-        return cls(*nums)
+            raise ValueError("alpha-beta player: 'alphabeta[:D[:Q[:r]]]', not %r" % (spec,))
+        return cls(*nums, repetitions=len(parts) == 4)
 
     def __str__(self):
-        return "%s:%d:%d" % (self.SPEC, self.depth, self.qdepth)
+        return "%s:%d:%d%s" % (self.SPEC, self.depth, self.qdepth, ":r" if self.repetitions else "")
 
     __repr__ = __str__
 
     def moves(self, engine, mask):
         """This player's moves in the lanes of `mask` (MOVE_NONE elsewhere)."""
-        return engine.games_ab_move(self.depth, self.qdepth, mask=mask.astype(np.uint8))[0]
+        kw = {"repetitions": True} if self.repetitions else {}
+        return engine.games_ab_move(self.depth, self.qdepth, mask=mask.astype(np.uint8), **kw)[0]
 
 
 def _as_player(x):
-    """A ChessModel, an Agent, a weights path, a model directory, 'alphabeta[:D[:Q]]', a HashPlayer or an
+    """A ChessModel, an Agent, a weights path, a model directory, 'alphabeta[:D[:Q[:r]]]', a HashPlayer or an
     AlphaBetaPlayer -> HashPlayer, AlphaBetaPlayer or ChessModel."""
     from .model import ChessModel
     from .selfplay import get_model_path
@@ -298,7 +305,7 @@ def _read_openings(path):
 
 
 def _label(arg, precision):
-    """How a CLI player is reported: 'alphabeta:D:Q' (its full parameters) or 'path (precision)'."""
+    """How a CLI player is reported: 'alphabeta:D:Q[:r]' (its full parameters) or 'path (precision)'."""
     ab = AlphaBetaPlayer.parse(arg)
     return str(ab) if ab is not None else "%s (%s)" % (arg, precision)
 
@@ -307,8 +314,8 @@ def main(argv=None):
     ap = argparse.ArgumentParser(description="Plays a search-vs-search match between two networks, or a network and the "
                                              "alpha-beta opponent, and prints the score and the Elo difference A - B with "
                                              "its 95 % interval.")
-    ap.add_argument("a", help="weights file (.h5) or model directory of player A, or alphabeta[:D[:Q]]")
-    ap.add_argument("b", help="weights file (.h5) or model directory of player B (may be A's), or alphabeta[:D[:Q]]")
+    ap.add_argument("a", help="weights file (.h5) or model directory of player A, or alphabeta[:D[:Q[:r]]]")
+    ap.add_argument("b", help="weights file (.h5) or model directory of player B (may be A's), or alphabeta[:D[:Q[:r]]]")
     ap.add_argument("--games", type=int, required=True)
     ap.add_argument("--lanes", type=int, default=None, help="concurrent games (default: one per game)")
     ap.add_argument("--sims", type=int, default=100, help="simulations per move")

@@ -9,7 +9,7 @@ the fixed yardstick that stands in for Stockfish.  `workers` concurrent games be
 engine; every ply of every running game is one batched network evaluation or one batched alpha-beta call.
 
     python -m chessrl_b200.benchmark modeldir [--games 10] [--workers 2]
-        [--opponent random|path/to/weights.h5|alphabeta[:D[:Q]]]
+        [--opponent random|path/to/weights.h5|alphabeta[:D[:Q[:r]]]]
 """
 
 from __future__ import annotations
@@ -40,7 +40,7 @@ def _as_model(x):
 
 def play_policy_games(agent, opponent="random", games=10, lanes=None, seed=None, device=None, max_plies=2000):
     """`games` games, agent (policy argmax) versus `opponent` ("random"; a ChessModel / Agent / weights path that
-    also moves by policy argmax; or an AlphaBetaPlayer / 'alphabeta[:D[:Q]]', searched on the agent's engine).  The
+    also moves by policy argmax; or an AlphaBetaPlayer / 'alphabeta[:D[:Q[:r]]]', searched on the agent's engine).  The
     agent's colour is drawn per game like benchmark.py:70.
     Returns one dict per game in game order: {'color', 'result' (white point of view, None if capped), 'moves'}."""
     from .engine import Engine
@@ -150,7 +150,7 @@ def main(argv=None):
     ap.add_argument("--games", type=int, default=10)
     ap.add_argument("--workers", type=int, default=2, help="concurrent games (lockstep lanes)")
     ap.add_argument("--opponent", default="random",
-                    help="'random', a path to the opponent's weights, or alphabeta[:D[:Q]] (fixed-depth alpha-beta)")
+                    help="'random', a path to the opponent's weights, or alphabeta[:D[:Q[:r]]] (fixed-depth alpha-beta)")
     ap.add_argument("--seed", type=int, default=None)
     args = ap.parse_args(argv)
     print(benchmark(args.model_dir, workers=args.workers, games=args.games, log=True, opponent=args.opponent, seed=args.seed))

@@ -7,6 +7,10 @@
 //   s(p)     centipawns for the side to move: its pieces minus the opponent's (table in ab_eval_side)
 //   T(p, h)  game_result(b, n_legal, in_check, 0): mate -(AB_MATE - h) for the side to move; stalemate, insufficient
 //            material and the fifty-move claim 0.  h = plies from the search root; repetitions are not tracked.
+//            With repetitions on (R, crl_games_ab_search_host CRL_AB_REPETITIONS): a position h >= 1 plies below the
+//            root that repeats an earlier position of its reversible run (on the search path, the root included, or in
+//            the game before the root) scores 0 before anything else, counts as one visited position and generates no
+//            moves -- python-chess's board.is_repetition(2) on the game's moves followed by the path.
 //   V(p,d,h) = T(p,h) if terminal;  Q(p,q,h) if d = 0;  max over legal m of -V(p.m, d-1, h+1)
 //   Q(p,k,h) = T(p,h) if terminal;  s(p) if k = 0;  max over legal m of -Q(p.m, k-1, h+1) if in check (no stand-pat);
 //              else max(s(p), max over m in C(p) of -Q(p.m, k-1, h+1)),  C(p) = legal captures (en passant included)
@@ -130,9 +134,40 @@ struct AbStack {
   int alpha[AB_MAX_PLY + 1], beta[AB_MAX_PLY + 1], best[AB_MAX_PLY];
 };
 
+// The repetition window of one search with R on (kept apart from AbStack, which the plain search uses as it is).
+//   key[L]    transposition key of the position at stack level L, stored for a node that has children a repetition
+//             could reach (level L + 4 <= d + q)
+//   game[i]   key of the position i plies before the root, i = 0..ngame (game[0]: the root, its key as the game
+//             recorded it, en passant included); ngame = min(revlen, ply) of the root record
+// A repetition needs the same side to move and a reversible run of at least 4 plies, so a node compares its key with
+// the positions 4, 6, .. plies above it, back to its own revlen.  A node whose run is non-empty has no en-passant square,
+// so its key is position_key(b, 0) and needs no move generation.
+enum { AB_REP_KEYS = 100 };   // game[] entries per lane: a searched root's reversible run is < 100 plies (fifty-move rule)
+struct AbPath {
+  u64 key[AB_MAX_PLY];
+  const u64* game;
+  int ngame;
+};
+
+// does the node at `level` (h = level + 1 plies below the root, revlen rev >= 4, key `key`) repeat an earlier position?
+CRL_HD bool ab_repeats(const AbPath& path, u64 key, int level, int h, int rev) {
+  for (int j = 4; j <= rev; j += 2) {
+    if (j <= level) {
+      if (path.key[level - j] == key) return true;
+    } else {
+      if (j - h > path.ngame) return false;
+      if (path.game[j - h] == key) return true;
+    }
+  }
+  return false;
+}
+
 // V(p, d, h0) of st.b[0] (d = 0: Q(p, q, h0)) with a full window; requires d + q <= AB_MAX_PLY.
 // *nodes += the positions visited (every position whose legal moves were generated, p included).
-CRL_HD int ab_value(AbStack& st, int d, int q, int h0, unsigned long long* nodes) {
+// REP: repetitions on, with the window in *path; requires h0 == 1 (st.b[0] is a root child, as in ab_root_child): the
+// positions above level 0 are then the root and the game before it, path->game[j - h] in ab_repeats.
+template <bool REP = false>
+CRL_HD int ab_value(AbStack& st, int d, int q, int h0, unsigned long long* nodes, AbPath* path = nullptr) {
   int level = 0, v = 0;
   bool done = false;                 // v is the value of the node at `level`
   st.alpha[0] = -AB_INF;
@@ -145,6 +180,18 @@ CRL_HD int ab_value(AbStack& st, int d, int q, int h0, unsigned long long* nodes
       const bool qnode = level >= d;
       const int k = qnode ? q - (level - d) : 0;
       *nodes += 1;
+      u64 key = 0;
+      if constexpr (REP) {
+        const int rev = meta_revlen(b.meta);
+        if (rev >= 4) {
+          key = position_key(b, 0);
+          if (ab_repeats(*path, key, level, h, rev)) {
+            v = 0;
+            done = true;
+            continue;
+          }
+        }
+      }
       if (qnode && k == 0) {
         CountSink cs{0};
         const GenInfo gi = generate_legal(b, cs);
@@ -157,6 +204,9 @@ CRL_HD int ab_value(AbStack& st, int d, int q, int h0, unsigned long long* nodes
       if (ab_terminal(b, ss.n, gi.in_check, h, &v)) {
         done = true;
         continue;
+      }
+      if constexpr (REP) {
+        if (level + 4 <= d + q) path->key[level] = meta_revlen(b.meta) >= 4 ? key : position_key(b, gi.ep_legal);
       }
       int best = -AB_INF;
       const bool stand = qnode && !gi.in_check;
@@ -201,10 +251,12 @@ CRL_HD int ab_value(AbStack& st, int d, int q, int h0, unsigned long long* nodes
 }
 
 // the score of root child `mv` at search depth D: -V(root.mv, D - 1, 1)
-CRL_HD int ab_root_child(AbStack& st, const Board& root, u16 mv, int depth, int qdepth, unsigned long long* nodes) {
+template <bool REP = false>
+CRL_HD int ab_root_child(AbStack& st, const Board& root, u16 mv, int depth, int qdepth, unsigned long long* nodes,
+                         AbPath* path = nullptr) {
   st.b[0] = root;
   make_move(st.b[0], mv);
-  return -ab_value(st, depth - 1, qdepth, 1, nodes);
+  return -ab_value<REP>(st, depth - 1, qdepth, 1, nodes, path);
 }
 
 CRL_HD bool ab_limits_ok(int depth, int qdepth) {

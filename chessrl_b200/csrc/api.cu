@@ -961,19 +961,26 @@ int crl_games_policy_move_host(crl_engine* e, const uint8_t* mask_host, uint16_t
   return check_pool_errors(e);
 }
 
-int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, uint16_t* move_host,
-                           int32_t* score_host, int64_t* nodes_host) {
-  CHECK_ENGINE(e);
+// crl_games_ab_move_host (salt_host NULL), crl_games_ab_pick_host and crl_games_ab_search_host: stage the salts (offset
+// 0) and the mask, search, copy the outputs back
+static int ab_search_host(crl_engine* e, const char* fn, const uint8_t* mask_host, int depth, int qdepth, bool reps,
+                          int margin, int pick_plies, const uint64_t* salt_host, uint16_t* move_host,
+                          int32_t* score_host, int64_t* nodes_host) {
   const size_t G = e->G;
+  const size_t off = salt_host ? G * 8 : 0;
   const u8* mask_dev = nullptr;
-  if (mask_host) {
-    int rc = ensure_stage(e, G);
+  if (salt_host || mask_host) {
+    int rc = ensure_stage(e, off + G);
     if (rc) return rc;
-    memcpy(e->h_stage, mask_host, G);
-    CRL_CUDA(cudaMemcpyAsync(e->d_stage, e->h_stage, G, cudaMemcpyHostToDevice, e->stream));
-    mask_dev = (const u8*)e->d_stage;
+    if (salt_host) memcpy(e->h_stage, salt_host, G * 8);
+    if (mask_host) {
+      memcpy((char*)e->h_stage + off, mask_host, G);
+      mask_dev = (const u8*)e->d_stage + off;
+    }
+    CRL_CUDA(cudaMemcpyAsync(e->d_stage, e->h_stage, off + (mask_host ? G : 0), cudaMemcpyHostToDevice, e->stream));
   }
-  int rc = launch_ab_move(e, mask_dev, depth, qdepth);
+  int rc = launch_ab_move(e, mask_dev, depth, qdepth, salt_host ? (const u64*)e->d_stage : nullptr, margin, pick_plies,
+                          reps, fn);
   if (rc) return rc;
   if (move_host) CRL_CUDA(cudaMemcpyAsync(move_host, e->ab_out_move, G * 2, cudaMemcpyDeviceToHost, e->stream));
   if (score_host) CRL_CUDA(cudaMemcpyAsync(score_host, e->ab_out_score, G * 4, cudaMemcpyDeviceToHost, e->stream));
@@ -982,31 +989,40 @@ int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, i
   return CRL_OK;
 }
 
+int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, uint16_t* move_host,
+                           int32_t* score_host, int64_t* nodes_host) {
+  CHECK_ENGINE(e);
+  return ab_search_host(e, "crl_games_ab_move_host", mask_host, depth, qdepth, false, 0, 0, nullptr, move_host,
+                        score_host, nodes_host);
+}
+
 int crl_games_ab_pick_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, int margin, int pick_plies,
                            const uint64_t* salt_host, uint16_t* move_host, int32_t* score_host, int64_t* nodes_host) {
   CHECK_ENGINE(e);
-  const size_t G = e->G;
   if (!salt_host) {
     set_error("crl_games_ab_pick_host: salt_host is NULL (one salt per lane)");
     return CRL_EINVAL;
   }
-  // staging: the salts at offset 0, then the mask
-  int rc = ensure_stage(e, G * 9);
-  if (rc) return rc;
-  memcpy(e->h_stage, salt_host, G * 8);
-  const u8* mask_dev = nullptr;
-  if (mask_host) {
-    memcpy((char*)e->h_stage + G * 8, mask_host, G);
-    mask_dev = (const u8*)e->d_stage + G * 8;
+  return ab_search_host(e, "crl_games_ab_pick_host", mask_host, depth, qdepth, false, margin, pick_plies, salt_host,
+                        move_host, score_host, nodes_host);
+}
+
+int crl_games_ab_search_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, int flags, int margin,
+                             int pick_plies, const uint64_t* salt_host, uint16_t* move_host, int32_t* score_host,
+                             int64_t* nodes_host) {
+  CHECK_ENGINE(e);
+  const char* fn = "crl_games_ab_search_host";
+  if (flags & ~CRL_AB_REPETITIONS) {
+    set_error("%s: unknown flag bits 0x%x", fn, (unsigned)(flags & ~CRL_AB_REPETITIONS));
+    return CRL_EINVAL;
   }
-  CRL_CUDA(cudaMemcpyAsync(e->d_stage, e->h_stage, mask_host ? G * 9 : G * 8, cudaMemcpyHostToDevice, e->stream));
-  rc = launch_ab_move(e, mask_dev, depth, qdepth, (const u64*)e->d_stage, margin, pick_plies);
-  if (rc) return rc;
-  if (move_host) CRL_CUDA(cudaMemcpyAsync(move_host, e->ab_out_move, G * 2, cudaMemcpyDeviceToHost, e->stream));
-  if (score_host) CRL_CUDA(cudaMemcpyAsync(score_host, e->ab_out_score, G * 4, cudaMemcpyDeviceToHost, e->stream));
-  if (nodes_host) CRL_CUDA(cudaMemcpyAsync(nodes_host, e->ab_out_nodes, G * 8, cudaMemcpyDeviceToHost, e->stream));
-  CRL_CUDA(cudaStreamSynchronize(e->stream));
-  return CRL_OK;
+  if (!salt_host && (margin || pick_plies)) {
+    set_error("%s: margin %d / pick_plies %d without salt_host (they apply to the seeded pick only)", fn, margin,
+              pick_plies);
+    return CRL_EINVAL;
+  }
+  return ab_search_host(e, fn, mask_host, depth, qdepth, (flags & CRL_AB_REPETITIONS) != 0, margin, pick_plies,
+                        salt_host, move_host, score_host, nodes_host);
 }
 
 int crl_set_reuse(crl_engine* e, int enable) {

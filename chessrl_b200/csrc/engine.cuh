@@ -82,6 +82,10 @@ struct crl_engine_impl {
   int* ab_out_score = nullptr;           // [G]
   long long* ab_out_nodes = nullptr;     // [G]
   int ab_grid = 0;                       // blocks of k_ab_items that fill the GPU
+  // repetitions on (crl_games_ab_search_host CRL_AB_REPETITIONS): allocated at the first such call
+  u64* ab_rep_keys = nullptr;            // [G][AB_REP_KEYS] keys of each searched root's reversible run, root first
+  int* ab_rep_n = nullptr;               // [G] earlier positions staged per lane
+  int ab_rep_grid = 0;                   // blocks of k_ab_items<true> that fill the GPU
   // pinned staging
   void* h_stage = nullptr;
   size_t h_stage_bytes = 0;
@@ -150,8 +154,10 @@ int launch_encode_boards(crl_engine_impl* e, const u64* boards, const u64* hist,
                          __nv_bfloat16* planes);
 int launch_policy_index(crl_engine_impl* e, const u16* moves, const int* counts, int n, int16_t* idx);
 // fixed-depth alpha-beta of every active, unfinished lane with mask_dev[g] != 0 (null: all) into e->ab_out_*; salt_dev null:
-// the first maximum, else the seeded near-best pick of DESIGN.md 3.7 (a salt per lane).  CRL_EINVAL for out-of-range limits
-int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth, const u64* salt_dev = nullptr, int margin = 0, int pick_plies = 0);
+// the first maximum, else the seeded near-best pick of DESIGN.md 3.7 (a salt per lane); reps: repetitions scored 0
+// (DESIGN.md 3.6).  CRL_EINVAL for out-of-range limits, reported as function `fn`
+int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth, const u64* salt_dev, int margin,
+                   int pick_plies, bool reps, const char* fn);
 int launch_hash_eval_boards(crl_engine_impl* e, const u64* boards, int n, u64 seed, int bits, float* policy,
                             float* value);
 

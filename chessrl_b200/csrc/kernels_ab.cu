@@ -8,6 +8,9 @@
 //                of magnitude in size, so a fixed assignment would leave most threads idle behind the largest ones)
 //   k_ab_reduce  per lane: the first maximum, its move, its score and the positions visited
 //   k_ab_pick    in its place for crl_games_ab_pick_host: the seeded near-best pick (ab_search.cuh ab_pick_index)
+// With repetitions on (crl_games_ab_search_host, CRL_AB_REPETITIONS) k_ab_rep_stage copies the keys of each searched
+// root's reversible run out of the lane's key ring, and k_ab_items<true> scores a repeated position 0.  The plain
+// search launches exactly what it launched before.
 #include "engine.cuh"
 #include "ab_search.cuh"
 
@@ -34,10 +37,29 @@ __global__ void __launch_bounds__(AB_BLOCK) k_ab_root(Pools P, const u8* __restr
   }
 }
 
+// per searched lane g (cnt[g] > 0): rep_keys[g][i] = the key of the position i plies before the root, i = 0..rep_n[g],
+// rep_n[g] = min(revlen, ply) of the root record (the ring holds ply q in slot q % KEY_RING)
+__global__ void __launch_bounds__(AB_BLOCK) k_ab_rep_stage(Pools P, const int* __restrict__ cnt,
+                                                           u64* __restrict__ rep_keys, int* __restrict__ rep_n) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= P.G || cnt[g] <= 0) return;
+  const u64 meta = P.g_cur[8LL * P.G + g];
+  const int ply = meta_ply(meta);
+  int n = meta_revlen(meta);
+  if (n > ply) n = ply;
+  if (n > AB_REP_KEYS - 1) n = AB_REP_KEYS - 1;
+  for (int i = 0; i <= n; ++i)
+    rep_keys[(long long)g * AB_REP_KEYS + i] = P.g_keys[(long long)((ply - i) % KEY_RING) * P.G + g];
+  rep_n[g] = n;
+}
+
+// REP: repetitions on, with the staged keys of k_ab_rep_stage (unused by the plain search)
+template <bool REP>
 __global__ void __launch_bounds__(AB_BLOCK) k_ab_items(const u64* __restrict__ cur, int G, const u16* __restrict__ moves,
                                                        const int* __restrict__ items, int* __restrict__ score,
                                                        unsigned long long* __restrict__ nodes,
-                                                       unsigned long long* __restrict__ ctl, int depth, int qdepth) {
+                                                       unsigned long long* __restrict__ ctl, int depth, int qdepth,
+                                                       const u64* __restrict__ rep_keys, const int* __restrict__ rep_n) {
   AbStack st;
   const unsigned long long total = ctl[0];
   for (;;) {
@@ -45,7 +67,15 @@ __global__ void __launch_bounds__(AB_BLOCK) k_ab_items(const u64* __restrict__ c
     if (it >= total) return;
     const int w = items[it];
     unsigned long long nn = 0;
-    score[w] = ab_root_child(st, load_soa(cur, G, w / MAX_MOVES), moves[w], depth, qdepth, &nn);
+    if constexpr (REP) {
+      const int g = w / MAX_MOVES;
+      AbPath path;
+      path.game = rep_keys + (long long)g * AB_REP_KEYS;
+      path.ngame = rep_n[g];
+      score[w] = ab_root_child<true>(st, load_soa(cur, G, g), moves[w], depth, qdepth, &nn, &path);
+    } else {
+      score[w] = ab_root_child(st, load_soa(cur, G, w / MAX_MOVES), moves[w], depth, qdepth, &nn);
+    }
     nodes[w] = nn;
   }
 }
@@ -113,7 +143,7 @@ static int ab_ensure(crl_engine_impl* e) {
   // enough threads to fill the GPU; each takes items until none is left
   int dev_sms = 0, per_sm = 0;
   CRL_CUDA(cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, e->device));
-  CRL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_ab_items, AB_BLOCK, 0));
+  CRL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_ab_items<false>, AB_BLOCK, 0));
   e->ab_grid = dev_sms * (per_sm > 0 ? per_sm : 1);
   const size_t items = (size_t)e->G * MAX_MOVES;
   const size_t bytes = items * (2 + 4 + 4 + 8) + (size_t)e->G * (4 + 2 + 4 + 8) + 16 * 8 + 64 * 10;
@@ -141,9 +171,28 @@ static int ab_ensure(crl_engine_impl* e) {
   return CRL_OK;
 }
 
+// scratch of the repetition window, allocated at the first call with repetitions on
+static int ab_rep_ensure(crl_engine_impl* e) {
+  if (e->ab_rep_keys) return CRL_OK;
+  int dev_sms = 0, per_sm = 0;
+  CRL_CUDA(cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, e->device));
+  CRL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_ab_items<true>, AB_BLOCK, 0));
+  e->ab_rep_grid = dev_sms * (per_sm > 0 ? per_sm : 1);
+  const size_t keys = (size_t)e->G * AB_REP_KEYS * 8, bytes = keys + (size_t)e->G * 4 + 64;
+  char* p = nullptr;
+  cudaError_t err = cudaMalloc(&p, bytes);
+  if (err != cudaSuccess) {
+    set_error("crl_games_ab_search_host: cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(err));
+    return CRL_ENOMEM;
+  }
+  e->allocs.push_back(p);
+  e->ab_rep_keys = (u64*)p;
+  e->ab_rep_n = (int*)(p + (keys + 63) / 64 * 64);
+  return CRL_OK;
+}
+
 int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth, const u64* salt_dev, int margin,
-                   int pick_plies) {
-  const char* fn = salt_dev ? "crl_games_ab_pick_host" : "crl_games_ab_move_host";
+                   int pick_plies, bool reps, const char* fn) {
   if (!ab_limits_ok(depth, qdepth)) {
     set_error("%s: depth %d / qdepth %d out of range (1..%d / 0..%d)", fn, depth, qdepth, (int)AB_MAX_DEPTH,
               (int)AB_MAX_QDEPTH);
@@ -155,6 +204,10 @@ int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth
   }
   int rc = ab_ensure(e);
   if (rc) return rc;
+  if (reps) {
+    rc = ab_rep_ensure(e);
+    if (rc) return rc;
+  }
   CRL_CUDA(cudaMemsetAsync(e->ab_ctl, 0, 2 * sizeof(unsigned long long), e->stream));
   {
     LaunchScope ls(e, KC_MOVEGEN);
@@ -162,12 +215,23 @@ int launch_ab_move(crl_engine_impl* e, const u8* mask_dev, int depth, int qdepth
                                                                   e->ab_ctl);
     CRL_CUDA(cudaGetLastError());
   }
+  if (reps) {
+    LaunchScope ls(e, KC_MOVEGEN);
+    k_ab_rep_stage<<<div_up(e->G, AB_BLOCK), AB_BLOCK, 0, e->stream>>>(e->P, e->ab_cnt, e->ab_rep_keys, e->ab_rep_n);
+    CRL_CUDA(cudaGetLastError());
+  }
   {
     // no more threads than items could exist (a few lanes need a few blocks)
     const int want = div_up((long long)e->G * MAX_MOVES, AB_BLOCK);
     LaunchScope ls(e, KC_MOVEGEN);
-    k_ab_items<<<want < e->ab_grid ? want : e->ab_grid, AB_BLOCK, 0, e->stream>>>(
-        e->P.g_cur, e->G, e->ab_moves, e->ab_items, e->ab_score, e->ab_nodes, e->ab_ctl, depth, qdepth);
+    if (reps)
+      k_ab_items<true><<<want < e->ab_rep_grid ? want : e->ab_rep_grid, AB_BLOCK, 0, e->stream>>>(
+          e->P.g_cur, e->G, e->ab_moves, e->ab_items, e->ab_score, e->ab_nodes, e->ab_ctl, depth, qdepth,
+          e->ab_rep_keys, e->ab_rep_n);
+    else
+      k_ab_items<false><<<want < e->ab_grid ? want : e->ab_grid, AB_BLOCK, 0, e->stream>>>(
+          e->P.g_cur, e->G, e->ab_moves, e->ab_items, e->ab_score, e->ab_nodes, e->ab_ctl, depth, qdepth, nullptr,
+          nullptr);
     CRL_CUDA(cudaGetLastError());
   }
   {

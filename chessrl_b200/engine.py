@@ -27,6 +27,7 @@ def _np(a, ctype):
 
 
 NET_SLOTS = 2      # CRL_NET_SLOTS: networks one engine holds (include/chessrl_b200.h crl_net_select_slot)
+CRL_AB_REPETITIONS = 1   # crl_games_ab_search_host flag: repetitions below the root score 0 (DESIGN.md 3.6)
 
 
 class Engine:
@@ -433,46 +434,69 @@ class Engine:
         torch.cuda.current_stream(self.device).synchronize()
         return picks
 
-    def games_ab_move(self, depth, qdepth=4, mask=None):
+    def games_ab_move(self, depth, qdepth=4, mask=None, repetitions=False):
         """Fixed-depth alpha-beta (DESIGN.md 3.6, include/chessrl_b200.h crl_games_ab_move_host) on the current position
         of every active, unfinished lane with mask[g] != 0 (None = all lanes).  Plays nothing.
+        repetitions: a position below the root that repeats an earlier one of its reversible run (on the search path or
+        in the lane's game) scores 0 (crl_games_ab_search_host CRL_AB_REPETITIONS).
         Returns numpy (moves uint16 [max_games], MOVE_NONE for lanes not searched; scores int32, centipawns for the side
         to move, +-(32000 - plies) for a mate; nodes int64, positions visited)."""
+        if repetitions:
+            return self.games_ab_search(depth, qdepth, CRL_AB_REPETITIONS, 0, 0, None, mask)
         G = self.max_games
         moves = np.zeros(G, dtype=np.uint16)
         scores = np.zeros(G, dtype=np.int32)
         nodes = np.zeros(G, dtype=np.int64)
-        m = None
-        if mask is not None:
-            mask = np.ascontiguousarray(np.asarray(mask, dtype=np.uint8))
-            if mask.shape != (G,):
-                raise ValueError("mask: one entry per lane (%d), got shape %s" % (G, mask.shape))
-            m = _np(mask, ctypes.c_uint8)
+        m = self._ab_mask(mask)
         check(self.lib.crl_games_ab_move_host(self.h, m, int(depth), int(qdepth), _np(moves, ctypes.c_uint16),
                                               _np(scores, ctypes.c_int32), _np(nodes, ctypes.c_int64)))
         return moves, scores, nodes
 
-    def games_ab_pick(self, depth, qdepth, margin, pick_plies, salt, mask=None):
+    def games_ab_pick(self, depth, qdepth, margin, pick_plies, salt, mask=None, repetitions=False):
         """games_ab_move with the seeded near-best root pick (DESIGN.md 3.7, include/chessrl_b200.h
         crl_games_ab_pick_host): a lane at ply < pick_plies whose best score is not a mate plays one of the root moves
         within `margin` centipawns of the best, chosen by splitmix64(salt[g] + ply); otherwise the first best move.
-        salt: one uint64 per lane.  Returns the same triple as games_ab_move; the score is the picked move's."""
+        salt: one uint64 per lane.  repetitions: as in games_ab_move.  Returns the same triple as games_ab_move; the
+        score is the picked move's."""
         G = self.max_games
         s = np.ascontiguousarray(np.asarray(salt, dtype=np.uint64))
         if s.shape != (G,):
             raise ValueError("salt: one entry per lane (%d), got shape %s" % (G, s.shape))
+        if repetitions:
+            return self.games_ab_search(depth, qdepth, CRL_AB_REPETITIONS, margin, pick_plies, s, mask)
         moves = np.zeros(G, dtype=np.uint16)
         scores = np.zeros(G, dtype=np.int32)
         nodes = np.zeros(G, dtype=np.int64)
-        m = None
-        if mask is not None:
-            mask = np.ascontiguousarray(np.asarray(mask, dtype=np.uint8))
-            if mask.shape != (G,):
-                raise ValueError("mask: one entry per lane (%d), got shape %s" % (G, mask.shape))
-            m = _np(mask, ctypes.c_uint8)
+        m = self._ab_mask(mask)
         check(self.lib.crl_games_ab_pick_host(self.h, m, int(depth), int(qdepth), int(margin), int(pick_plies),
                                               _np(s, ctypes.c_uint64), _np(moves, ctypes.c_uint16),
                                               _np(scores, ctypes.c_int32), _np(nodes, ctypes.c_int64)))
+        return moves, scores, nodes
+
+    def _ab_mask(self, mask):
+        if mask is None:
+            return None
+        mask = np.ascontiguousarray(np.asarray(mask, dtype=np.uint8))
+        if mask.shape != (self.max_games,):
+            raise ValueError("mask: one entry per lane (%d), got shape %s" % (self.max_games, mask.shape))
+        return _np(mask, ctypes.c_uint8)                 # (the pointer keeps the array alive)
+
+    def games_ab_search(self, depth, qdepth, flags=0, margin=0, pick_plies=0, salt=None, mask=None):
+        """include/chessrl_b200.h crl_games_ab_search_host: games_ab_move (salt None; margin and pick_plies must be 0)
+        or games_ab_pick (a salt per lane) with option bits `flags` (CRL_AB_REPETITIONS).  Returns the same triple."""
+        G = self.max_games
+        if salt is not None:
+            salt = np.ascontiguousarray(np.asarray(salt, dtype=np.uint64))
+            if salt.shape != (G,):
+                raise ValueError("salt: one entry per lane (%d), got shape %s" % (G, salt.shape))
+        moves = np.zeros(G, dtype=np.uint16)
+        scores = np.zeros(G, dtype=np.int32)
+        nodes = np.zeros(G, dtype=np.int64)
+        m = self._ab_mask(mask)
+        check(self.lib.crl_games_ab_search_host(self.h, m, int(depth), int(qdepth), int(flags), int(margin),
+                                                int(pick_plies), None if salt is None else _np(salt, ctypes.c_uint64),
+                                                _np(moves, ctypes.c_uint16), _np(scores, ctypes.c_int32),
+                                                _np(nodes, ctypes.c_int64)))
         return moves, scores, nodes
 
     def mcts_begin_move(self):

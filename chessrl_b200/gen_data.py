@@ -6,9 +6,11 @@ while fewer than `pick_plies` plies have been played, a side may play any root m
 the best one (never when the best score is a mate), chosen by a per-game salt.  Every ply is still a move the search
 rates as near-best, so every ply is a fair policy target.  Game j's salt is splitmix64(base + j), with base drawn from
 the seed as in arena, so the games depend only on the seed and the parameters -- not on the lanes or the number of GPUs.
+With --repetitions the search scores a position that repeats an earlier one of its reversible run as a draw (DESIGN.md
+3.6), so a side that is ahead stops repeating moves; it is off by default.
 
     python -m chessrl_b200.gen_data OUT.json --games N [--lanes L] [--depth 3] [--qdepth 4] [--margin CP]
-        [--pick-plies P] [--max-plies M] [--seed S]
+        [--pick-plies P] [--max-plies M] [--seed S] [--repetitions]
 
 OUT.json is the DatasetGame format that `supervised` reads; games are appended to what the file holds, in game order.
 Under torchrun the games are sharded by rank and gathered to rank 0, which writes the file.
@@ -87,11 +89,12 @@ def summarize(facts, wall_s):
 
 
 def generate_games(n_games, lanes=None, depth=DEPTH, qdepth=QDEPTH, margin=MARGIN, pick_plies=PICK_PLIES,
-                   max_plies=MAX_PLIES, seed=None, first=0, device=None, engine=None):
+                   max_plies=MAX_PLIES, seed=None, first=0, device=None, engine=None, repetitions=False):
     """Games first..first+n_games-1 of the alpha-beta player against itself with the seeded near-best pick, `lanes` at
     a time on one engine (default: a new Engine on `device` with no tree).  A game that reaches `max_plies` plies stops
     unfinished.  Every step makes one Engine.games_ab_pick call for all running lanes -- both colours -- and plays the
     picks with one games_play; finished games are harvested, and their lanes start the next game or are parked.
+    repetitions: the search scores repeated positions 0 (Engine.games_ab_pick repetitions=True).
 
     Returns (games in game order, summary).  A game is {'moves' (UCI), 'result' (white's point of view, None if
     unfinished), 'player_color' (game index even), 'end' (one of ENDS)}."""
@@ -107,6 +110,7 @@ def generate_games(n_games, lanes=None, depth=DEPTH, qdepth=QDEPTH, margin=MARGI
     if e.max_games < lanes:
         raise ValueError("the engine has %d lanes, %d asked for" % (e.max_games, lanes))
     salts = game_salts(seed, first, n_games)
+    kw = {"repetitions": True} if repetitions else {}
     out = [None] * n_games
     t0 = time.perf_counter()
     try:
@@ -144,7 +148,7 @@ def generate_games(n_games, lanes=None, depth=DEPTH, qdepth=QDEPTH, margin=MARGI
                 if not live.any():
                     break
                 continue
-            e.games_play(e.games_ab_pick(depth, qdepth, margin, pick_plies, salt)[0])
+            e.games_play(e.games_ab_pick(depth, qdepth, margin, pick_plies, salt, **kw)[0])
     finally:
         if own:
             e.close()
@@ -176,6 +180,8 @@ def main(argv=None):
     ap.add_argument("--pick-plies", type=int, default=PICK_PLIES, help="plies of each game that use the margin")
     ap.add_argument("--max-plies", type=int, default=MAX_PLIES, help="a game stops here, unfinished (result null)")
     ap.add_argument("--seed", type=int, default=None, help="default: drawn at random and printed")
+    ap.add_argument("--repetitions", action="store_true",
+                    help="the search scores a position that repeats an earlier one of its reversible run as a draw")
     args = ap.parse_args(argv)
     if args.games <= 0 or args.margin < 0 or args.pick_plies < 0 or args.max_plies <= 0:
         ap.error("--games and --max-plies must be positive, --margin and --pick-plies non-negative")
@@ -200,7 +206,7 @@ def main(argv=None):
     if hi > lo:
         games, s = generate_games(hi - lo, lanes=args.lanes, depth=args.depth, qdepth=args.qdepth, margin=args.margin,
                                   pick_plies=args.pick_plies, max_plies=args.max_plies, seed=seed, first=lo,
-                                  device=local_rank)
+                                  device=local_rank, repetitions=args.repetitions)
         wall = s["wall_s"]
     facts = tally(games)
     data = to_dataset(games)
@@ -212,7 +218,8 @@ def main(argv=None):
         data = sharding.gather_games(data)
     summary = summarize(facts, wall)
     summary.update({"seed": seed, "depth": args.depth, "qdepth": args.qdepth, "margin": args.margin,
-                    "pick_plies": args.pick_plies, "max_plies": args.max_plies, "ranks": world})
+                    "pick_plies": args.pick_plies, "max_plies": args.max_plies, "repetitions": args.repetitions,
+                    "ranks": world})
     if rank == 0:
         data.save(args.out)
         s = summary

@@ -233,6 +233,20 @@ int crl_games_ab_move_host(crl_engine* e, const uint8_t* mask_host, int depth, i
    and for margin < 0 or pick_plies < 0.  Plays nothing and leaves every other engine state unchanged. */
 int crl_games_ab_pick_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, int margin, int pick_plies,
                            const uint64_t* salt_host, uint16_t* move_host, int32_t* score_host, int64_t* nodes_host);
+/* The alpha-beta search of crl_games_ab_move_host / crl_games_ab_pick_host with options in `flags`:
+ *   CRL_AB_REPETITIONS  a position at least one ply below the root that repeats an earlier position of its reversible
+ *                       run -- on the search path, the root included, or in the lane's game before the root, back to the
+ *                       last irreversible move -- scores 0 (python-chess's board.is_repetition(2) on the game's moves
+ *                       followed by the path; DESIGN.md 3.6).  It counts as one visited position and generates no
+ *                       moves.  The root itself is never scored by the rule.
+ * salt_host NULL: the first best move, and margin and pick_plies must be 0.  Otherwise the seeded near-best pick of
+ * crl_games_ab_pick_host.  With flags 0 the outputs equal those two calls'.  CRL_EINVAL for unknown flag bits, the
+ * depth / qdepth limits, margin < 0 or pick_plies < 0, and a margin or pick_plies without a salt.  Plays nothing and
+ * leaves every other engine state unchanged. */
+#define CRL_AB_REPETITIONS 1
+int crl_games_ab_search_host(crl_engine* e, const uint8_t* mask_host, int depth, int qdepth, int flags,
+                             int margin, int pick_plies, const uint64_t* salt_host,
+                             uint16_t* move_host, int32_t* score_host, int64_t* nodes_host);
 /* Two networks in one engine: a match between them in one lockstep batch (chessrl_b200/arena.py, DESIGN.md 3.5).
  *   crl_net_select_slot       : the network slot (0 or 1, else CRL_EINVAL) that crl_net_load_host,
  *                               crl_net_load_fp8_host, crl_net_calibrate_host, crl_net_set_precision, crl_set_evaluator,

@@ -1,7 +1,8 @@
 """Compares the SASS of two builds kernel by kernel: `python scripts/sass_compare.py OLD.sass NEW.sass`, each the output
 of `cuobjdump -sass` on an object file.  Instructions are compared with their addresses and encodings stripped; k_trunk4
-instantiations are matched by their template arguments, a missing FP8 argument counting as false (the bf16 tower), and
-k_encode_rows by its bf16 form.  Prints one line per kernel: identical, DIFFERENT or new."""
+instantiations are matched by their template arguments, a missing FP8 argument counting as false (the bf16 tower),
+k_encode_rows by its bf16 form, and k_ab_items by its repetition argument, the untemplated kernel counting as false
+(the plain search).  Prints one line per kernel: identical, DIFFERENT or new."""
 import re
 import sys
 
@@ -25,6 +26,9 @@ def key(name):
         return "k_trunk4<%s,%s,%s,%s>" % (m.group(1), m.group(2), m.group(3), m.group(4) or "0")
     if re.match(r"_ZN3crl13k_encode_rows(ENS_5Pools|I13__nv_bfloat16E)", name):
         return "k_encode_rows<bf16>"
+    m = re.match(r"_ZN3crl10k_ab_items(?:ILb(\d)EE)?", name)
+    if m:
+        return "k_ab_items<%s>" % (m.group(1) or "0")
     return name
 
 

@@ -57,6 +57,7 @@ SIGNATURES = {
                                                     c_u64p, c_i32p]),
     "crl_encode": (ctypes.c_int, [vp, vp, vp, vp, ctypes.c_int, vp]),
     "crl_policy_index": (ctypes.c_int, [vp, vp, vp, ctypes.c_int, vp]),
+    "crl_search_targets": (ctypes.c_int, [vp, vp, vp, vp, ctypes.c_int, ctypes.c_float, vp, vp, vp]),
     "crl_label_table_host": (ctypes.c_int, [vp, c_i16p]),
     "crl_net_load_host": (ctypes.c_int, [vp, ctypes.POINTER(c_f32p), c_i64p, ctypes.c_int]),
     "crl_net_forward": (ctypes.c_int, [vp, vp, ctypes.c_int, vp, vp]),
@@ -82,6 +83,7 @@ SIGNATURES = {
                                               c_u16p, c_i32p, c_i64p]),
     "crl_games_ab_search_host": (ctypes.c_int, [vp, c_u8p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                 ctypes.c_int, c_u64p, c_u16p, c_i32p, c_i64p]),
+    "crl_games_ab_root_scores_host": (ctypes.c_int, [vp, c_i32p, c_i32p]),
     "crl_net_select_slot": (ctypes.c_int, [vp, ctypes.c_int]),
     "crl_games_set_players_host": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int, c_u8p, c_u8p]),
     "crl_mcts_begin_move": (ctypes.c_int, [vp]),

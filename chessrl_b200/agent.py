@@ -19,14 +19,15 @@ class Agent(AgentDistributed):
         # the working search of AgentDistributed is used instead
         return super().best_move(game, real_game=real_game, max_iters=max_iters, ai_move=ai_move, verbose=verbose)
 
-    def train(self, dataset: DatasetGame, epochs=1, logdir=None, batch_size=1, validation_split=0):
+    def train(self, dataset: DatasetGame, epochs=1, logdir=None, batch_size=1, validation_split=0, targets=None):
         """Trains the model on recorded games (agent.py:64-89): one sample per ply, targets = the move played and the
-        white-point-of-view result."""
+        white-point-of-view result, or with targets=training.SearchTargets(...) the search targets of DESIGN.md 3.8
+        for games that carry root scores."""
         if len(dataset) <= 0:
             return
         from . import training
         training.train(self.model, dataset, epochs=epochs, logdir=logdir, batch_size=batch_size,
-                       validation_split=validation_split)
+                       validation_split=validation_split, targets=targets)
 
     def save(self, path):
         self.model.save_weights(path)

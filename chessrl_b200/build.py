@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libchessrl_b200.so")
 SOURCES = ["api.cu", "kernels_rules.cu", "kernels_encode.cu", "kernels_tree.cu", "net.cu", "kernels_ab.cu"]
-HEADERS = ["engine.cuh", "chess_core.cuh", "tree_core.cuh", "hash_eval.cuh", "ab_search.cuh", os.path.join("..", "..", "include", "chessrl_b200.h")]
+HEADERS = ["engine.cuh", "chess_core.cuh", "tree_core.cuh", "hash_eval.cuh", "ab_search.cuh", "search_targets.cuh", os.path.join("..", "..", "include", "chessrl_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
          "--fmad=true", "-Xptxas", "-v"]

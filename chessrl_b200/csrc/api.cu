@@ -220,6 +220,12 @@ using namespace crl;
     if (_d != cudaSuccess) return cuda_fail(_d, "cudaSetDevice"); \
   } while (0)
 
+// kernels_encode.cu (declared here rather than in engine.cuh, whose lines the other kernels' line info refers to)
+namespace crl {
+int launch_search_targets(crl_engine_impl* e, const u64* boards, const int* scores, const int* offsets, int n,
+                          float temperature, float* policy, float* score_value, int* legal_count);
+}
+
 extern "C" {
 
 const char* crl_last_error(void) { return g_err; }
@@ -576,6 +582,21 @@ int crl_policy_index(crl_engine* e, const uint16_t* moves_dev, const int32_t* co
     return CRL_EINVAL;
   }
   return launch_policy_index(e, moves_dev, counts_dev, n, idx_dev);
+}
+int crl_search_targets(crl_engine* e, const uint64_t* boards_dev, const int32_t* scores_dev, const int32_t* offsets_dev,
+                       int n, float temperature, float* policy_dev, float* score_value_dev, int32_t* legal_count_dev) {
+  CHECK_ENGINE(e);
+  if (n < 0 || (n > 0 && (!boards_dev || !scores_dev || !offsets_dev || !policy_dev || !score_value_dev ||
+                          !legal_count_dev))) {
+    set_error("crl_search_targets: bad arguments");
+    return CRL_EINVAL;
+  }
+  if (!(temperature > 0.0f) || !isfinite(temperature)) {
+    set_error("crl_search_targets: temperature %g must be positive and finite", (double)temperature);
+    return CRL_EINVAL;
+  }
+  return launch_search_targets(e, boards_dev, scores_dev, offsets_dev, n, temperature, policy_dev, score_value_dev,
+                               legal_count_dev);
 }
 int crl_label_table_host(crl_engine* e, int16_t* idx_host) {
   if (!idx_host) {
@@ -1023,6 +1044,27 @@ int crl_games_ab_search_host(crl_engine* e, const uint8_t* mask_host, int depth,
   }
   return ab_search_host(e, fn, mask_host, depth, qdepth, (flags & CRL_AB_REPETITIONS) != 0, margin, pick_plies,
                         salt_host, move_host, score_host, nodes_host);
+}
+
+int crl_games_ab_root_scores_host(crl_engine* e, int32_t* scores_host, int32_t* counts_host) {
+  CHECK_ENGINE(e);
+  if (!scores_host || !counts_host) {
+    set_error("crl_games_ab_root_scores_host: null output");
+    return CRL_EINVAL;
+  }
+  if (!e->ab_moves) {
+    set_error("crl_games_ab_root_scores_host: no alpha-beta call has run on this engine");
+    return CRL_ESTATE;
+  }
+  const size_t G = e->G;
+  CRL_CUDA(cudaMemcpyAsync(scores_host, e->ab_score, G * MAX_MOVES * 4, cudaMemcpyDeviceToHost, e->stream));
+  CRL_CUDA(cudaMemcpyAsync(counts_host, e->ab_cnt, G * 4, cudaMemcpyDeviceToHost, e->stream));
+  CRL_CUDA(cudaStreamSynchronize(e->stream));
+  for (size_t g = 0; g < G; ++g) {                   // entries past a lane's count hold older calls' scores
+    const int c = counts_host[g] > 0 ? counts_host[g] : 0;
+    memset(scores_host + g * MAX_MOVES + c, 0, (MAX_MOVES - c) * 4);
+  }
+  return CRL_OK;
 }
 
 int crl_set_reuse(crl_engine* e, int enable) {

@@ -12,6 +12,7 @@
 // 2 KB contiguous span per block-wide store.
 #include "engine.cuh"
 #include "hash_eval.cuh"
+#include "search_targets.cuh"
 
 namespace crl {
 
@@ -155,6 +156,58 @@ __global__ void k_policy_index(const u16* __restrict__ moves, const int* __restr
     if (m != MOVE_NONE && mv_promo(m) < 5) v = label_of[(int)mv_promo(m) * 4096 + mv_from(m) * 64 + mv_to(m)];
   }
   idx[t] = v;
+}
+
+// ---- search targets (crl_search_targets, DESIGN.md 3.8) -----------------------------------------------------
+// One block per row.  Thread 0 regenerates the legal moves into shared memory and reduces best and the sum in
+// generation order (search_targets.cuh); meanwhile the block zero-fills the row.  After the barrier each thread
+// scatters some of the n probabilities.  A row's bits depend on its own inputs only.
+static constexpr int ST_THREADS = 128;
+__global__ void __launch_bounds__(ST_THREADS) k_search_targets(const u64* __restrict__ boards,
+                                                               const int* __restrict__ scores,
+                                                               const int* __restrict__ offsets, int n,
+                                                               float temperature, const int16_t* __restrict__ label_of,
+                                                               float* __restrict__ policy,
+                                                               float* __restrict__ score_value,
+                                                               int* __restrict__ legal_count) {
+  __shared__ u16 s_moves[MAX_MOVES];
+  __shared__ SearchRowStats s_r;
+  __shared__ int s_n;
+  const int i = blockIdx.x;
+  const int o = offsets[i], ns = offsets[i + 1] - o;
+  const int* s = scores + o;
+  float* row = policy + (long long)i * CRL_N_LABELS;
+  if (threadIdx.x == 0) {
+    const Board b = load_soa(boards, n, i);
+    StoreSink sink{s_moves, 0};
+    generate_legal(b, sink);
+    legal_count[i] = sink.n;
+    float v = 0.0f;
+    int use = 0;                                       // a count mismatch leaves the row zero (the caller reports it)
+    if (sink.n == ns && ns > 0) {
+      s_r = search_row_stats(s, ns, temperature);
+      v = search_score_value(s_r.best, meta_turn(b.meta));
+      use = ns;
+    }
+    s_n = use;
+    score_value[i] = v;
+  }
+  for (int l = threadIdx.x; l < CRL_N_LABELS; l += ST_THREADS) row[l] = 0.0f;
+  __syncthreads();
+  for (int k = threadIdx.x; k < s_n; k += ST_THREADS) {
+    const int l = search_label(label_of, s_moves[k]);
+    if (l >= 0) row[l] = search_prob(s[k], s_r, temperature);
+  }
+}
+
+int launch_search_targets(crl_engine_impl* e, const u64* boards, const int* scores, const int* offsets, int n,
+                          float temperature, float* policy, float* score_value, int* legal_count) {
+  if (n <= 0) return CRL_OK;
+  LaunchScope ls(e, KC_ENCODE);
+  k_search_targets<<<n, ST_THREADS, 0, e->stream>>>(boards, scores, offsets, n, temperature, e->d_label_of, policy,
+                                                     score_value, legal_count);
+  CRL_CUDA(cudaGetLastError());
+  return CRL_OK;
 }
 
 // ---- deterministic test evaluator ---------------------------------------------------------------------

@@ -171,6 +171,19 @@ class Engine:
         check(self.lib.crl_policy_index(self.h, _ptr(moves_t), _ptr(counts_t), n, _ptr(idx)))
         return idx
 
+    def search_targets(self, boards_t, scores_t, offsets_t, temperature):
+        """Policy and score-value targets from root scores (DESIGN.md 3.8, include/chessrl_b200.h crl_search_targets):
+        boards_t uint64 SoA [9, n] on the device, scores_t int32 (all rows' scores concatenated), offsets_t int32 [n+1].
+        Returns device tensors (policy float32 [n, 1968], score value float32 [n], legal count int32 [n]); a row whose
+        legal count differs from its score count is all zeros.  Does not synchronise."""
+        n = boards_t.shape[1]
+        policy = torch.empty((n, _lib.N_LABELS), dtype=torch.float32, device=self.device)
+        value = torch.empty(n, dtype=torch.float32, device=self.device)
+        count = torch.empty(n, dtype=torch.int32, device=self.device)
+        check(self.lib.crl_search_targets(self.h, _ptr(boards_t), _ptr(scores_t), _ptr(offsets_t), n, float(temperature),
+                                          _ptr(policy), _ptr(value), _ptr(count)))
+        return policy, value, count
+
     def label_table(self):
         t = np.zeros(5 * 4096, dtype=np.int16)
         check(self.lib.crl_label_table_host(self.h, _np(t, ctypes.c_int16)))
@@ -498,6 +511,15 @@ class Engine:
                                                 _np(moves, ctypes.c_uint16), _np(scores, ctypes.c_int32),
                                                 _np(nodes, ctypes.c_int64)))
         return moves, scores, nodes
+
+    def games_ab_root_scores(self):
+        """The exact value of every root child from the most recent games_ab_* call (include/chessrl_b200.h
+        crl_games_ab_root_scores_host): numpy (scores int32 [max_games, MAX_MOVES] in generation order, 0 past a lane's
+        count; counts int32 [max_games], -1 for lanes that call did not search)."""
+        scores = np.zeros((self.max_games, B.MAX_MOVES), dtype=np.int32)
+        counts = np.zeros(self.max_games, dtype=np.int32)
+        check(self.lib.crl_games_ab_root_scores_host(self.h, _np(scores, ctypes.c_int32), _np(counts, ctypes.c_int32)))
+        return scores, counts
 
     def mcts_begin_move(self):
         check(self.lib.crl_mcts_begin_move(self.h))

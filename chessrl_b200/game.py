@@ -80,6 +80,9 @@ class Game(object):
     NULL_MOVE = B.NULL_MOVE
     WHITE = True
     BLACK = False
+    # the alpha-beta root scores of every ply (DESIGN.md 3.8): one list of ints per move, the scores of that ply's legal
+    # moves in generation order; None for a game recorded without them (copies and new games)
+    search_scores = None
 
     def __init__(self, board=None, player_color=True, date=None):
         self.player_color = player_color
@@ -105,6 +108,7 @@ class Game(object):
             # bulk load: the kernel hands back the record after every accepted ply (crl_game_replay_records_host)
             r = eng.game_replay(self._start, words, records=True)
             self._moves = [m for m, ok in zip(cand, r["accepted"]) if ok]
+            self._accepted = r["accepted"][n_old:]        # of `extra` (DatasetGame.loads aligns scores with it)
             self._records = [rec.copy() for rec in r["records"]]
             played = len(self._moves) > n_old
         else:
@@ -149,8 +153,11 @@ class Game(object):
         return moves
 
     def get_history(self):
-        return {"moves": list(self._moves), "result": self.get_result(), "player_color": self.player_color,
-                "date": self.date}
+        h = {"moves": list(self._moves), "result": self.get_result(), "player_color": self.player_color,
+             "date": self.date}
+        if self.search_scores is not None:
+            h["scores"] = [list(s) for s in self.search_scores]
+        return h
 
     def get_fen(self):
         return B.board_fen_from_record(self._record)

@@ -7,10 +7,12 @@ the best one (never when the best score is a mate), chosen by a per-game salt.  
 rates as near-best, so every ply is a fair policy target.  Game j's salt is splitmix64(base + j), with base drawn from
 the seed as in arena, so the games depend only on the seed and the parameters -- not on the lanes or the number of GPUs.
 With --repetitions the search scores a position that repeats an earlier one of its reversible run as a draw (DESIGN.md
-3.6), so a side that is ahead stops repeating moves; it is off by default.
+3.6), so a side that is ahead stops repeating moves; it is off by default.  With --scores every game also records the
+search's root scores of each ply (DESIGN.md 3.8): the exact value of every legal move, the data of soft policy and score
+value targets (supervised --targets search); the games themselves are the same.
 
     python -m chessrl_b200.gen_data OUT.json --games N [--lanes L] [--depth 3] [--qdepth 4] [--margin CP]
-        [--pick-plies P] [--max-plies M] [--seed S] [--repetitions]
+        [--pick-plies P] [--max-plies M] [--seed S] [--repetitions] [--scores]
 
 OUT.json is the DatasetGame format that `supervised` reads; games are appended to what the file holds, in game order.
 Under torchrun the games are sharded by rank and gathered to rank 0, which writes the file.
@@ -89,12 +91,15 @@ def summarize(facts, wall_s):
 
 
 def generate_games(n_games, lanes=None, depth=DEPTH, qdepth=QDEPTH, margin=MARGIN, pick_plies=PICK_PLIES,
-                   max_plies=MAX_PLIES, seed=None, first=0, device=None, engine=None, repetitions=False):
+                   max_plies=MAX_PLIES, seed=None, first=0, device=None, engine=None, repetitions=False, scores=False):
     """Games first..first+n_games-1 of the alpha-beta player against itself with the seeded near-best pick, `lanes` at
     a time on one engine (default: a new Engine on `device` with no tree).  A game that reaches `max_plies` plies stops
     unfinished.  Every step makes one Engine.games_ab_pick call for all running lanes -- both colours -- and plays the
     picks with one games_play; finished games are harvested, and their lanes start the next game or are parked.
     repetitions: the search scores repeated positions 0 (Engine.games_ab_pick repetitions=True).
+    scores: after every pick call one Engine.games_ab_root_scores call records the root scores of the ply each lane is
+    about to play; a game then also has 'scores', one int32 array per ply (the scores of its legal moves in generation
+    order).  The per-step work is a few array operations over all lanes; the arrays are split per game at the end.
 
     Returns (games in game order, summary).  A game is {'moves' (UCI), 'result' (white's point of view, None if
     unfinished), 'player_color' (game index even), 'end' (one of ENDS)}."""
@@ -112,6 +117,7 @@ def generate_games(n_games, lanes=None, depth=DEPTH, qdepth=QDEPTH, margin=MARGI
     salts = game_salts(seed, first, n_games)
     kw = {"repetitions": True} if repetitions else {}
     out = [None] * n_games
+    kept = []                  # with scores: per pick call (game, ply, count, the counts' scores concatenated)
     t0 = time.perf_counter()
     try:
         e.games_set(np.tile(B.record_from_fen(), (e.max_games, 1)))
@@ -148,21 +154,48 @@ def generate_games(n_games, lanes=None, depth=DEPTH, qdepth=QDEPTH, margin=MARGI
                 if not live.any():
                     break
                 continue
-            e.games_play(e.games_ab_pick(depth, qdepth, margin, pick_plies, salt, **kw)[0])
+            picks = e.games_ab_pick(depth, qdepth, margin, pick_plies, salt, **kw)[0]
+            if scores:
+                sc, cnt = e.games_ab_root_scores()
+                lanes_s = np.nonzero(cnt > 0)[0]
+                c = cnt[lanes_s]
+                kept.append((lane_game[lanes_s], plies[lanes_s], c, sc[lanes_s][_COLS[None, :] < c[:, None]]))
+            e.games_play(picks)
     finally:
         if own:
             e.close()
+    if scores:
+        _attach_scores(out, kept)
     return out, summarize(tally(out), time.perf_counter() - t0)
 
 
+_COLS = np.arange(B.MAX_MOVES)
+
+
+def _attach_scores(games, kept):
+    """games[j]['scores'] = the recorded score arrays of game j, one per ply in ply order."""
+    game, ply, cnt, flat = (np.concatenate(part) for part in zip(*kept))     # (every run makes a pick call)
+    start = np.zeros(len(cnt) + 1, dtype=np.int64)
+    start[1:] = np.cumsum(cnt)
+    order = np.lexsort((ply, game))
+    bounds = np.searchsorted(game[order], np.arange(len(games) + 1))
+    for j, g in enumerate(games):
+        rows = order[bounds[j]:bounds[j + 1]]
+        assert np.array_equal(ply[rows], np.arange(len(g["moves"]))), j
+        g["scores"] = [flat[start[r]:start[r + 1]] for r in rows]
+
+
 def to_dataset(games):
-    """The games as a DatasetGame (each replayed once on the device, as selfplay.LockstepRun.dataset does)."""
+    """The games as a DatasetGame (each replayed once on the device, as selfplay.LockstepRun.dataset does); recorded
+    scores become Game.search_scores."""
     from .dataset import DatasetGame
     from .game import Game
     data = DatasetGame()
     for g in games:
         gm = Game(player_color=g["player_color"])
         gm._sync(extra=g["moves"])
+        if "scores" in g:
+            gm.search_scores = [s.tolist() for s in g["scores"]]
         data.append(gm)
     return data
 
@@ -182,6 +215,8 @@ def main(argv=None):
     ap.add_argument("--seed", type=int, default=None, help="default: drawn at random and printed")
     ap.add_argument("--repetitions", action="store_true",
                     help="the search scores a position that repeats an earlier one of its reversible run as a draw")
+    ap.add_argument("--scores", action="store_true",
+                    help="record the search's score of every legal move at every ply (training targets, DESIGN.md 3.8)")
     args = ap.parse_args(argv)
     if args.games <= 0 or args.margin < 0 or args.pick_plies < 0 or args.max_plies <= 0:
         ap.error("--games and --max-plies must be positive, --margin and --pick-plies non-negative")
@@ -206,20 +241,29 @@ def main(argv=None):
     if hi > lo:
         games, s = generate_games(hi - lo, lanes=args.lanes, depth=args.depth, qdepth=args.qdepth, margin=args.margin,
                                   pick_plies=args.pick_plies, max_plies=args.max_plies, seed=seed, first=lo,
-                                  device=local_rank, repetitions=args.repetitions)
+                                  device=local_rank, repetitions=args.repetitions, scores=args.scores)
         wall = s["wall_s"]
     facts = tally(games)
     data = to_dataset(games)
     if world > 1:
         gathered = [None] * world
-        dist.all_gather_object(gathered, (facts, wall))
-        facts = [f for part, _ in gathered for f in part]
-        wall = max(w for _, w in gathered)                 # the ranks generate concurrently
+        scores = [g.search_scores for g in data.games] if args.scores else None
+        dist.all_gather_object(gathered, (facts, wall, scores))
+        facts = [f for part, _, _ in gathered for f in part]
+        wall = max(w for _, w, _ in gathered)              # the ranks generate concurrently
         data = sharding.gather_games(data)
+        if args.scores and rank == 0:                      # gather_games keeps rank order, then game order
+            lists = [s for _, _, part in gathered for s in part]
+            if len(lists) != len(data.games):
+                raise RuntimeError("gathered %d games but %d score lists" % (len(data.games), len(lists)))
+            for g, s in zip(data.games, lists):
+                g.search_scores = s
     summary = summarize(facts, wall)
     summary.update({"seed": seed, "depth": args.depth, "qdepth": args.qdepth, "margin": args.margin,
                     "pick_plies": args.pick_plies, "max_plies": args.max_plies, "repetitions": args.repetitions,
                     "ranks": world})
+    if args.scores:
+        summary["scores"] = True
     if rank == 0:
         data.save(args.out)
         s = summary

@@ -1,10 +1,13 @@
 """supervised: drop-in for the reference's entry point (supervised.py:36-95)
 
     python -m chessrl_b200.supervised modeldir datadir [--epochs 1] [--bs 8] [--debug]
+        [--targets played|search] [--temperature 50] [--value-weight 0.5]
 
 Contract kept: `train(model_dir, dataset_path, epochs=1, batch_size=8)` resumes from the newest `model-<n>.h5` of the
 directory (or starts fresh when there is none), trains with a 25 % validation split and writes the weights back under
 the same name; the same command-line flags.  The training step itself is chessrl_b200/training.py.
+--targets search (opt-in) trains games recorded by `gen_data --scores` on the search's soft policy and score-value targets
+(DESIGN.md 3.8); the default, played, is the reference's one-hot of the move played and the game's result.
 """
 
 from __future__ import annotations
@@ -28,6 +31,12 @@ _FLAGS = (
     (("--precision",), dict(choices=("fp32", "tf32", "bf16"), default=None,
                             help="arithmetic of the training step (default fp32 = the parity setting; tf32 / bf16 run the "
                                  "convolutions on the tensor cores, 8-10 x faster, gradients no longer parity-grade)")),
+    (("--targets",), dict(choices=("played", "search"), default="played",
+                          help="played: one-hot of the move played and the result (default); search: softmax of the "
+                               "recorded root scores and a score-blended value (games from gen_data --scores)")),
+    (("--temperature",), dict(type=float, default=50.0, help="search targets: softmax temperature in centipawns")),
+    (("--value-weight",), dict(type=float, default=0.5,
+                               help="search targets: weight w of tanh(score / 400) in the value target, 0..1")),
 )
 
 
@@ -41,7 +50,13 @@ def _resume(weights_file):
         return agent, False
 
 
-def train(model_dir, dataset_path, epochs=1, batch_size=8):
+def train(model_dir, dataset_path, epochs=1, batch_size=8, targets="played", temperature=50.0, value_weight=0.5):
+    """targets "played" (the reference's) or "search" (DESIGN.md 3.8, with `temperature` and `value_weight`)."""
+    from . import training
+    if targets not in ("played", "search"):
+        raise ValueError("targets: 'played' or 'search', got %r" % (targets,))
+    search = training.check_targets(training.SearchTargets(float(temperature), float(value_weight))) \
+        if targets == "search" else None
     log = Logger.get_instance()
     games = DatasetGame()
     games.load(dataset_path)
@@ -52,7 +67,11 @@ def train(model_dir, dataset_path, epochs=1, batch_size=8):
         log.info("resuming from %s" % weights_file)
     else:
         log.warning("no checkpoint at %s: training a fresh model" % weights_file)
-    agent.train(games, epochs=epochs, batch_size=batch_size, validation_split=VALIDATION_SPLIT, logdir=model_dir)
+    if search is not None:
+        log.info("search targets: %d of %d games carry root scores"
+                 % (sum(g.search_scores is not None for g in games.games), len(games)))
+    agent.train(games, epochs=epochs, batch_size=batch_size, validation_split=VALIDATION_SPLIT, logdir=model_dir,
+                targets=search)
     agent.save(weights_file)
     log.info("weights written to %s" % weights_file)
 
@@ -65,7 +84,8 @@ def main(argv=None):
     Logger.get_instance().set_level(0 if opts.debug else 1)
     if opts.precision:
         os.environ["CRL_TRAIN_PRECISION"] = opts.precision
-    train(opts.model_dir, opts.data_path, epochs=opts.epochs, batch_size=opts.bs)
+    train(opts.model_dir, opts.data_path, epochs=opts.epochs, batch_size=opts.bs, targets=opts.targets,
+          temperature=opts.temperature, value_weight=opts.value_weight)
 
 
 if __name__ == "__main__":

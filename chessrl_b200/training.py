@@ -12,8 +12,11 @@ planes are rotated by 180 degrees with probability 0.1 while the policy target i
 from __future__ import annotations
 
 import contextlib
+import itertools
+import math
 import os
 import random
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -22,6 +25,8 @@ import torch.nn.functional as F
 from . import boards as B
 from . import runtime
 from .netencoder import get_uci_labels
+
+N_LABELS = 1968
 
 L2 = 0.01
 BN_EPS = 1e-3
@@ -213,6 +218,77 @@ def encode_games(games, flips, device=None):
     return planes, torch.from_numpy(pol).to(eng.device), torch.from_numpy(val).to(eng.device)
 
 
+# Opt-in search targets (DESIGN.md 3.8) for games recorded with their alpha-beta root scores (gen_data --scores): the
+# policy target is softmax(scores / temperature) over the legal moves, the value target (1 - value_weight) * result +
+# value_weight * tanh(best score / 400) from white's point of view.  The defaults are starting points, not tuned values.
+SearchTargets = namedtuple("SearchTargets", ("temperature", "value_weight"), defaults=(50.0, 0.5))
+
+
+def check_targets(targets):
+    """targets None (the move played and the result) or a SearchTargets with 0 < temperature < inf, 0 <= weight <= 1."""
+    if targets is None:
+        return None
+    if not isinstance(targets, SearchTargets):
+        raise ValueError("targets: None or training.SearchTargets, got %r" % (targets,))
+    if not (math.isfinite(targets.temperature) and targets.temperature > 0):
+        raise ValueError("search targets: the temperature must be positive and finite, got %r" % (targets.temperature,))
+    if not 0.0 <= targets.value_weight <= 1.0:
+        raise ValueError("search targets: the value weight must lie in [0, 1], got %r" % (targets.value_weight,))
+    return targets
+
+
+def encode_search_games(games, flips, targets, first=0):
+    """encode_games plus the search targets of the games that carry root scores (Game.search_scores): returns (planes,
+    policy index, value target, policy probabilities float32 [N, 1968]).  Rows of games without scores keep the one-hot
+    of the move played and the result.  One crl_search_targets launch covers every scored row; the kernel's legal count
+    is checked against each row's score count, and a mismatch raises ValueError naming the game and the ply.  The game
+    is named by its index in DatasetGame.games, `first` + its index in `games` (a file's games without moves are not
+    loaded, so this can be below the game's position in the JSON list).  The ply is its index in the game's moves.
+    Flipped games keep their targets, as encode_games does (reference quirk)."""
+    eng = runtime.scalar_engine()
+    planes, pol, val = encode_games(games, flips)
+    probs = F.one_hot(pol, N_LABELS).float()
+    rows, recs, counts, flat, where = [], [], [], [], []
+    off = 0
+    for j, g in enumerate(games):
+        n = len(g._moves)
+        if n and g.search_scores is not None:
+            if len(g.search_scores) != n:
+                raise ValueError("dataset game %d: %d score lists for %d moves" % (first + j, len(g.search_scores), n))
+            rows.append(np.arange(off, off + n))
+            recs.append(np.stack(g._records[:n]).astype(np.uint64))
+            counts += [len(x) for x in g.search_scores]
+            flat += g.search_scores
+            where += [(first + j, i) for i in range(n)]
+        off += n
+    if not rows:
+        return planes, pol, val, probs
+    cnt = np.array(counts, dtype=np.int32)
+    flat = np.fromiter(itertools.chain.from_iterable(flat), dtype=np.int32, count=int(cnt.sum()))
+    offsets = np.zeros(len(cnt) + 1, dtype=np.int32)
+    offsets[1:] = np.cumsum(cnt)
+    dev = eng.device
+    policy, score_value, legal = eng.search_targets(eng.boards_to_device(np.concatenate(recs)),
+                                                    torch.from_numpy(flat).to(dev),
+                                                    torch.from_numpy(offsets).to(dev), targets.temperature)
+    bad = np.nonzero(legal.cpu().numpy() != cnt)[0]          # (the step synchronises on its loss anyway)
+    if len(bad):
+        k = int(bad[0])
+        raise ValueError("dataset game %d, ply %d: %d root scores for %d legal moves"
+                         % (where[k][0], where[k][1], cnt[k], int(legal[k])))
+    idx = torch.from_numpy(np.concatenate(rows)).to(dev)
+    probs[idx] = policy
+    val = val.clone()
+    val[idx] = blend_value(val[idx], score_value, targets.value_weight)
+    return planes, pol, val, probs
+
+
+def blend_value(result, score_value, w):
+    """The search-target value (1 - w) * result + w * score value; with w = 0 exactly the result."""
+    w = float(w)
+    return (1.0 - w) * result + w * score_value
+
+
 class KerasAdam:
     """tf.keras.optimizers.Adam(lr=0.002) (model.py:69) step for step: beta_1 0.9, beta_2 0.999, epsilon 1e-7 applied
     as the paper's "epsilon hat":  lr_t = lr * sqrt(1 - b2^t) / (1 - b1^t);  w -= lr_t * m / (sqrt(v) + eps).
@@ -238,12 +314,16 @@ class KerasAdam:
         torch._foreach_addcdiv_(self.params, self.m, denom, value=-lr_t)
 
 
-def loss_terms(params, planes, pol, val, training=True):
+def loss_terms(params, planes, pol, val, training=True, probs=None):
     """The compiled Keras loss (model.py:68-72 + kernel_regularizer='l2' on every conv / dense layer):
     mean categorical cross-entropy(one-hot of the move played) + mean squared error(value, result) + 0.01 * sum w^2.
-    Returns (total, policy_loss, value_loss, regulariser, logits)."""
+    probs: policy target rows [N, 1968] (search targets) in place of the one-hot of `pol`: the policy term is then
+    mean(-sum_k probs_k log_softmax(logits)_k).  Returns (total, policy_loss, value_loss, regulariser, logits)."""
     logits, value = forward_logits(params, planes, training=training)
-    loss_p = F.cross_entropy(logits, pol)
+    if probs is None:
+        loss_p = F.cross_entropy(logits, pol)
+    else:
+        loss_p = -(probs * F.log_softmax(logits, dim=1)).sum(dim=1).mean()
     loss_v = F.mse_loss(value, val)
     reg = sum((params[i] ** 2).sum() for i in _kernel_indices()) * L2
     return loss_p + loss_v + reg, loss_p, loss_v, reg, logits
@@ -255,10 +335,11 @@ def trainable_indices():
     return [i for i, s in enumerate(pack_shapes()) if not (len(s) == 1 and _is_bn_running(i))]
 
 
-def train_step(params, opt, planes, pol, val):
+def train_step(params, opt, planes, pol, val, probs=None):
     """One fit_generator batch: forward in training mode (BatchNorm batch statistics, moving statistics updated in
-    place), backward, Adam.  Returns the history record of the batch."""
-    total, loss_p, loss_v, reg, logits = loss_terms(params, planes, pol, val, training=True)
+    place), backward, Adam.  probs: search-target policy rows (loss_terms).  Returns the history record of the batch;
+    policy_acc is the argmax against the move played in every target mode."""
+    total, loss_p, loss_v, reg, logits = loss_terms(params, planes, pol, val, training=True, probs=probs)
     grads = torch.autograd.grad(total, opt.params)
     opt.step(list(grads))
     acc = (logits.argmax(1) == pol).float().mean().item()
@@ -266,16 +347,21 @@ def train_step(params, opt, planes, pol, val):
             "policy_acc": acc}
 
 
-def validate(params, val_games, batch_size, dev):
+def validate(params, val_games, batch_size, dev, targets=None, first=0):
     """The validation generator of Agent.train (agent.py:73-75): `batch_size` games per batch, no flips; Keras
-    averages the per-batch means over the batches."""
+    averages the per-batch means over the batches.  targets: the training run's search targets (None: the move played);
+    `first` is the dataset index of val_games[0], for error messages."""
     bs = max(1, min(batch_size, len(val_games)))
     sums, n = {"val_loss": 0.0, "val_policy_loss": 0.0, "val_value_loss": 0.0, "val_policy_acc": 0.0}, 0
     with torch.no_grad():
         for b in range(len(val_games) // bs):
             batch = val_games[b * bs:(b + 1) * bs]
-            planes, pol, val = encode_games(batch, [False] * len(batch), dev)
-            total, loss_p, loss_v, _, logits = loss_terms(params, planes, pol, val, training=False)
+            probs = None
+            if targets is None:
+                planes, pol, val = encode_games(batch, [False] * len(batch), dev)
+            else:
+                planes, pol, val, probs = encode_search_games(batch, [False] * len(batch), targets, first + b * bs)
+            total, loss_p, loss_v, _, logits = loss_terms(params, planes, pol, val, training=False, probs=probs)
             sums["val_loss"] += total.item()
             sums["val_policy_loss"] += loss_p.item()
             sums["val_value_loss"] += loss_v.item()
@@ -284,8 +370,12 @@ def validate(params, val_games, batch_size, dev):
     return {k: v / max(n, 1) for k, v in sums.items()}
 
 
-def train(model, dataset, epochs=1, logdir=None, batch_size=1, validation_split=0, verbose=True, precision=None):
+def train(model, dataset, epochs=1, logdir=None, batch_size=1, validation_split=0, verbose=True, precision=None,
+          targets=None):
+    """targets: None (the move played and the game's result, the reference's targets) or a SearchTargets: search
+    targets for the games that carry root scores, today's for the others (their number is reported)."""
     precision = resolve_precision(precision)
+    targets = check_targets(targets)
     eng = runtime.scalar_engine()
     dev = eng.device
     games = list(dataset.games)
@@ -303,21 +393,34 @@ def train(model, dataset, epochs=1, logdir=None, batch_size=1, validation_split=
         opt = KerasAdam(trainable, lr=0.002, epsilon=1e-7)
         bs = max(1, min(batch_size, len(games))) if games else 1
         history = []
+        if targets is not None:
+            rec = {"search_targets": {"temperature": targets.temperature, "value_weight": targets.value_weight,
+                                      "games": len(games) + len(val_games),
+                                      "games_without_scores": sum(g.search_scores is None for g in games + val_games)}}
+            history.append(rec)
+            if verbose:
+                print("search targets (T %g, w %g): %d of %d games have no root scores and keep the played-move "
+                      "targets" % (targets.temperature, targets.value_weight, rec["search_targets"]["games_without_scores"],
+                                   rec["search_targets"]["games"]))
         for ep in range(epochs):
             order = list(range(len(games) // bs))
             random.shuffle(order)                    # fit_generator shuffles a Sequence's batch order every epoch
             for b in order:
                 batch = games[b * bs:(b + 1) * bs]
                 flips = draw_flips(len(batch), 0.1)                      # agent.py:82-84: random_flips=.1
-                planes, pol, val = encode_games(batch, flips, dev)
-                rec = train_step(params, opt, planes, pol, val)
+                if targets is None:
+                    planes, pol, val = encode_games(batch, flips, dev)
+                    rec = train_step(params, opt, planes, pol, val)
+                else:
+                    planes, pol, val, probs = encode_search_games(batch, flips, targets, b * bs)
+                    rec = train_step(params, opt, planes, pol, val, probs)
                 rec.update({"epoch": ep, "batch": b})
                 history.append(rec)
                 if verbose:
                     print("epoch %d batch %d loss %.4f (policy %.4f value %.4f) acc %.3f" %
                           (ep, b, rec["loss"], rec["policy_loss"], rec["value_loss"], rec["policy_acc"]))
             if val_games:
-                rec = validate(params, val_games, batch_size, dev)
+                rec = validate(params, val_games, batch_size, dev, targets, len(games))
                 rec["epoch"] = ep
                 history.append(rec)
                 if verbose:

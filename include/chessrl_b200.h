@@ -329,6 +329,13 @@ int crl_counters_host(crl_engine* e, int64_t* out3);
 int crl_profile(crl_engine* e, int enable);
 int crl_profile_read_host(crl_engine* e, double* ms_by_class, int64_t* launches_by_class, int n_classes);
 
+/* ---- training targets from the alpha-beta search (DESIGN.md 3.8) ------------------------------------ */
+/* root-child scores of the last crl_games_ab_* call: [n_games][CRL_MAX_MOVES], counts -1 = lane not searched */
+int crl_games_ab_root_scores_host(crl_engine* e, int32_t* scores_host, int32_t* counts_host);
+/* soft policy [n][CRL_N_LABELS] and score value [n] from the root scores of rows offsets[i]..offsets[i+1] */
+int crl_search_targets(crl_engine* e, const uint64_t* boards_dev, const int32_t* scores_dev, const int32_t* offsets_dev,
+                       int n, float temperature, float* policy_dev, float* score_value_dev, int32_t* legal_count_dev);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,27 +1,11 @@
 // net.cu -- forward pass of the policy/value ResNet (model.ChessModel, model.py:31-63, 111-122) for sm_100a.
 //
-// The 21 3x3 convolutions (1 stem + 10 residual blocks x 2) are >99.9% of the FLOPs (1.548 GFLOP/position)
-// and run as ONE kernel each: an implicit GEMM on the 5th-generation tensor cores.
-//
-//   GEMM view      D[M = 64*B board squares][N = 256 filters] = A[M][K = 9*Cin] * W[K][N]
-//   A operand      never materialised.  Activations stay NHWC bf16 [B][8][8][Cin]; for filter tap (dy,dx) and a
-//                  64-channel slice, one TMA box {64ch, 8, 8, 2 boards} fetched at coordinates
-//                  {c0, dx, dy, 2*tile} IS the im2col tile: rows that fall off the board are zero-filled by
-//                  the TMA unit's out-of-bounds handling ('same' padding), and the box lands in shared memory
-//                  as 128 rows x 128 B with the 128-byte swizzle tcgen05 expects for a K-major operand.
-//   B operand      weights re-laid out once as [256][9*Cin] bf16 (K-major), one TMA box {64, 256} per k-block.
-//   MMA            tcgen05.mma.cta_group::1.kind::f16, M=128 N=256 K=16, issued by one thread, fp32 accumulators
-//                  in tensor memory (2 x 256 columns, double buffered so the epilogue of tile i overlaps the
-//                  MMAs of tile i+1).
-//   pipeline       4-stage shared-memory ring (48 KB per stage) fed by a TMA producer thread; mbarriers
-//                  full/empty per stage, tmem_full/tmem_empty per accumulator.
-//   epilogue       4 warps: tcgen05.ld (32 lanes x 32 columns per instruction), folded BatchNorm scale/shift
-//                  (+bias), optional residual add and ReLU in fp32, bf16 pack, 16-byte stores to NHWC.
-//   scheduling     persistent: one CTA per SM, tiles of 2 boards strided over the grid; the row count is
-//                  read from device memory so search batches compact without a host round trip.
-//
-// The heads (1x1 convs, Dense 128->1968 softmax, Dense 64->256->1 tanh: 0.04% of the FLOPs) are one
-// CUDA-core kernel over 8 positions per block.
+// The 21 3x3 convolutions (1 stem + 10 residual blocks x 2) are >99.9% of the FLOPs (1.548 GFLOP/position) and run as
+// ONE persistent kernel per evaluation batch, k_trunk4: implicit GEMMs on the 5th-generation tensor cores
+// (tcgen05.mma.cta_group::2 across a CTA pair, fp32 accumulators in tensor memory), activations kept in an L2-resident
+// scratch between layers, the three 1x1 head convolutions fused into the last layer's epilogue.  Then the policy head's
+// Dense 128->1968 runs as a tcgen05 GEMM through k_conv_v2 (taps = 1), and k_softmax_value finishes the softmax and the
+// value head (Dense 64->256->1 tanh).  k_conv_v2 with taps = 9 is one convolution layer on its own (crl_debug_conv).
 #include "engine.cuh"
 
 #include <cuda.h>
@@ -29,7 +13,6 @@
 #include <cuda_fp8.h>
 #include <math.h>
 #include <type_traits>
-#include <stdlib.h>
 #include <string.h>
 
 namespace crl {
@@ -69,38 +52,10 @@ __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarr
 __device__ __forceinline__ void tcgen05_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tcgen05_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-__device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
-                                            int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)map) : "memory");
 }
 
-// D[tmem] (+)= A[smem] * B[smem], bf16 x bf16 -> fp32
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrives on the mbarrier once every previously issued MMA of this thread has completed
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* v) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -122,329 +77,18 @@ __device__ __forceinline__ uint64_t make_kmajor_sw128_desc(uint32_t smem_addr) {
   return (uint64_t)((smem_addr >> 4) & 0x3FFF) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
-// ======================================================================================================
-// the 3x3 convolution kernel
-// ======================================================================================================
 static constexpr int CONV_THREADS = 256;
-static constexpr int CONV_STAGES = 4;
-static constexpr int TILE_M = 128;                       // 2 boards x 64 squares
 static constexpr int TILE_N = 256;                       // all filters
 static constexpr int BLOCK_K = 64;                       // one 128-byte swizzle atom of bf16
-static constexpr int A_STAGE_BYTES = TILE_M * BLOCK_K * 2;   // 16 KB
-static constexpr int B_STAGE_BYTES = TILE_N * BLOCK_K * 2;   // 32 KB
-static constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
-static constexpr int CONV_SMEM_BYTES = 1024 /*align slack*/ + CONV_STAGES * STAGE_BYTES + 2 * TILE_N * 4 + 256;
-// instruction descriptor: fp32 accumulate, bf16 x bf16, both K-major, N=256, M=128
-static constexpr uint32_t CONV_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((TILE_N >> 3) << 17) | ((TILE_M >> 4) << 24);
-
-struct ConvParams {
-  const int* n_rows_dev;        // board count on the device (or null)
-  int n_rows_host;              // board count / upper bound
-  int k_chunks;                 // Cin / 64
-  const float* scale;           // [256] folded BatchNorm scale (1 when the layer has no BN)
-  const float* shift;           // [256] folded bias / BatchNorm shift
-  const __nv_bfloat16* residual;  // [rows][64][256] or null
-  __nv_bfloat16* out;           // [rows][64][256]
-  int relu;
-};
-
-__global__ void __launch_bounds__(CONV_THREADS, 1)
-k_conv3x3(const __grid_constant__ CUtensorMap map_act, const __grid_constant__ CUtensorMap map_w, ConvParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);   // 128B swizzle: 1024-aligned
-  uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem + CONV_STAGES * A_STAGE_BYTES;
-  float* s_scale = (float*)(smem + CONV_STAGES * STAGE_BYTES);
-  float* s_shift = s_scale + TILE_N;
-  uint64_t* bars = (uint64_t*)(s_shift + TILE_N);
-  uint64_t* full_bar = bars;                    // [CONV_STAGES]
-  uint64_t* empty_bar = bars + CONV_STAGES;     // [CONV_STAGES]
-  uint64_t* tmem_full = bars + 2 * CONV_STAGES; // [2]
-  uint64_t* tmem_empty = tmem_full + 2;         // [2]
-  uint32_t* tmem_slot = (uint32_t*)(tmem_empty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  int n_rows = p.n_rows_host;
-  if (p.n_rows_dev) n_rows = min(n_rows, *p.n_rows_dev);
-  const int n_tiles = (n_rows + 1) >> 1;
-  const int n_kblocks = 9 * p.k_chunks;
-
-  if (threadIdx.x == 0) {
-    prefetch_tmap(&map_act);
-    prefetch_tmap(&map_w);
-  }
-  if (threadIdx.x == 32) {
-    for (int i = 0; i < CONV_STAGES; ++i) {
-      mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tmem_full[i], 1);
-      mbar_init(&tmem_empty[i], 128);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  for (int i = threadIdx.x; i < TILE_N; i += CONV_THREADS) {
-    s_scale[i] = p.scale[i];
-    s_shift[i] = p.shift[i];
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (threadIdx.x == 0) {
-    // ================= TMA producer =================
-    int stage = 0;
-    uint32_t phase = 0;
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      for (int kb = 0; kb < n_kblocks; ++kb) {
-        const int tap = kb / p.k_chunks, kc = kb - tap * p.k_chunks;
-        const int dy = tap / 3 - 1, dx = tap % 3 - 1;
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        mbar_arrive_expect_tx(&full_bar[stage], STAGE_BYTES);
-        tma_load_4d(smem_a + stage * A_STAGE_BYTES, &map_act, &full_bar[stage], kc * BLOCK_K, dx, dy, tile * 2);
-        tma_load_2d(smem_b + stage * B_STAGE_BYTES, &map_w, &full_bar[stage], kb * BLOCK_K, 0);
-        if (++stage == CONV_STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
-      }
-    }
-  } else if (threadIdx.x == 32) {
-    // ================= MMA issuer =================
-    int stage = 0;
-    uint32_t phase = 0;
-    int it = 0;
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
-      tcgen05_fence_after();
-      const uint32_t tmem_d = tmem_base + acc * TILE_N;
-      for (int kb = 0; kb < n_kblocks; ++kb) {
-        mbar_wait(&full_bar[stage], phase);
-        tcgen05_fence_after();
-        const uint64_t da = make_kmajor_sw128_desc(smem_u32(smem_a + stage * A_STAGE_BYTES));
-        const uint64_t db = make_kmajor_sw128_desc(smem_u32(smem_b + stage * B_STAGE_BYTES));
-#pragma unroll
-        for (int k = 0; k < BLOCK_K / 16; ++k) {
-          // advancing K by 16 bf16 = 32 bytes inside the swizzle atom = +2 in the (addr >> 4) field
-          umma_bf16(tmem_d, da + 2 * k, db + 2 * k, CONV_IDESC, (kb | k) != 0);
-        }
-        umma_commit(&empty_bar[stage]);                   // frees the smem stage when these MMAs retire
-        if (kb == n_kblocks - 1) umma_commit(&tmem_full[acc]);   // accumulator complete
-        if (++stage == CONV_STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
-      }
-    }
-  } else if (warp >= 4) {
-    // ================= epilogue: TMEM -> registers -> BN/residual/ReLU -> bf16 -> global =================
-    const int q = warp & 3;                     // TMEM lane quarter this warp may read
-    const int row_in_tile = q * 32 + lane;      // GEMM row = accumulator lane
-    int it = 0;
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      mbar_wait(&tmem_full[acc], acc_phase);
-      tcgen05_fence_after();
-      const long long grow = (long long)tile * TILE_M + row_in_tile;     // global row = board*64 + square
-      const bool valid = grow < (long long)n_rows * 64;
-      __nv_bfloat16* orow = p.out + grow * TILE_N;
-      const __nv_bfloat16* rrow = p.residual ? p.residual + grow * TILE_N : nullptr;
-#pragma unroll 1
-      for (int c0 = 0; c0 < TILE_N; c0 += 32) {
-        uint32_t v[32];
-        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + acc * TILE_N + c0, v);
-        tmem_ld_wait();
-        if (valid) {
-          uint4 res[4];
-          if (rrow) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j) res[j] = *reinterpret_cast<const uint4*>(rrow + c0 + 8 * j);
-          }
-          uint4 outv[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            uint32_t packed[4];
-            const uint32_t* rj = reinterpret_cast<const uint32_t*>(&res[j]);
-#pragma unroll
-            for (int h = 0; h < 4; ++h) {
-              const int c = c0 + 8 * j + 2 * h;
-              float a0 = __uint_as_float(v[8 * j + 2 * h]) * s_scale[c] + s_shift[c];
-              float a1 = __uint_as_float(v[8 * j + 2 * h + 1]) * s_scale[c + 1] + s_shift[c + 1];
-              if (rrow) {
-                a0 += __uint_as_float(rj[h] << 16);
-                a1 += __uint_as_float(rj[h] & 0xFFFF0000u);
-              }
-              if (p.relu) {
-                a0 = fmaxf(a0, 0.f);
-                a1 = fmaxf(a1, 0.f);
-              }
-              __nv_bfloat162 b2 = __floats2bfloat162_rn(a0, a1);
-              packed[h] = *reinterpret_cast<uint32_t*>(&b2);
-            }
-            outv[j] = make_uint4(packed[0], packed[1], packed[2], packed[3]);
-          }
-#pragma unroll
-          for (int j = 0; j < 4; ++j) *reinterpret_cast<uint4*>(orow + c0 + 8 * j) = outv[j];
-        }
-      }
-      tcgen05_fence_before();
-      mbar_arrive(&tmem_empty[acc]);
-    }
-  }
-
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
 
 // ======================================================================================================
-// heads: 1x1 convs + BN + ReLU, Dense 128->1968 softmax, Dense 64->256 ReLU -> Dense 256->1 tanh
-// ======================================================================================================
-static constexpr int HEAD_POS = 8;        // positions per block
-static constexpr int HEAD_THREADS = 256;
-
-struct HeadParams {
-  const int* n_rows_dev;
-  int n_rows_host;
-  const __nv_bfloat16* x;      // [rows][64][256] trunk output
-  const float* w1x1;           // [3][256]: policy ch0, policy ch1, value ch
-  const float* s1x1;           // [3] folded scale, [3] folded shift
-  const float* wp;             // [128][1968]
-  const float* bp;             // [1968]
-  const float* wv1;            // [64][256]
-  const float* bv1;            // [256]
-  const float* wv2;            // [256]
-  const float* bv2;            // [1]
-  float* policy;               // [rows][1968]
-  float* value;                // [rows]
-};
-
-__global__ void __launch_bounds__(HEAD_THREADS) k_heads(HeadParams p) {
-  extern __shared__ float hs[];
-  float* s_w = hs;                              // [3][256]
-  float* s_pf = s_w + 3 * 256;                  // [HEAD_POS][128] policy features (h,w,c) flatten
-  float* s_vf = s_pf + HEAD_POS * 128;          // [HEAD_POS][64]
-  float* s_hid = s_vf + HEAD_POS * 64;          // [HEAD_POS][256]
-  float* s_logit = s_hid + HEAD_POS * 256;      // [HEAD_POS][1968]
-  int n_rows = p.n_rows_host;
-  if (p.n_rows_dev) n_rows = min(n_rows, *p.n_rows_dev);
-  const int pos0 = blockIdx.x * HEAD_POS;
-  if (pos0 >= n_rows) return;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < 3 * 256; i += HEAD_THREADS) s_w[i] = p.w1x1[i];
-  __syncthreads();
-
-  // (1) 1x1 convolutions: warp w owns position pos0+w; lanes split the 256 channels 8 apiece
-  {
-    const int pos = pos0 + warp;
-    const bool ok = pos < n_rows;
-    for (int sq = 0; sq < 64; ++sq) {
-      float a0 = 0.f, a1 = 0.f, a2 = 0.f;
-      if (ok) {
-        uint4 raw = *reinterpret_cast<const uint4*>(p.x + ((long long)pos * 64 + sq) * 256 + lane * 8);
-        const uint32_t* r = reinterpret_cast<const uint32_t*>(&raw);
-#pragma unroll
-        for (int h = 0; h < 4; ++h) {
-          float x0 = __uint_as_float(r[h] << 16), x1 = __uint_as_float(r[h] & 0xFFFF0000u);
-          int c = lane * 8 + 2 * h;
-          a0 += x0 * s_w[c] + x1 * s_w[c + 1];
-          a1 += x0 * s_w[256 + c] + x1 * s_w[256 + c + 1];
-          a2 += x0 * s_w[512 + c] + x1 * s_w[512 + c + 1];
-        }
-      }
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1) {
-        a0 += __shfl_xor_sync(0xffffffffu, a0, off);
-        a1 += __shfl_xor_sync(0xffffffffu, a1, off);
-        a2 += __shfl_xor_sync(0xffffffffu, a2, off);
-      }
-      if (lane == 0) {
-        s_pf[warp * 128 + sq * 2 + 0] = fmaxf(a0 * p.s1x1[0] + p.s1x1[3], 0.f);
-        s_pf[warp * 128 + sq * 2 + 1] = fmaxf(a1 * p.s1x1[1] + p.s1x1[4], 0.f);
-        s_vf[warp * 64 + sq] = fmaxf(a2 * p.s1x1[2] + p.s1x1[5], 0.f);
-      }
-    }
-  }
-  __syncthreads();
-
-  // (2) policy logits: thread owns output columns j, j+256, ...; weights stream from L2 once per 8 positions
-  for (int j = threadIdx.x; j < CRL_N_LABELS; j += HEAD_THREADS) {
-    float acc[HEAD_POS];
-#pragma unroll
-    for (int q = 0; q < HEAD_POS; ++q) acc[q] = 0.f;
-    for (int i = 0; i < 128; ++i) {
-      const float w = p.wp[(long long)i * CRL_N_LABELS + j];
-#pragma unroll
-      for (int q = 0; q < HEAD_POS; ++q) acc[q] = fmaf(s_pf[q * 128 + i], w, acc[q]);
-    }
-    const float b = p.bp[j];
-#pragma unroll
-    for (int q = 0; q < HEAD_POS; ++q) s_logit[q * CRL_N_LABELS + j] = acc[q] + b;
-  }
-  // value hidden layer: thread j owns hidden unit j
-  {
-    const int j = threadIdx.x;
-    float acc[HEAD_POS];
-#pragma unroll
-    for (int q = 0; q < HEAD_POS; ++q) acc[q] = 0.f;
-    for (int i = 0; i < 64; ++i) {
-      const float w = p.wv1[i * 256 + j];
-#pragma unroll
-      for (int q = 0; q < HEAD_POS; ++q) acc[q] = fmaf(s_vf[q * 64 + i], w, acc[q]);
-    }
-    const float b = p.bv1[j];
-#pragma unroll
-    for (int q = 0; q < HEAD_POS; ++q) s_hid[q * 256 + j] = fmaxf(acc[q] + b, 0.f);
-  }
-  __syncthreads();
-
-  // (3) softmax and value output: warp w finishes position pos0+w
-  {
-    const int pos = pos0 + warp;
-    if (pos < n_rows) {
-      const float* lg = s_logit + warp * CRL_N_LABELS;
-      float m = -INFINITY;
-      for (int j = lane; j < CRL_N_LABELS; j += 32) m = fmaxf(m, lg[j]);
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
-      float s = 0.f;
-      for (int j = lane; j < CRL_N_LABELS; j += 32) s += expf(lg[j] - m);
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
-      const float inv = 1.0f / s;
-      float* out = p.policy + (long long)pos * CRL_N_LABELS;
-      for (int j = lane; j < CRL_N_LABELS; j += 32) out[j] = expf(lg[j] - m) * inv;
-      float v = 0.f;
-      for (int j = lane; j < 256; j += 32) v = fmaf(s_hid[warp * 256 + j], p.wv2[j], v);
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-      if (lane == 0) p.value[pos] = tanhf(v + p.bv2[0]);
-    }
-  }
-}
-static constexpr int HEAD_SMEM_BYTES = (3 * 256 + HEAD_POS * (128 + 64 + 256 + CRL_N_LABELS)) * 4;
-
-// ======================================================================================================
-// v2: CTA-pair (cta_group::2) implicit-GEMM kernel.  Two CTAs of a cluster share one 256-row tile: each loads
-// its own 128 rows of A and HALF of the weight tile (128 of the 256 filters), so the weight traffic out of L2 per
-// SM is halved and a stage shrinks to 32 KB -> 6 stages (deeper TMA prefetch).  The leader CTA issues
-// tcgen05.mma.cta_group::2 (M=256 across the pair, N=256, K=16); tcgen05.commit multicasts stage-release and
-// accumulator-ready to both CTAs; both CTAs run their own epilogue out of their own tensor memory.
-// The same kernel also runs plain GEMMs (taps = 1, A through a 2-D map) -- used for the policy head's dense layer --
-// and, for the last convolution, fuses the three 1x1 head convolutions (+BN+ReLU) into its epilogue.
+// k_conv_v2: CTA-pair (cta_group::2) implicit-GEMM kernel.  Two CTAs of a cluster share one 256-row tile: each loads
+// its own 128 rows of A and HALF of the weight tile (128 of the 256 filters), so a stage is 32 KB and the ring has
+// 6 stages.  The leader CTA issues tcgen05.mma.cta_group::2 (M=256 across the pair, N=256, K=16); tcgen05.commit
+// multicasts stage-release and accumulator-ready to both CTAs; both CTAs run their own epilogue out of their own
+// tensor memory.  With taps = 9 it is one 3x3 convolution layer (A: one TMA box per tap and 64-channel slice, the
+// im2col tile with 'same' padding from the TMA unit's zero fill); with taps = 1 a plain GEMM (A through a 2-D map),
+// the policy head's dense layer.  Its epilogue can also fuse the three 1x1 head convolutions (+BN+ReLU, head_w).
 // ======================================================================================================
 static constexpr int V2_STAGES = 6;
 static constexpr int V2_A_BYTES = 128 * BLOCK_K * 2;      // 16 KB: this CTA's 128 rows
@@ -452,7 +96,6 @@ static constexpr int V2_B_BYTES = 128 * BLOCK_K * 2;      // 16 KB: this CTA's h
 static constexpr int V2_STAGE_BYTES = V2_A_BYTES + V2_B_BYTES;
 static constexpr int V2_SMEM_BYTES = 1024 + V2_STAGES * V2_STAGE_BYTES + 2 * TILE_N * 4 + 3 * 256 * 4 + 64 + 512;
 static constexpr uint32_t V2_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((TILE_N >> 3) << 17) | ((256u >> 4) << 24);
-static constexpr uint32_t V2_IDESC_N128 = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((256u >> 4) << 24);
 static constexpr uint32_t PEER_MASK = 0xFEFFFFFFu;        // clears the CTA-rank bit of a shared::cluster address
 
 struct ConvParams2 {
@@ -776,20 +419,8 @@ k_conv_v2(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
   }
 }
 
-// ======================================================================================================
-// v3: the whole residual tower in ONE persistent kernel.
-// A 3x3 'same' convolution of a board only reads that board, so a CTA pair can carry its boards through all 21
-// layers without any grid-wide synchronisation.  Each pair works on a GROUP of two 256-row tiles (2 x 4 boards),
-// tile X bound to tensor-memory accumulator X, and walks  for layer: for tile in (A, B): k-blocks .  While the
-// tensor cores run tile B of layer L, the epilogue warps drain tile A of layer L and publish its activations, so
-// the producer can prefetch tile A of layer L+1 as ring slots free up: no kernel boundaries, no pipeline ramp,
-// no tail wave between layers, and activations never leave L2.
-//   extra barrier: act_ready[X] (128 local epilogue arrivals) = "tile X's output of the previous layer is in global
-//   memory"; the epilogue makes its generic-proxy stores visible to the TMA (async proxy) with
-//   __threadfence + fence.proxy.async before arriving.
-// ======================================================================================================
 struct LayerDesc {
-  int map_in;            // index into the tensor-map table: 0 planes, 1 act[0], 2 act[1]
+  int map_in;            // index into the tensor-map table: 0 planes, 1 act4[0], 2 act4[1]
   int map_w;             // 3 + layer
   int k_chunks;
   int relu;
@@ -828,245 +459,33 @@ struct TrunkParams {
   float* vf_out;
   __nv_bfloat16* dbg_out;   // test tap (crl_debug_tower): layer dbg_layer's output [boards][64][256], else null
   int dbg_layer;
-  // L2 eviction priorities of the v4 tower's TMA loads: the planes are read once (evict first), the weights are re-read
-  // by every CTA pair for every group (evict last), the activation scratch keeps the default
+  // L2 eviction priorities of the tower's TMA loads: the planes are read once (evict first), the weights are re-read
+  // by every CTA pair for every group (evict last), the activation scratch keeps the default.  Kernel parameters
+  // rather than compile-time constants: as immediates they compile to 8 more instructions per instantiation.
   uint64_t hint_planes, hint_weights;
-  // TIMING PROBE ONLY (CRL_T4_NSPLIT_PROBE=1, scripts/trunk4_nsplit_probe.py): issue every K step as two M=256 x N=128
-  // MMAs (filter halves of the weight stage, accumulator columns 0-127 / 128-255) instead of one N=256 MMA.  The
-  // accumulator columns come out permuted, so the network's RESULTS ARE WRONG in this mode; it exists to measure whether
-  // N=128 MMAs with both operands in shared memory (the image operand read twice) sustain the N=256 rate -- the
-  // precondition of sharing a weight stage between the two tiles of a group (DESIGN.md section 8).
-  int probe_nsplit;
 };
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CONV_THREADS, 1)
-k_trunk(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __restrict__ maps,
-        const LayerDesc* __restrict__ layers, TrunkParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem + V2_STAGES * V2_A_BYTES;
-  float* s_scale = (float*)(smem + V2_STAGES * V2_STAGE_BYTES);
-  float* s_shift = s_scale + TILE_N;
-  float* s_hw = s_shift + TILE_N;
-  float* s_hs = s_hw + 3 * 256;
-  uint64_t* bars = (uint64_t*)(s_hs + 16);
-  uint64_t* full_bar = bars;
-  uint64_t* empty_bar = bars + V2_STAGES;
-  uint64_t* tmem_full = bars + 2 * V2_STAGES;
-  uint64_t* tmem_empty = tmem_full + 2;
-  uint64_t* act_ready = tmem_empty + 2;
-  uint32_t* tmem_slot = (uint32_t*)(act_ready + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-  int n_boards = p.n_host;
-  if (p.n_dev) n_boards = min(n_boards, *p.n_dev);
-  const long long total_rows = (long long)n_boards * 64;
-  const int n_tiles = (n_boards + 3) >> 2;          // 256-row tiles (4 boards)
-  const int n_groups = (n_tiles + 1) >> 1;
-  const int NL = p.n_layers;
-
-  if (threadIdx.x == 0) prefetch_tmap(&map_planes);
-  if (threadIdx.x == 32) {
-    for (int i = 0; i < V2_STAGES; ++i) {
-      mbar_init(&full_bar[i], 2);
-      mbar_init(&empty_bar[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tmem_full[i], 1);
-      mbar_init(&tmem_empty[i], 256);
-      mbar_init(&act_ready[i], 128);
-    }
-    fence_barrier_init();
-  }
-  cluster_sync_all();
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  for (int i = threadIdx.x; i < 3 * 256; i += CONV_THREADS) s_hw[i] = p.head_w[i];
-  if (threadIdx.x < 6) s_hs[threadIdx.x] = p.head_s[threadIdx.x];
-  tcgen05_fence_before();
-  cluster_sync_all();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (threadIdx.x == 0) {
-    // ================= TMA producer =================
-    int stage = 0;
-    uint32_t phase = 0;
-    int uses = 0;                                   // completed (tile, layer) units per accumulator slot
-    for (int grp = pair; grp < n_groups; grp += n_pairs) {
-      for (int L = 0; L < NL; ++L, ++uses) {
-        const LayerDesc ld = layers[L];
-        const CUtensorMap* map_a = ld.map_in == 0 ? &map_planes : maps + ld.map_in;   // planes: kernel parameter
-        const CUtensorMap* map_w = maps + ld.map_w;
-        const int n_kblocks = 9 * ld.k_chunks;
-        for (int X = 0; X < 2; ++X) {
-          const int tile = 2 * grp + X;
-          // this tile's input is the previous layer's output: wait until our own epilogue has published it
-          if (L > 0) mbar_wait(&act_ready[X], (uint32_t)((uses - 1) & 1));
-          for (int kb = 0; kb < n_kblocks; ++kb) {
-            const int tap = kb / ld.k_chunks, kc = kb - tap * ld.k_chunks;
-            mbar_wait(&empty_bar[stage], phase ^ 1);
-            if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * V2_STAGE_BYTES);
-            tma2_load_4d(smem_a + stage * V2_A_BYTES, map_a, &full_bar[stage], kc * BLOCK_K, tap % 3 - 1, tap / 3 - 1,
-                         tile * 4 + (int)rank * 2);
-            tma2_load_2d(smem_b + stage * V2_B_BYTES, map_w, &full_bar[stage], kb * BLOCK_K, (int)rank * 128);
-            if (rank != 0) mbar_arrive_remote(&full_bar[stage], 0);
-            if (++stage == V2_STAGES) {
-              stage = 0;
-              phase ^= 1;
-            }
-          }
-        }
-      }
-    }
-  } else if (threadIdx.x == 32 && rank == 0) {
-    // ================= MMA issuer (leader CTA) =================
-    int stage = 0;
-    uint32_t phase = 0;
-    int uses = 0;
-    for (int grp = pair; grp < n_groups; grp += n_pairs) {
-      for (int L = 0; L < NL; ++L, ++uses) {
-        const int n_kblocks = 9 * layers[L].k_chunks;
-        for (int X = 0; X < 2; ++X) {
-          mbar_wait(&tmem_empty[X], (uint32_t)((uses & 1) ^ 1));
-          tcgen05_fence_after();
-          const uint32_t tmem_d = tmem_base + X * TILE_N;
-          for (int kb = 0; kb < n_kblocks; ++kb) {
-            mbar_wait(&full_bar[stage], phase);
-            tcgen05_fence_after();
-            const uint64_t da = make_kmajor_sw128_desc(smem_u32(smem_a + stage * V2_A_BYTES));
-            const uint64_t db = make_kmajor_sw128_desc(smem_u32(smem_b + stage * V2_B_BYTES));
-#pragma unroll
-            for (int k = 0; k < BLOCK_K / 16; ++k) umma2_bf16(tmem_d, da + 2 * k, db + 2 * k, V2_IDESC, (kb | k) != 0);
-            umma2_commit_both(&empty_bar[stage]);
-            if (kb == n_kblocks - 1) umma2_commit_both(&tmem_full[X]);
-            if (++stage == V2_STAGES) {
-              stage = 0;
-              phase ^= 1;
-            }
-          }
-        }
-      }
-    }
-    if (uses > 0) {
-      mbar_wait(&tmem_empty[0], (uint32_t)((uses - 1) & 1));
-      mbar_wait(&tmem_empty[1], (uint32_t)((uses - 1) & 1));
-    }
-  } else if (warp >= 4) {
-    // ================= epilogue (both CTAs) =================
-    const int q = warp & 3;
-    const int row_in_cta = q * 32 + lane;
-    int uses = 0;
-    for (int grp = pair; grp < n_groups; grp += n_pairs) {
-      for (int L = 0; L < NL; ++L, ++uses) {
-        const LayerDesc ld = layers[L];
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        for (int i = threadIdx.x - 128; i < TILE_N; i += 128) {
-          s_scale[i] = ld.scale[i];
-          s_shift[i] = ld.shift[i];
-        }
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        for (int X = 0; X < 2; ++X) {
-          const int tile = 2 * grp + X;
-          mbar_wait(&tmem_full[X], (uint32_t)(uses & 1));
-          tcgen05_fence_after();
-          const long long grow = (long long)tile * 256 + rank * 128 + row_in_cta;
-          const bool valid = grow < total_rows;
-          __nv_bfloat16* orow = ld.write_out ? ld.out + grow * TILE_N : nullptr;
-          const __nv_bfloat16* rrow = ld.residual ? ld.residual + grow * TILE_N : nullptr;
-          float h0 = 0.f, h1 = 0.f, h2 = 0.f;
-#pragma unroll 1
-          for (int c0 = 0; c0 < TILE_N; c0 += 32) {
-            uint32_t v[32];
-            tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + X * TILE_N + c0, v);
-            tmem_ld_wait();
-            if (!valid) continue;
-            uint4 res[4];
-            if (rrow) {
-#pragma unroll
-              for (int j = 0; j < 4; ++j) res[j] = *reinterpret_cast<const uint4*>(rrow + c0 + 8 * j);
-            }
-            float a[32];
-#pragma unroll
-            for (int j = 0; j < 32; ++j) a[j] = __uint_as_float(v[j]) * s_scale[c0 + j] + s_shift[c0 + j];
-            if (rrow) {
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const uint32_t* rj = reinterpret_cast<const uint32_t*>(&res[j]);
-#pragma unroll
-                for (int h = 0; h < 4; ++h) {
-                  a[8 * j + 2 * h] += __uint_as_float(rj[h] << 16);
-                  a[8 * j + 2 * h + 1] += __uint_as_float(rj[h] & 0xFFFF0000u);
-                }
-              }
-            }
-            if (ld.relu) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j) a[j] = fmaxf(a[j], 0.f);
-            }
-            if (ld.fuse_heads) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j) {
-                const float x = __bfloat162float(__float2bfloat16_rn(a[j]));
-                h0 = fmaf(x, s_hw[c0 + j], h0);
-                h1 = fmaf(x, s_hw[256 + c0 + j], h1);
-                h2 = fmaf(x, s_hw[512 + c0 + j], h2);
-              }
-            }
-            if (orow) {
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                uint32_t pk[4];
-#pragma unroll
-                for (int h = 0; h < 4; ++h) {
-                  __nv_bfloat162 b2 = __floats2bfloat162_rn(a[8 * j + 2 * h], a[8 * j + 2 * h + 1]);
-                  pk[h] = *reinterpret_cast<uint32_t*>(&b2);
-                }
-                *reinterpret_cast<uint4*>(orow + c0 + 8 * j) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-              }
-            }
-          }
-          tcgen05_fence_before();
-          mbar_arrive_remote(&tmem_empty[X], 0);
-          if (ld.fuse_heads && valid) {
-            const float f0 = fmaxf(h0 * s_hs[0] + s_hs[3], 0.f), f1 = fmaxf(h1 * s_hs[1] + s_hs[4], 0.f);
-            reinterpret_cast<__nv_bfloat162*>(p.pf_out)[grow] = __floats2bfloat162_rn(f0, f1);
-            p.vf_out[grow] = fmaxf(h2 * s_hs[2] + s_hs[5], 0.f);
-          }
-          // publish this tile's activations to the TMA unit (generic proxy -> async proxy), then release the producer
-          __threadfence();
-          asm volatile("fence.proxy.async.global;" ::: "memory");
-          mbar_arrive(&act_ready[X]);
-        }
-      }
-    }
-  }
-
-  tcgen05_fence_before();
-  cluster_sync_all();
-  if (warp == 2) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
-
 // ======================================================================================================
-// v4: the tower kernel with the im2col operand REUSED across the nine filter taps.
-// v3 fetches one 16 KB A tile per (tap, 64-channel slice): the same activations cross L2 -> shared memory nine times.
-// Here the TMA unit loads, once per 64-channel slice, the zero-padded IMAGE of the CTA's two boards
+// k_trunk4: the whole residual tower in ONE persistent kernel.
+// A 3x3 'same' convolution of a board only reads that board, so a CTA pair can carry its boards through all 21
+// layers without any grid-wide synchronisation.  Each pair works on a GROUP of two 256-row tiles (2 x 4 boards),
+// tile X bound to tensor-memory accumulator X, and walks  for layer: for tile in (A, B): k-blocks .  While the
+// tensor cores run tile B of layer L, the epilogue warps drain tile A of layer L and publish its activations, so
+// the producer can prefetch tile A of layer L+1 as ring slots free up: no kernel boundaries, no pipeline ramp,
+// no tail wave between layers, and activations never leave L2.
+//   extra barrier: act_ready[X] (128 local epilogue arrivals) = "tile X's output of the previous layer is in global
+//   memory"; the epilogue makes its generic-proxy stores visible to the TMA (async proxy) with
+//   __threadfence + fence.proxy.async before arriving.
+//
+// The im2col operand is REUSED across the nine filter taps: the TMA unit loads, once per 64-channel slice, the
+// zero-padded IMAGE of the CTA's two boards
 //     rows [y = -1..8][board 0..1][x = -1..8] x 64 channels  (200 rows of 128 bytes, 128-byte swizzle)
 // through a tensor map whose dimensions are ordered (C, W, B, H), so that out-of-board rows / columns are zero-filled
-// by the TMA unit exactly as before.  The A operand of tap (dy, dx) is then the SAME image addressed through a
-// shifted shared-memory descriptor: start row (1+dy)*20 + (1+dx), 8-row groups 1,280 bytes apart (one image row of
-// ten pixels), group g = 2*y + board.  Rows of a tile are therefore ordered (y, board, x) instead of (board, y, x);
-// the epilogue un-permutes when it computes its global row.  Per (tile, layer) a CTA now reads 4 x 25.6 KB of
-// activations instead of 36 x 16 KB; the weight stream (36 x 16 KB) is unchanged and gets its own, deeper ring.
+// by the TMA unit.  The A operand of tap (dy, dx) is then the SAME image addressed through a shifted shared-memory
+// descriptor: start row (1+dy)*20 + (1+dx), 8-row groups 1,280 bytes apart (one image row of ten pixels), group
+// g = 2*y + board.  Rows of a tile are therefore ordered (y, board, x) instead of (board, y, x); the epilogue
+// un-permutes when it computes its global row.  Per (tile, layer) a CTA reads 4 x 25.6 KB of activations where one
+// box per (tap, slice) would read 36 x 16 KB; the weight stream (36 x 16 KB) has its own, deeper ring.
 //
 // Activation scratch is indexed by CTA-PAIR SLOT, not by board: a pair carries its group of 8 boards through all 21
 // layers before it takes the next group, so the two ping-pong buffers only need 8 boards per pair
@@ -1074,25 +493,24 @@ k_trunk(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __res
 // overwritten by the next layer before it is evicted, so the activations stop being written back to HBM
 // (board-indexed buffers: 2 x 134 MB per 4,096-position batch, 4.85 x the algorithmic DRAM traffic).
 // ======================================================================================================
-// ring sizes are template parameters: T4_NA padded-image slots, T4_NB weight stages (default 3 / 7)
+static constexpr int T4_NA = 3;                           // padded-image slots
+static constexpr int T4_NB = 7;                           // weight stages
 static constexpr int T4_IMG_ROWS = 200;                   // 10 x 2 x 10
 static constexpr int T4_IMG_BYTES = T4_IMG_ROWS * 128;    // 25,600
 static constexpr int T4_A_SLOT = 26 * 1024;               // slot pitch (1,024-byte aligned)
 static constexpr int T4_B_BYTES = 128 * BLOCK_K * 2;      // 16 KB: this CTA's half of the 256 filters
-constexpr int t4_smem_bytes(int na, int nb) {
-  return 1024 + na * T4_A_SLOT + nb * T4_B_BYTES + 2 * TILE_N * 4 + 3 * 256 * 4 + 64 + 512;
-}
+static constexpr int T4_SMEM_BYTES = 1024 + T4_NA * T4_A_SLOT + T4_NB * T4_B_BYTES + 2 * TILE_N * 4 + 3 * 256 * 4 + 64 + 512;
 
 // K-major SWIZZLE_128B descriptor with an explicit stride between 8-row groups
 __device__ __forceinline__ uint64_t make_kmajor_sw128_desc_sbo(uint32_t smem_addr, uint32_t sbo_bytes) {
   return (uint64_t)((smem_addr >> 4) & 0x3FFF) | ((uint64_t)(sbo_bytes >> 4) << 32) | (1ull << 46) | (2ull << 61);
 }
 
-// FP8 (a separate instantiation, <3, 7> only): the same pipeline on e4m3 operands.  A 128-byte swizzle row then holds
+// FP8 (a separate instantiation): the same pipeline on e4m3 operands.  A 128-byte swizzle row then holds
 // 128 channels, so a slice is 128 channels and the boxes keep their byte sizes; each MMA is kind::f8f6f4 with K = 32.
 // The epilogue applies the per-layer scales of LayerDesc8 and stores e4m3 codes; the last convolution (fused heads only)
 // rounds to bf16 exactly as the bf16 tower does.
-template <int T4_NA, int T4_NB, bool SINGLE = false, bool FP8 = false>
+template <bool SINGLE, bool FP8>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CONV_THREADS, 1)
 k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __restrict__ maps,
          const typename std::conditional<FP8, LayerDesc8, LayerDesc>::type* __restrict__ layers, TrunkParams p) {
@@ -1228,13 +646,6 @@ k_trunk4(const __grid_constant__ CUtensorMap map_planes, const CUtensorMap* __re
               if constexpr (FP8) {
 #pragma unroll
                 for (int k = 0; k < 4; ++k) umma2_fp8(tmem_d, da + 2 * k, db + 2 * k, V2_IDESC_FP8, (kc | tap | k) != 0);
-              } else if (p.probe_nsplit) {
-                // (timing probe, see TrunkParams) rows 64..127 of this CTA's weight tile start 8 KB = 512 x 16 B further on
-#pragma unroll
-                for (int k = 0; k < BLOCK_K / 16; ++k) {
-                  umma2_bf16(tmem_d, da + 2 * k, db + 2 * k, V2_IDESC_N128, (kc | tap | k) != 0);
-                  umma2_bf16(tmem_d + 128, da + 2 * k, db + 512 + 2 * k, V2_IDESC_N128, (kc | tap | k) != 0);
-                }
               } else {
 #pragma unroll
                 for (int k = 0; k < BLOCK_K / 16; ++k) umma2_bf16(tmem_d, da + 2 * k, db + 2 * k, V2_IDESC, (kc | tap | k) != 0);
@@ -1565,18 +976,11 @@ struct NetWeights {
   float* scale[N_CONVS] = {nullptr};
   float* shift[N_CONVS] = {nullptr};
   int cin[N_CONVS] = {0};
-  CUtensorMap map_w[N_CONVS];
-  __nv_bfloat16* act[2] = {nullptr, nullptr};   // [cap][64][256]
-  CUtensorMap map_act[2];
-  CUtensorMap map_planes;
   const void* planes_ptr = nullptr;
   int planes_rows = 0;
-  float *w1x1 = nullptr, *s1x1 = nullptr, *wp = nullptr, *bp = nullptr, *wv1 = nullptr, *bv1 = nullptr,
-        *wv2 = nullptr, *bv2 = nullptr;
+  float *w1x1 = nullptr, *s1x1 = nullptr, *wv1 = nullptr, *bv1 = nullptr, *wv2 = nullptr, *bv2 = nullptr;
   PFN_encodeTiled encode = nullptr;
   int n_sms = 148;
-  // v2 (CTA-pair kernel, fused heads)
-  bool use_v2 = true;
   CUtensorMap map_w2[N_CONVS];              // weight boxes of 128 filters (one CTA's half)
   __nv_bfloat16* pf = nullptr;              // [cap][128] policy features (bf16)
   float* vf = nullptr;                      // [cap][64] value features
@@ -1585,23 +989,14 @@ struct NetWeights {
   float* bp_pad = nullptr;                  // [2048]
   float* ones = nullptr;                    // [2048]
   CUtensorMap map_pf, map_wp;
-  // v4 (tower kernel with the padded-image A operand reused across the nine taps)
-  bool use_trunk4 = true;
-  int t4_ring = 0;                          // index into the instantiated (image slots, weight stages) pairs
-  int probe_nsplit = 0;                     // CRL_T4_NSPLIT_PROBE=1: timing probe, WRONG results (see TrunkParams)
-  bool t4_single = true;                    // single-tile instantiation for small batches (CRL_T4_NO_SINGLE=1: off)
+  // the tower (k_trunk4)
   __nv_bfloat16* act4[2] = {nullptr, nullptr};  // [n_sms/2 pairs x 8 boards][64][256]: ping-pong scratch by CTA-pair slot
   int act4_rows = 0;
-  bool l2_hints = true;                     // CRL_T4_L2_HINTS=0 turns the eviction-priority hints off (A/B)
   CUtensorMap map_act4[2];
   CUtensorMap map_planes4;
-  CUtensorMap* d_maps4 = nullptr;
+  CUtensorMap* d_maps4 = nullptr;           // [3 + N_CONVS] device copies: (unused: the planes map is a kernel
+                                            // parameter), act4[0], act4[1], weights (128-filter boxes)
   LayerDesc* d_layers4 = nullptr;           // [N_CONVS], out / residual pointing into act4
-  // v3 (whole tower in one persistent kernel)
-  bool use_trunk = true;
-  CUtensorMap* d_maps = nullptr;            // [3 + N_CONVS] device copies: (unused: the planes map is a kernel
-                                            // parameter), act[0], act[1], weights (128-filter boxes)
-  LayerDesc* d_layers = nullptr;            // [N_CONVS]
   // fp8 tower (crl_net_load_fp8_host); buffers are allocated by the first fp8 load
   bool fp8_loaded = false;
   bool fp8 = false;                         // the fp8 tower is selected
@@ -1708,12 +1103,9 @@ int net_create(crl_engine_impl* e, int slot) {
     if ((rc = dev_alloc(e, &nw->w[i], (size_t)TILE_N * 9 * nw->cin[i]))) return rc;
     if ((rc = dev_alloc(e, &nw->scale[i], 256))) return rc;
     if ((rc = dev_alloc(e, &nw->shift[i], 256))) return rc;
-    if ((rc = make_w_map(nw, &nw->map_w[i], nw->w[i], 9 * nw->cin[i]))) return rc;
     if ((rc = make_w_map(nw, &nw->map_w2[i], nw->w[i], 9 * nw->cin[i], TILE_N, 128))) return rc;
   }
   {
-    const char* v1 = getenv("CRL_CONV_V1");
-    nw->use_v2 = !(v1 && v1[0] == '1');
     if ((rc = dev_alloc(e, &nw->pf, (size_t)(nw->cap_rows + 256) * 128))) return rc;
     if ((rc = dev_alloc(e, &nw->vf, (size_t)(nw->cap_rows + 256) * 64))) return rc;
     if (slot == 0) {
@@ -1728,106 +1120,62 @@ int net_create(crl_engine_impl* e, int slot) {
     if ((rc = make_w_map(nw, &nw->map_pf, nw->pf, 128, nw->cap_rows + 256, 128))) return rc;
     if ((rc = make_w_map(nw, &nw->map_wp, nw->wp_bf16, 128, 2048, 128))) return rc;
   }
-  {
-    // which tower runs is fixed at creation (debug knobs), so only its activation buffers are allocated
-    const char* nt = getenv("CRL_NO_TRUNK");
-    const char* t3 = getenv("CRL_TRUNK_V3");
-    nw->use_trunk = nw->use_v2 && !(nt && nt[0] == '1');
-    nw->use_trunk4 = nw->use_trunk && !(t3 && t3[0] == '1');
-  }
-  if (nw->use_trunk4) {
-    nw->act4_rows = (nw->n_sms / 2) * 8;
-    for (int i = 0; i < 2; ++i) {
-      if ((rc = dev_alloc(e, &nw->act4[i], (size_t)nw->act4_rows * 64 * 256))) return rc;
-      CRL_CUDA(cudaMemsetAsync(nw->act4[i], 0, (size_t)nw->act4_rows * 64 * 256 * 2, e->stream));
-      if ((rc = make_act_map4(nw, &nw->map_act4[i], nw->act4[i], 256, nw->act4_rows))) return rc;
-    }
-  } else {
-    for (int i = 0; i < 2; ++i) {
-      if ((rc = dev_alloc(e, &nw->act[i], (size_t)nw->cap_rows * 64 * 256))) return rc;
-      CRL_CUDA(cudaMemsetAsync(nw->act[i], 0, (size_t)nw->cap_rows * 64 * 256 * 2, e->stream));
-      if ((rc = make_act_map(nw, &nw->map_act[i], nw->act[i], 256, nw->cap_rows))) return rc;
-    }
+  nw->act4_rows = (nw->n_sms / 2) * 8;
+  for (int i = 0; i < 2; ++i) {
+    if ((rc = dev_alloc(e, &nw->act4[i], (size_t)nw->act4_rows * 64 * 256))) return rc;
+    CRL_CUDA(cudaMemsetAsync(nw->act4[i], 0, (size_t)nw->act4_rows * 64 * 256 * 2, e->stream));
+    if ((rc = make_act_map4(nw, &nw->map_act4[i], nw->act4[i], 256, nw->act4_rows))) return rc;
   }
   if ((rc = dev_alloc(e, &nw->w1x1, 3 * 256))) return rc;
   if ((rc = dev_alloc(e, &nw->s1x1, 6))) return rc;
-  if ((rc = dev_alloc(e, &nw->wp, (size_t)128 * CRL_N_LABELS))) return rc;
-  if ((rc = dev_alloc(e, &nw->bp, CRL_N_LABELS))) return rc;
   if ((rc = dev_alloc(e, &nw->wv1, 64 * 256))) return rc;
   if ((rc = dev_alloc(e, &nw->bv1, 256))) return rc;
   if ((rc = dev_alloc(e, &nw->wv2, 256))) return rc;
   if ((rc = dev_alloc(e, &nw->bv2, 1))) return rc;
-  CRL_CUDA(cudaFuncSetAttribute(k_conv3x3, cudaFuncAttributeMaxDynamicSharedMemorySize, CONV_SMEM_BYTES));
-  CRL_CUDA(cudaFuncSetAttribute(k_heads, cudaFuncAttributeMaxDynamicSharedMemorySize, HEAD_SMEM_BYTES));
   CRL_CUDA(cudaFuncSetAttribute(k_conv_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, V2_SMEM_BYTES));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk, cudaFuncAttributeMaxDynamicSharedMemorySize, V2_SMEM_BYTES));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 7)));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 7, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 7)));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 8)));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<2, 9>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(2, 9)));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<2, 10>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(2, 10)));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 7, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 7)));
-  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<3, 7, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, t4_smem_bytes(3, 7)));
+  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, T4_SMEM_BYTES));
+  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, T4_SMEM_BYTES));
+  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, T4_SMEM_BYTES));
+  CRL_CUDA(cudaFuncSetAttribute(k_trunk4<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, T4_SMEM_BYTES));
   {
-    const char* r = getenv("CRL_T4_RING");   // tuning knob: 0 = 3/7 (default), 1 = 3/8, 2 = 2/9, 3 = 2/10
-    nw->t4_ring = r ? atoi(r) : 0;
-    const char* ns_ = getenv("CRL_T4_NO_SINGLE");
-    nw->t4_single = !(ns_ && ns_[0] == '1');
-    const char* np_ = getenv("CRL_T4_NSPLIT_PROBE");
-    nw->probe_nsplit = (np_ && np_[0] == '1') ? 1 : 0;
-    if (nw->t4_ring < 0 || nw->t4_ring > 3) nw->t4_ring = 0;
-    const char* h = getenv("CRL_T4_L2_HINTS");
-    nw->l2_hints = !(h && h[0] == '0');
-  }
-  {
-    // tensor-map table + layer table for the whole-tower kernel
-    if ((rc = dev_alloc(e, &nw->d_maps, 3 + N_CONVS))) return rc;
-    if ((rc = dev_alloc(e, &nw->d_layers, N_CONVS))) return rc;
+    // tensor-map table + layer table of the tower kernel
+    if ((rc = dev_alloc(e, &nw->d_maps4, 3 + N_CONVS))) return rc;
     if ((rc = dev_alloc(e, &nw->d_layers4, N_CONVS))) return rc;
     std::vector<CUtensorMap> hm(3 + N_CONVS);
     memset(hm.data(), 0, hm.size() * sizeof(CUtensorMap));
-    hm[1] = nw->map_act[0];
-    hm[2] = nw->map_act[1];
+    hm[1] = nw->map_act4[0];
+    hm[2] = nw->map_act4[1];
     for (int i = 0; i < N_CONVS; ++i) hm[3 + i] = nw->map_w2[i];
-    CRL_CUDA(cudaMemcpyAsync(nw->d_maps, hm.data(), hm.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice, e->stream));
-    if ((rc = dev_alloc(e, &nw->d_maps4, 3 + N_CONVS))) return rc;
-    std::vector<CUtensorMap> hm4(hm);
-    hm4[1] = nw->map_act4[0];
-    hm4[2] = nw->map_act4[1];
-    CRL_CUDA(cudaMemcpyAsync(nw->d_maps4, hm4.data(), hm4.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice, e->stream));
-    CRL_CUDA(cudaStreamSynchronize(e->stream));   // hm4 is a local
+    CRL_CUDA(cudaMemcpyAsync(nw->d_maps4, hm.data(), hm.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice, e->stream));
     std::vector<LayerDesc> hl(N_CONVS);
-    for (int variant = 0; variant < 2; ++variant) {     // 0: board-indexed buffers (v3), 1: slot-indexed scratch (v4)
-      __nv_bfloat16* const* act = variant ? nw->act4 : nw->act;
-      for (int L = 0; L < N_CONVS; ++L) {
-        LayerDesc& d = hl[L];
-        memset(&d, 0, sizeof(d));
-        d.map_w = 3 + L;
-        d.k_chunks = nw->cin[L] / BLOCK_K;
-        d.scale = nw->scale[L];
-        d.shift = nw->shift[L];
-        if (L == 0) {                      // stem: planes -> act[0], no BN / activation
-          d.map_in = 0;
-          d.out = act[0];
-          d.write_out = 1;
-        } else if ((L - 1) % 2 == 0) {     // conv_a: act[0] -> act[1], BN + ReLU
-          d.map_in = 1;
-          d.out = act[1];
-          d.relu = 1;
-          d.write_out = 1;
-        } else {                           // conv_b: act[1] -> act[0] in place (+ residual act[0]), BN, ReLU
-          d.map_in = 2;
-          d.out = act[0];
-          d.residual = act[0];
-          d.relu = 1;
-          d.write_out = L != N_CONVS - 1;  // the last layer only feeds the fused heads
-          d.fuse_heads = L == N_CONVS - 1;
-        }
+    __nv_bfloat16* const* act = nw->act4;
+    for (int L = 0; L < N_CONVS; ++L) {
+      LayerDesc& d = hl[L];
+      memset(&d, 0, sizeof(d));
+      d.map_w = 3 + L;
+      d.k_chunks = nw->cin[L] / BLOCK_K;
+      d.scale = nw->scale[L];
+      d.shift = nw->shift[L];
+      if (L == 0) {                      // stem: planes -> act[0], no BN / activation
+        d.map_in = 0;
+        d.out = act[0];
+        d.write_out = 1;
+      } else if ((L - 1) % 2 == 0) {     // conv_a: act[0] -> act[1], BN + ReLU
+        d.map_in = 1;
+        d.out = act[1];
+        d.relu = 1;
+        d.write_out = 1;
+      } else {                           // conv_b: act[1] -> act[0] in place (+ residual act[0]), BN, ReLU
+        d.map_in = 2;
+        d.out = act[0];
+        d.residual = act[0];
+        d.relu = 1;
+        d.write_out = L != N_CONVS - 1;  // the last layer only feeds the fused heads
+        d.fuse_heads = L == N_CONVS - 1;
       }
-      CRL_CUDA(cudaMemcpyAsync(variant ? nw->d_layers4 : nw->d_layers, hl.data(), hl.size() * sizeof(LayerDesc),
-                               cudaMemcpyHostToDevice, e->stream));
-      CRL_CUDA(cudaStreamSynchronize(e->stream));
     }
+    CRL_CUDA(cudaMemcpyAsync(nw->d_layers4, hl.data(), hl.size() * sizeof(LayerDesc), cudaMemcpyHostToDevice, e->stream));
+    CRL_CUDA(cudaStreamSynchronize(e->stream));   // hm and hl are locals
   }
   return CRL_OK;
 }
@@ -2001,8 +1349,6 @@ int net_load(crl_engine_impl* e, const float* const* w, const int64_t* sizes, in
   }
   CRL_CUDA(cudaMemcpyAsync(nw->w1x1, w1.data(), w1.size() * 4, cudaMemcpyHostToDevice, e->stream));
   CRL_CUDA(cudaMemcpyAsync(nw->s1x1, s1.data(), s1.size() * 4, cudaMemcpyHostToDevice, e->stream));
-  CRL_CUDA(cudaMemcpyAsync(nw->wp, w[P0 + 6], (size_t)128 * CRL_N_LABELS * 4, cudaMemcpyHostToDevice, e->stream));
-  CRL_CUDA(cudaMemcpyAsync(nw->bp, w[P0 + 7], CRL_N_LABELS * 4, cudaMemcpyHostToDevice, e->stream));
   CRL_CUDA(cudaMemcpyAsync(nw->wv1, w[V0 + 6], 64 * 256 * 4, cudaMemcpyHostToDevice, e->stream));
   CRL_CUDA(cudaMemcpyAsync(nw->bv1, w[V0 + 7], 256 * 4, cudaMemcpyHostToDevice, e->stream));
   CRL_CUDA(cudaMemcpyAsync(nw->wv2, w[V0 + 8], 256 * 4, cudaMemcpyHostToDevice, e->stream));
@@ -2024,28 +1370,8 @@ int net_load(crl_engine_impl* e, const float* const* w, const int64_t* sizes, in
   return CRL_OK;
 }
 
-static int launch_conv(crl_engine_impl* e, NetWeights* nw, const CUtensorMap& map_in, int L, const int* n_dev, int n_host,
-                       const __nv_bfloat16* residual, __nv_bfloat16* out, int relu) {
-  ConvParams p;
-  p.n_rows_dev = n_dev;
-  p.n_rows_host = n_host;
-  p.k_chunks = nw->cin[L] / BLOCK_K;
-  p.scale = nw->scale[L];
-  p.shift = nw->shift[L];
-  p.residual = residual;
-  p.out = out;
-  p.relu = relu;
-  int tiles = (n_host + 1) / 2;
-  int grid = tiles < nw->n_sms ? tiles : nw->n_sms;
-  if (grid < 1) grid = 1;
-  LaunchScope ls(e, KC_CONV);
-  k_conv3x3<<<grid, CONV_THREADS, CONV_SMEM_BYTES, e->stream>>>(map_in, nw->map_w[L], p);
-  CRL_CUDA(cudaGetLastError());
-  return CRL_OK;
-}
-
 static int launch_conv_v2(crl_engine_impl* e, NetWeights* nw, const CUtensorMap& map_in, int L, const int* n_dev,
-                          int n_host, const __nv_bfloat16* residual, __nv_bfloat16* out, int relu, bool fuse_heads) {
+                          int n_host, const __nv_bfloat16* residual, __nv_bfloat16* out, int relu) {
   ConvParams2 p;
   memset(&p, 0, sizeof(p));
   p.n_units_dev = n_dev;
@@ -2059,12 +1385,6 @@ static int launch_conv_v2(crl_engine_impl* e, NetWeights* nw, const CUtensorMap&
   p.residual = residual;
   p.out = out;
   p.relu = relu;
-  if (fuse_heads) {
-    p.head_w = nw->w1x1;
-    p.head_s = nw->s1x1;
-    p.pf_out = nw->pf;
-    p.vf_out = nw->vf;
-  }
   int work = (n_host + 3) / 4;
   int pairs = work < nw->n_sms / 2 ? work : nw->n_sms / 2;
   if (pairs < 1) pairs = 1;
@@ -2111,13 +1431,8 @@ static int launch_heads_v2(crl_engine_impl* e, NetWeights* nw, const int* n_dev,
   t.value = value;
   t.stats = nullptr;
   if (view_out) {
-    static const bool full = []() { const char* f = getenv("CRL_FULL_SOFTMAX"); return f && f[0] == '1'; }();
-    if (full) {
-      *view_out = PolicyView{policy, CRL_N_LABELS, nullptr};
-    } else {
-      t.stats = nw->stats;
-      *view_out = PolicyView{nw->logits, 2048, nw->stats};
-    }
+    t.stats = nw->stats;
+    *view_out = PolicyView{nw->logits, 2048, nw->stats};
   }
   LaunchScope ls(e, KC_HEADS);
   k_softmax_value<<<div_up(n_host, 8), 256, 0, e->stream>>>(t);
@@ -2155,102 +1470,46 @@ static int forward_nw(crl_engine_impl* e, NetWeights* nw, const __nv_bfloat16* p
     // GEMM depends on its own board's rows only, and the epilogue skips the boards at or after the row count.
     const int rows = fp8 ? e->R + 2 : planes == own ? e->R : n_host;
     if (planes != nw->planes_ptr || rows != nw->planes_rows || fp8 != nw->planes_fp8) {
-      int rc;
-      if (fp8) {
-        if ((rc = make_act_map4(nw, &nw->map_planes4, planes, 128, rows, true))) return rc;
-      } else {
-        if ((rc = make_act_map(nw, &nw->map_planes, planes, 128, rows))) return rc;
-        if ((rc = make_act_map4(nw, &nw->map_planes4, planes, 128, rows))) return rc;
-      }
+      const int rc = make_act_map4(nw, &nw->map_planes4, planes, 128, rows, fp8);
+      if (rc) return rc;
       nw->planes_ptr = planes;
       nw->planes_rows = rows;
       nw->planes_fp8 = fp8;
     }
   }
-  int rc;
-  if (nw->use_trunk) {
-    TrunkParams tp;
-    tp.n_dev = n_dev;
-    tp.n_host = n_host;
-    tp.n_layers = N_CONVS;
-    tp.head_w = nw->w1x1;
-    tp.head_s = nw->s1x1;
-    tp.pf_out = nw->pf;
-    tp.vf_out = nw->vf;
-    tp.dbg_out = dbg_out;
-    tp.dbg_layer = dbg_layer;
-    tp.hint_planes = nw->l2_hints ? L2_EVICT_FIRST : L2_EVICT_NORMAL;
-    tp.hint_weights = nw->l2_hints ? L2_EVICT_LAST : L2_EVICT_NORMAL;
-    tp.probe_nsplit = nw->probe_nsplit;
-    int groups = ((n_host + 3) / 4 + 1) / 2;
-    int pairs = groups < nw->n_sms / 2 ? groups : nw->n_sms / 2;
-    if (pairs < 1) pairs = 1;
-    // small batches (every tile of the batch BOUND gets a CTA pair of its own): the single-tile instantiation, one pair per tile
-    const int tiles = (n_host + 3) / 4;
-    const bool single = nw->use_trunk4 && nw->t4_single && tiles <= nw->n_sms / 2;
-    if (single) pairs = tiles < 1 ? 1 : tiles;
-    {
-      LaunchScope ls(e, KC_CONV);
-      if (fp8) {
-        if (single)
-          k_trunk4<3, 7, true, true><<<dim3(2 * pairs), dim3(CONV_THREADS), t4_smem_bytes(3, 7), e->stream>>>(
-              nw->map_planes4, nw->d_maps8, nw->d_layers8, tp);
-        else
-          k_trunk4<3, 7, false, true><<<dim3(2 * pairs), dim3(CONV_THREADS), t4_smem_bytes(3, 7), e->stream>>>(
-              nw->map_planes4, nw->d_maps8, nw->d_layers8, tp);
-      } else if (single) {
-        k_trunk4<3, 7, true><<<dim3(2 * pairs), dim3(CONV_THREADS), t4_smem_bytes(3, 7), e->stream>>>(nw->map_planes4, nw->d_maps4,
-                                                                                                  nw->d_layers4, tp);
-      } else if (nw->use_trunk4) {
-        const dim3 grid(2 * pairs), block(CONV_THREADS);
-        switch (nw->t4_ring) {
-          case 1: k_trunk4<3, 8><<<grid, block, t4_smem_bytes(3, 8), e->stream>>>(nw->map_planes4, nw->d_maps4, nw->d_layers4, tp); break;
-          case 2: k_trunk4<2, 9><<<grid, block, t4_smem_bytes(2, 9), e->stream>>>(nw->map_planes4, nw->d_maps4, nw->d_layers4, tp); break;
-          case 3: k_trunk4<2, 10><<<grid, block, t4_smem_bytes(2, 10), e->stream>>>(nw->map_planes4, nw->d_maps4, nw->d_layers4, tp); break;
-          default: k_trunk4<3, 7><<<grid, block, t4_smem_bytes(3, 7), e->stream>>>(nw->map_planes4, nw->d_maps4, nw->d_layers4, tp); break;
-        }
-      } else
-        k_trunk<<<2 * pairs, CONV_THREADS, V2_SMEM_BYTES, e->stream>>>(nw->map_planes, nw->d_maps, nw->d_layers, tp);
-      CRL_CUDA(cudaGetLastError());
+  TrunkParams tp;
+  tp.n_dev = n_dev;
+  tp.n_host = n_host;
+  tp.n_layers = N_CONVS;
+  tp.head_w = nw->w1x1;
+  tp.head_s = nw->s1x1;
+  tp.pf_out = nw->pf;
+  tp.vf_out = nw->vf;
+  tp.dbg_out = dbg_out;
+  tp.dbg_layer = dbg_layer;
+  tp.hint_planes = L2_EVICT_FIRST;
+  tp.hint_weights = L2_EVICT_LAST;
+  // small batches (every tile of the batch BOUND gets a CTA pair of its own): the single-tile instantiation, one pair per
+  // tile; otherwise groups of two tiles on at most one pair per two SMs
+  const int tiles = (n_host + 3) / 4;
+  const bool single = tiles <= nw->n_sms / 2;
+  const int pairs = single ? tiles : std::min((tiles + 1) / 2, nw->n_sms / 2);
+  {
+    LaunchScope ls(e, KC_CONV);
+    const dim3 grid(2 * pairs), block(CONV_THREADS);
+    if (fp8) {
+      if (single)
+        k_trunk4<true, true><<<grid, block, T4_SMEM_BYTES, e->stream>>>(nw->map_planes4, nw->d_maps8, nw->d_layers8, tp);
+      else
+        k_trunk4<false, true><<<grid, block, T4_SMEM_BYTES, e->stream>>>(nw->map_planes4, nw->d_maps8, nw->d_layers8, tp);
+    } else if (single) {
+      k_trunk4<true, false><<<grid, block, T4_SMEM_BYTES, e->stream>>>(nw->map_planes4, nw->d_maps4, nw->d_layers4, tp);
+    } else {
+      k_trunk4<false, false><<<grid, block, T4_SMEM_BYTES, e->stream>>>(nw->map_planes4, nw->d_maps4, nw->d_layers4, tp);
     }
-    return launch_heads_v2(e, nw, n_dev, n_host, policy, value, view_out);
+    CRL_CUDA(cudaGetLastError());
   }
-  if (nw->use_v2) {
-    if ((rc = launch_conv_v2(e, nw, nw->map_planes, 0, n_dev, n_host, nullptr, nw->act[0], 0, false))) return rc;
-    for (int b = 0; b < 10; ++b) {
-      if ((rc = launch_conv_v2(e, nw, nw->map_act[0], 1 + 2 * b, n_dev, n_host, nullptr, nw->act[1], 1, false))) return rc;
-      const bool last = b == 9;   // the last convolution feeds only the heads: fuse them, skip the activation write
-      if ((rc = launch_conv_v2(e, nw, nw->map_act[1], 2 + 2 * b, n_dev, n_host, nw->act[0], last ? nullptr : nw->act[0], 1,
-                               last)))
-        return rc;
-    }
-    return launch_heads_v2(e, nw, n_dev, n_host, policy, value, view_out);
-  }
-  // stem: conv only (model.py:33-34 -- no BatchNorm / activation after it)
-  if ((rc = launch_conv(e, nw, nw->map_planes, 0, n_dev, n_host, nullptr, nw->act[0], 0))) return rc;
-  for (int b = 0; b < 10; ++b) {
-    // x -> conv+BN+ReLU -> conv+BN -> +x -> ReLU  (model.py:111-122); the block output overwrites x in place
-    if ((rc = launch_conv(e, nw, nw->map_act[0], 1 + 2 * b, n_dev, n_host, nullptr, nw->act[1], 1))) return rc;
-    if ((rc = launch_conv(e, nw, nw->map_act[1], 2 + 2 * b, n_dev, n_host, nw->act[0], nw->act[0], 1))) return rc;
-  }
-  HeadParams hp;
-  hp.n_rows_dev = n_dev;
-  hp.n_rows_host = n_host;
-  hp.x = nw->act[0];
-  hp.w1x1 = nw->w1x1;
-  hp.s1x1 = nw->s1x1;
-  hp.wp = nw->wp;
-  hp.bp = nw->bp;
-  hp.wv1 = nw->wv1;
-  hp.bv1 = nw->bv1;
-  hp.wv2 = nw->wv2;
-  hp.bv2 = nw->bv2;
-  hp.policy = policy;
-  hp.value = value;
-  LaunchScope ls(e, KC_HEADS);
-  k_heads<<<div_up(n_host, HEAD_POS), HEAD_THREADS, HEAD_SMEM_BYTES, e->stream>>>(hp);
-  CRL_CUDA(cudaGetLastError());
-  return CRL_OK;
+  return launch_heads_v2(e, nw, n_dev, n_host, policy, value, view_out);
 }
 
 int net_forward(crl_engine_impl* e, const __nv_bfloat16* planes, int n_host, const int* n_dev, float* policy,
@@ -2280,8 +1539,7 @@ int net_debug_conv(crl_engine_impl* e, int layer, const __nv_bfloat16* in, int c
   CUtensorMap m;
   int rc = make_act_map(nw, &m, in, cin, n);
   if (rc) return rc;
-  if (nw->use_v2) return launch_conv_v2(e, nw, m, layer, nullptr, n, residual, out, relu, false);
-  return launch_conv(e, nw, m, layer, nullptr, n, residual, out, relu);
+  return launch_conv_v2(e, nw, m, layer, nullptr, n, residual, out, relu);
 }
 
 
@@ -2292,10 +1550,6 @@ int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int 
   NetWeights* nw = e->net;
   if (!nw || !nw->loaded) {
     set_error("network weights are not loaded");
-    return CRL_ESTATE;
-  }
-  if (!nw->use_trunk4) {
-    set_error("crl_debug_tower: the tap exists in the v4 tower kernel only (unset CRL_TRUNK_V3 / CRL_NO_TRUNK / CRL_CONV_V1)");
     return CRL_ESTATE;
   }
   if (n <= 0 || n > nw->cap_rows || (act_out && (layer < 0 || layer >= N_CONVS))) {
@@ -2317,17 +1571,6 @@ int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int 
 // ======================================================================================================
 bool net_fp8(const crl_engine_impl* e, int slot) { return e->nets[slot] && e->nets[slot]->fp8; }
 
-// the fp8 tower exists as k_trunk4<3, 7> (two tiles and single tile) only
-static int fp8_tower_available(const NetWeights* nw, const char* fn) {
-  if (!nw->use_trunk4 || nw->t4_ring != 0 || nw->probe_nsplit) {
-    set_error("%s: the fp8 tower is k_trunk4<3, 7> only; CRL_NO_TRUNK / CRL_TRUNK_V3 / CRL_CONV_V1 / CRL_T4_RING / "
-              "CRL_T4_NSPLIT_PROBE select another tower",
-              fn);
-    return CRL_ESTATE;
-  }
-  return CRL_OK;
-}
-
 // activation scale of one layer: the power of two 2^ceil(log2(amax / 448)), 1 for amax = 0
 static float act_scale(float amax) {
   const float r = amax / 448.f;
@@ -2341,10 +1584,6 @@ int net_calibrate(crl_engine_impl* e, const __nv_bfloat16* planes, int n, float*
   NetWeights* nw = e->net;
   if (!nw || !nw->loaded) {
     set_error("crl_net_calibrate_host: network weights are not loaded");
-    return CRL_ESTATE;
-  }
-  if (!nw->use_trunk4) {
-    set_error("crl_net_calibrate_host: the tap exists in the v4 tower kernel only");
     return CRL_ESTATE;
   }
   if (n <= 0 || n > nw->cap_rows) {
@@ -2383,15 +1622,14 @@ int net_calibrate(crl_engine_impl* e, const __nv_bfloat16* planes, int n, float*
 int net_load_fp8(crl_engine_impl* e, const float* const* w, const int64_t* sizes, int n, const float* act_amax) {
   NetWeights* nw = e->net;
   nw->fp8 = false;                                     // whatever fails below, the engine is left in bf16
-  int rc = fp8_tower_available(nw, "crl_net_load_fp8_host");
-  if (rc) return rc;
   for (int L = 0; L < N_CONVS; ++L) {
     if (!(act_amax[L] >= 0.f) || !isfinite(act_amax[L])) {
       set_error("crl_net_load_fp8_host: activation amax %d is %g (must be finite and >= 0)", L, (double)act_amax[L]);
       return CRL_EINVAL;
     }
   }
-  if ((rc = net_load(e, w, sizes, n))) return rc;      // validates the pack, loads the bf16 tower, drops fp8 state
+  int rc = net_load(e, w, sizes, n);                   // validates the pack, loads the bf16 tower, drops fp8 state
+  if (rc) return rc;
   if (!nw->act8[0]) {
     for (int L = 0; L < N_CONVS; ++L) {
       if ((rc = dev_alloc(e, &nw->w8[L], (size_t)TILE_N * 9 * nw->cin[L]))) return rc;
@@ -2442,7 +1680,7 @@ int net_load_fp8(crl_engine_impl* e, const float* const* w, const int64_t* sizes
     CRL_CUDA(cudaMemcpyAsync(nw->scale8[L], sc.data(), 1024, cudaMemcpyHostToDevice, e->stream));
     CRL_CUDA(cudaMemcpyAsync(nw->shift8[L], sh.data(), 1024, cudaMemcpyHostToDevice, e->stream));
     CRL_CUDA(cudaStreamSynchronize(e->stream));
-    // the same dataflow as the bf16 v4 tower's layer table (net_create), on the e4m3 scratch
+    // the same dataflow as the bf16 tower's layer table (net_create), on the e4m3 scratch
     LayerDesc8& d = hl[L];
     memset(&d, 0, sizeof(d));
     d.map_w = 3 + L;
@@ -2491,8 +1729,6 @@ int net_set_precision(crl_engine_impl* e, int precision) {
     set_error("crl_net_set_precision: no fp8 weights in slot %d (crl_net_load_fp8_host)", e->sel_slot);
     return CRL_ESTATE;
   }
-  int rc = fp8_tower_available(nw, "crl_net_set_precision");
-  if (rc) return rc;
   if (!nw->fp8_loaded) {
     set_error("crl_net_set_precision: no fp8 weights (crl_net_load_fp8_host)");
     return CRL_ESTATE;

@@ -172,9 +172,8 @@ int crl_debug_forward_counted(crl_engine* e, const void* planes_bf16_dev, int n_
  *                            >= 0, else CRL_EINVAL); selects fp8.  On any error the engine is left in bf16.
  *   crl_net_set_precision  : CRL_NET_BF16 or CRL_NET_FP8 (CRL_ESTATE without an fp8 load).  crl_net_load_host returns
  *                            the engine to bf16 and drops the fp8 tower.
- * fp8 exists in the default tower only: with CRL_NO_TRUNK, CRL_TRUNK_V3, CRL_CONV_V1, CRL_T4_RING != 0 or
- * CRL_T4_NSPLIT_PROBE set at crl_create, selecting it returns CRL_ESTATE.  In fp8 mode crl_net_forward,
- * crl_debug_tower and crl_debug_forward_counted take bf16 planes as before and convert them. */
+ * In fp8 mode crl_net_forward, crl_debug_tower and crl_debug_forward_counted take bf16 planes as before and convert
+ * them. */
 #define CRL_NET_BF16 0
 #define CRL_NET_FP8 1
 int crl_net_calibrate_host(crl_engine* e, const void* planes_bf16_dev, int n, float* amax_host);

@@ -1,15 +1,14 @@
 #!/bin/bash
-# Round 2, second GPU call: two-phase tree kernels, L2 eviction hints (A/B), one-block first perft plies, fresh rule-kernel ncu
+# Round 2, second GPU call: two-phase tree kernels, L2 eviction hints, one-block first perft plies, fresh rule-kernel ncu
 mkdir -p gpurun_out
 T0=$SECONDS
 timeout 900 python -m pytest tests -m gpu -q --timeout 300 -x > gpurun_out/pytest_gpu.log 2>&1; echo "== pytest -m gpu: $? at $((SECONDS-T0)) s"; tail -8 gpurun_out/pytest_gpu.log
 S="--no-cpu-baseline --no-perft --no-kernels --no-whole-games --no-large"
 timeout 300 python bench.py --steps 4 --warmup 3 $S > gpurun_out/bench_hints_on.log 2>&1; echo "== hints on: $?"
-CRL_T4_L2_HINTS=0 timeout 300 python bench.py --steps 4 --warmup 3 $S > gpurun_out/bench_hints_off.log 2>&1; echo "== hints off: $?"
 timeout 300 python bench.py --games 512 --sims 200 --steps 4 --warmup 3 $S > gpurun_out/bench_512x200.log 2>&1; echo "== 512 lanes: $?"
 python - <<'PY'
 import json
-for f in ("hints_on", "hints_off", "512x200"):
+for f in ("hints_on", "512x200"):
     try:
         d = json.loads(open("gpurun_out/bench_%s.log" % f).read().strip().splitlines()[-1])
         print(f, "value", round(d["value"]), "e2e", round(d["e2e"]["value"]), "roof", round(d["roofline"]["achieved"]), d["roofline"]["share_of_step_ms"], d["clocks"])

@@ -6,10 +6,9 @@ T0=$SECONDS
 timeout 600 python -m pytest tests -m gpu -q -x --timeout 300 > gpurun_out/pytest_gpu.log 2>&1; echo "== pytest -m gpu: $? at $((SECONDS-T0)) s"; tail -4 gpurun_out/pytest_gpu.log
 timeout 60 python -c "import __graft_entry__ as g; g.smoke()" > gpurun_out/smoke.log 2>&1; echo "== smoke: $? at $((SECONDS-T0)) s"; tail -1 gpurun_out/smoke.log
 timeout 300 python bench.py --steps 5 --warmup 3 --no-cpu-baseline --no-perft --no-kernels --no-large > gpurun_out/bench_sixth.log 2> gpurun_out/bench_sixth.err; echo "== bench: $? at $((SECONDS-T0)) s"
-CRL_FULL_SOFTMAX=1 timeout 200 python bench.py --steps 5 --warmup 3 --no-cpu-baseline --no-perft --no-kernels --no-large --no-whole-games > gpurun_out/bench_sixth_fullsoftmax.log 2> gpurun_out/bench_sixth_fullsoftmax.err; echo "== bench (full softmax rows): $? at $((SECONDS-T0)) s"
 python - <<'PY'
 import json
-for f in ("bench_sixth", "bench_sixth_fullsoftmax"):
+for f in ("bench_sixth",):
     try:
         d = json.loads(open("gpurun_out/%s.log" % f).read().strip().splitlines()[-1])
         print(f, "value", round(d["value"]), "e2e", round(d["e2e"]["value"]), d["clocks"], d["roofline"]["share_of_step_ms"], "launches", d["gpu_launches"])

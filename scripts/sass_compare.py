@@ -1,7 +1,8 @@
 """Compares the SASS of two builds kernel by kernel: `python scripts/sass_compare.py OLD.sass NEW.sass`, each the output
 of `cuobjdump -sass` on an object file.  Instructions are compared with their addresses and encodings stripped; k_trunk4
-instantiations are matched by their template arguments, a missing FP8 argument counting as false (the bf16 tower),
-k_encode_rows by its bf16 form, and k_ab_items by its repetition argument, the untemplated kernel counting as false
+instantiations are matched by their SINGLE / FP8 arguments, a missing FP8 argument counting as false (the bf16 tower) and
+the image-slot / weight-stage arguments of older builds dropped when they are the 3 / 7 that is now fixed (other ring
+sizes keep them), k_encode_rows by its bf16 form, and k_ab_items by its repetition argument, the untemplated kernel counting as false
 (the plain search).  Prints one line per kernel: identical, DIFFERENT or new."""
 import re
 import sys
@@ -21,9 +22,10 @@ def functions(path):
 
 
 def key(name):
-    m = re.match(r"_ZN3crl8k_trunk4ILi(\d+)ELi(\d+)ELb(\d)E(?:Lb(\d)E)?", name)
+    m = re.match(r"_ZN3crl8k_trunk4I(?:Li(\d+)ELi(\d+)E)?Lb(\d)E(?:Lb(\d)E)?", name)
     if m:
-        return "k_trunk4<%s,%s,%s,%s>" % (m.group(1), m.group(2), m.group(3), m.group(4) or "0")
+        ring = "" if m.group(1) in (None, "3") and m.group(2) in (None, "7") else "%s,%s," % (m.group(1), m.group(2))
+        return "k_trunk4<%s%s,%s>" % (ring, m.group(3), m.group(4) or "0")
     if re.match(r"_ZN3crl13k_encode_rows(ENS_5Pools|I13__nv_bfloat16E)", name):
         return "k_encode_rows<bf16>"
     m = re.match(r"_ZN3crl10k_ab_items(?:ILb(\d)EE)?", name)

@@ -3,8 +3,7 @@ on the host, the two-tile tower instantiation -- against the uncounted forward p
 real network against the oracle.
 
 Every comparison here is bit-exact (torch.equal / array equality): the kernels' rows must not depend on the batch they
-sit in, on where they sit in it, on the tower instantiation or its tuning knobs, or on rows that are not part of the
-batch.  That is what lets the oracle be served by crl_net_forward in small batches while the engine evaluates the same
+sit in, on where they sit in it, on the tower instantiation, or on rows that are not part of the batch.  That is what lets the oracle be served by crl_net_forward in small batches while the engine evaluates the same
 positions as rows of 4,096-row batches (net_oracle.py).
 
 Default sizes keep this file to a few minutes; CRL_PARITY_SIMS=200 CRL_PARITY_MOVES=4 runs the searches at BASELINE's
@@ -120,44 +119,31 @@ def test_counted_batch_rejects_bad_arguments(wide, planes):
     assert lib.crl_debug_forward_counted(h, None, 0, cnt.data_ptr(), None, None) == 0     # an empty launch bound: nothing to do
 
 
-# ---- b. instantiations and knobs -----------------------------------------------------------------------------------
-@pytest.mark.parametrize("env", [("CRL_T4_NO_SINGLE", "1"), ("CRL_T4_RING", "1"), ("CRL_T4_RING", "2"),
-                                 ("CRL_T4_RING", "3"), ("CRL_T4_L2_HINTS", "0")])
-def test_tower_instantiations_and_knobs_give_the_same_bits(wide, pack, planes, monkeypatch, env):
-    """Single-tile vs two-tile instantiation (n <= 296 takes the single-tile one unless CRL_T4_NO_SINGLE=1), the
-    shared-memory ring variants and the L2 eviction hints: same arithmetic, so bit-identical outputs."""
-    x, _ = planes
-    monkeypatch.setenv(*env)
-    other = Engine(max_games=600, max_nodes=2)
-    other.load_weights(pack)
-    sizes = (1, 5, 37, 296) if env[0] == "CRL_T4_NO_SINGLE" else (1, 5, 37, 296, 593)
-    for n in sizes:
-        xs = x[:n].contiguous()
-        p0, v0 = wide.net_forward(xs)
-        p1, v1 = other.net_forward(xs)
-        assert torch.equal(p0, p1) and torch.equal(v0, v1), (env, n)
-    other.close()
+# ---- b. the bit-identity checks can fail -----------------------------------------------------------------------------
+def _rel_err(a, b):
+    a, b = a.float(), b.float()
+    return ((a - b).abs().max() / b.abs().max().clamp_min(1e-30)).item()
 
 
-def test_bit_identity_is_not_vacuous(wide, pack, planes, monkeypatch):
-    """The v3 tower (a different accumulation order) lands within the emulation's tolerance but differs in at least one
-    bit: the outputs are sensitive to summation order, so the torch.equal checks above mean something."""
+def test_bit_identity_is_not_vacuous_per_layer(wide, pack, planes):
+    """Layer 1 of the tower recomputed by k_conv_v2 from the tower's own layer-0 output: the same convolution on the same
+    bf16 input, but k_conv_v2 accumulates tap-outer / channel-slice-inner where k_trunk4 accumulates channel-slice-outer /
+    tap-inner.  It lands within the emulation's tolerance but differs in at least one bit: the outputs are sensitive to
+    summation order, so the torch.equal checks in this file mean something."""
     x, _ = planes
-    n = 593
-    monkeypatch.setenv("CRL_TRUNK_V3", "1")
-    v3 = Engine(max_games=600, max_nodes=2)
-    v3.load_weights(pack)
-    xs = x[:n].contiguous()
-    p0, v0 = wide.net_forward(xs)
-    p1, v1 = v3.net_forward(xs)
-    v3.close()
+    xs = x[:593].contiguous()
+    tap0 = wide.debug_tower(xs, layer=0)["act"]
+    tap1 = wide.debug_tower(xs, layer=1)["act"]
+    conv = wide.debug_conv(1, tap0, None, relu=True)
+    torch.cuda.synchronize()
     xf = xs.float().cpu().numpy()[..., :127]
-    rp, rv = model_torch.forward(pack, xf, device="cuda")
-    ep, ev = model_torch.forward(pack, xf, device="cuda", emulate_bf16_activations=True)
+    f32, emu = {}, {}
+    rp, rv = model_torch.forward(pack, xf, device="cuda", taps=f32)
+    model_torch.forward(pack, xf, device="cuda", emulate_bf16_activations=True, taps=emu)
     netpacks.assert_lively(rp, rv)
-    Ep, Ev = (ep - rp).abs().max().item(), (ev - rv).abs().max().item()
-    assert (p0 - p1).abs().max().item() <= 2 * Ep + 1e-7 and (v0 - v1).abs().max().item() <= 2 * Ev + 1e-6
-    assert not (torch.equal(p0, p1) and torch.equal(v0, v1))
+    E = _rel_err(emu["act"][1], f32["act"][1])
+    assert _rel_err(conv, tap1) <= 2 * E, (_rel_err(conv, tap1), E)
+    assert not torch.equal(conv, tap1)
 
 
 # ---- c. row independence in the two-tile instantiation ----------------------------------------------------------------

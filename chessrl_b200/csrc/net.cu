@@ -1571,10 +1571,12 @@ int net_debug_tower(crl_engine_impl* e, const __nv_bfloat16* planes, int n, int 
 // ======================================================================================================
 bool net_fp8(const crl_engine_impl* e, int slot) { return e->nets[slot] && e->nets[slot]->fp8; }
 
-// activation scale of one layer: the power of two 2^ceil(log2(amax / 448)), 1 for amax = 0
+// activation scale of one layer: the power of two max(2^ceil(log2(amax / 448)), 2^-126), 1 for amax = 0.  The floor is
+// the smallest normal power of two: below it 1 / s overflows to inf and the epilogue's e4m3(a * inf) is NaN for a = 0.
 static float act_scale(float amax) {
+  if (!(amax > 0.f)) return 1.f;
+  if (amax <= 448.f * 0x1p-126f) return 0x1p-126f;   // also where amax / 448 would round to a subnormal or to 0
   const float r = amax / 448.f;
-  if (!(r > 0.f)) return 1.f;
   int ex;
   const float m = frexpf(r, &ex);   // r = m * 2^ex, m in [0.5, 1)
   return ldexpf(1.f, m == 0.5f ? ex - 1 : ex);

@@ -164,8 +164,8 @@ int crl_debug_forward_counted(crl_engine* e, const void* planes_bf16_dev, int n_
                               float* policy_dev, float* value_dev);
 /* Opt-in fp8 evaluation.  The 21 tower convolutions run on e4m3 operands (tcgen05 kind::f8f6f4, fp32 accumulation):
  * planes exactly, weights per output channel scaled to max |W| = 448, each layer's output (but the last, which feeds
- * the bf16 heads) as e4m3 x a power-of-two scale 2^ceil(log2(amax / 448)) from calibration.  Heads, softmax and search
- * are unchanged.  Not bit-exact with bf16; DESIGN.md section 3.1 states the definition and the measured deviation.
+ * the bf16 heads) as e4m3 x a power-of-two scale max(2^ceil(log2(amax / 448)), 2^-126) from calibration (1 for
+ * amax 0; the floor keeps 1 / scale finite).  Heads, softmax and search are unchanged.  Not bit-exact with bf16; DESIGN.md section 3.1 states the definition and the measured deviation.
  *   crl_net_calibrate_host : runs the bf16 tower on planes_bf16_dev [n][8][8][128] and writes max |output| of each
  *                            convolution to amax_host [21]
  *   crl_net_load_fp8_host  : crl_net_load_host, then the fp8 tower from the same pack and act_amax_host [21] (finite,

@@ -4,7 +4,8 @@ The numeric definition, shared with csrc/net.cu:
   - planes are e4m3 (0 / 1: exact);
   - weights per output channel n of convolution L: ws[n] = max_k |W[k][n]| / 448 (1 for an all-zero column),
     Wq = e4m3_rn_satfinite(W / ws[n]);
-  - the outputs of convolutions 0..19 are stored as e4m3(a / s_L) with s_L = 2^ceil(log2(amax_L / 448)) (1 for amax 0);
+  - the outputs of convolutions 0..19 are stored as e4m3(a / s_L) with s_L = max(2^ceil(log2(amax_L / 448)), 2^-126)
+    (1 for amax 0; the floor is the smallest normal power of two, so that 1 / s_L is finite);
     convolution 20 feeds only the heads and keeps the bf16 rounding of the bf16 tower;
   - epilogue: a = acc * (ws[n] * s_in * bn_scale[n]) + bn_shift[n], + dequant(residual) * s_res, ReLU.
 The heads are the bf16 tower's (oracle/model_torch.forward with emulate_bf16_activations=True).
@@ -17,6 +18,7 @@ import torch
 import torch.nn.functional as F
 
 E4M3_MAX = 448.0
+SCALE_FLOOR = 2.0 ** -126       # the smallest normal float32 power of two: the least activation scale
 BN_EPS = np.float32(1e-3)
 
 
@@ -26,10 +28,13 @@ def e4m3(x):
 
 
 def act_scale(amax):
-    """2^ceil(log2(amax / 448)) in float32 arithmetic, 1 for amax = 0."""
-    r = np.float32(amax) / np.float32(E4M3_MAX)
-    if not r > 0:
+    """max(2^ceil(log2(amax / 448)), 2^-126) in float32 arithmetic, 1 for amax = 0 (the floor keeps 1 / s finite)."""
+    a = np.float32(amax)
+    if not a > 0:
         return 1.0
+    if a <= np.float32(E4M3_MAX * SCALE_FLOOR):
+        return SCALE_FLOOR
+    r = a / np.float32(E4M3_MAX)
     m, e = np.frexp(r)
     return float(np.ldexp(np.float32(1.0), int(e) - 1 if m == 0.5 else int(e)))
 

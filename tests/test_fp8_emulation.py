@@ -30,6 +30,16 @@ def test_activation_scale_rule():
     for a in np.float32([1e-3, 0.37, 5.0, 91.0, 4096.0]):
         s = fp8_emu.act_scale(a)
         assert a / s <= 448.0 < 2 * a / s
+    # the floor: scales below the smallest normal power of two would have an infinite reciprocal (NaN codes for a = 0)
+    floor = 2.0 ** -126
+    edge = np.float32(448.0 * floor)
+    for a in (np.float32(1e-37), np.float32(1e-40), np.float32(448.0 * 2.0 ** -128),
+              np.nextafter(np.float32(0), np.float32(1)), edge):         # ... the smallest subnormal, the floor's own amax
+        s = fp8_emu.act_scale(a)
+        assert s == floor, (a, s)
+        assert np.isfinite(np.float32(1.0) / np.float32(s))
+        assert np.float32(a) * (np.float32(1.0) / np.float32(s)) <= 448.0
+    assert fp8_emu.act_scale(np.nextafter(edge, np.float32(1))) == 2.0 ** -125
 
 
 def test_weight_quantisation_maps_each_column_max_to_448():
